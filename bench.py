@@ -18,6 +18,10 @@ roofline = the dominant kernel family (tcgen05 implicit-GEMM: all convolutions a
          in a separate profiled step with CUDA events around every launch on the launching stream.
 cpu_baseline = the oracle port of the reference forward (oracle/forward_oracle.py, fp32, all host
          threads) timed on a bounded sample of the same workload, rank 0, N=1 only.
+
+--dump-outputs DIR writes what the last timed step returned, so that two builds can be compared output for
+output on the same seeded inputs: DIR/logits.npy (the gathered [global_batch, 10] logits) and, unless
+--no-e2e, DIR/e2e_logits.npy (the same through the host path), float32.
 """
 
 from __future__ import annotations
@@ -39,6 +43,7 @@ UNIT = "samples/s"
 FLOP_PER_SAMPLE = 30.53e9  # BASELINE.md section 2: full multimodal forward, S=128
 SEQ = 128
 IMG = 224
+DUMP_LIMIT = 64 << 20  # bytes of --dump-outputs in all
 
 
 def _peaks():
@@ -122,6 +127,22 @@ def make_shard(lo, hi, device=None, pin=False):
     if device is not None:
         return images.to(device), ids.to(device), mask.to(device)
     return images, ids, mask
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes out_dir/<name>.npy for each [rows, ...] float32 array (all with the same rows).  Above DUMP_LIMIT
+    bytes in all, every array keeps the same fixed, seeded sample of rows, listed in rows.npy (float64)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    n = next(iter(arrays.values())).shape[0]
+    keep = (DUMP_LIMIT - 4096) // (sum(a[:1].nbytes for a in arrays.values()) + 8)  # 4096: room for the npy headers
+    if n > keep:
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def cpu_forward_timer(samples: int, iters: int, warmup: int):
@@ -283,7 +304,13 @@ def main():
                     help="mrd_ctx_set_option switches for A/B runs, e.g. fuse_ds=0")
     ap.add_argument("--no-other-configs", action="store_true",
                     help="skip the short timings of configs[1], [2] and [4] in the N=1 line")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the logits of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -371,6 +398,8 @@ def main():
     # bit-exact digest of the gathered logits: inputs are generated by global sample index and no op of the
     # forward mixes samples, so this is the same string at N = 1, 2, 4, 8 (SURVEY.md section 4(iv))
     logits_digest = synth.tensor_digest(logits) if rank == 0 else None
+    # host copy now: the e2e path below writes into the same gather buffer
+    dumps = {"logits": logits.float().cpu().numpy()} if rank == 0 and args.dump_outputs else None
 
     # ---------------------------------------------------------------- e2e: host buffers -> logits on host
     e2e = None
@@ -399,6 +428,8 @@ def main():
             tt = torch.tensor([ems], device=dev, dtype=torch.float64)
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
             ems = tt.item()
+        if dumps is not None:
+            dumps["e2e_logits"] = h_logits.numpy().copy()
         h2d = sum(x.numel() * x.element_size() for x in (h_images, h_ids, h_mask))
         e2e = {"value": total / (ems / args.steps * 1e-3), "unit": UNIT,
                "logits_sha256": synth.tensor_digest(h_logits) if rank == 0 else None,
@@ -502,6 +533,8 @@ def main():
             "kernel_families": families, "cpu_baseline": cpu, "bert_live_token_fraction": live_frac,
             "device_bytes": eng.device_bytes,
         }
+        if dumps is not None:
+            dump_outputs(args.dump_outputs, dumps)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

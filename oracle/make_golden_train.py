@@ -88,6 +88,8 @@ def main():
                                                          "cnn_encoder.backbone.layer4.2.bn3.running_var",
                                                          "cnn_encoder.backbone.layer4.0.downsample.1.running_mean")}
             fix["num_batches_tracked"] = int(sd["cnn_encoder.backbone.bn1.num_batches_tracked"])
+        # two files, each under 1 MB: tests/synth.py load_train_golden() joins them
+        torch.save(fix.pop("post"), os.path.join(out_dir, name + ".post.pt"))
         torch.save(fix, os.path.join(out_dir, name + ".pt"))
         print(name, "loss", loss.item(), "grad norm", float(total_norm), "params with grad", len(grads),
               "requires_grad but None:", len(none_grad))

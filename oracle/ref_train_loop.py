@@ -5,7 +5,8 @@ tests/test_train_gpu.py::test_training_loop_follows_reference.  Build container 
     python oracle/ref_train_loop.py
 """
 import sys, os, torch, torch.nn as nn
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tests'); sys.path.insert(0,'/root/repo/oracle')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+for p in (ROOT, os.path.join(ROOT, 'tests'), os.path.join(ROOT, 'oracle')): sys.path.insert(0, p)
 import synth
 from make_golden import build_reference
 torch.manual_seed(3)

@@ -1,9 +1,10 @@
 """Accuracy of the fused tail (one launch) against the per-layer launches, both against the oracle (imports oracle/, so it lives under tests/)."""
 import os, sys, torch
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import mrd_b200, synth
 from oracle import forward_oracle as oracle
-GOLD = "tests/golden"
+GOLD = os.path.join(ROOT, "tests", "golden")
 model = synth.build_model(0)
 plain = {k: v.clone() for k, v in model.state_dict().items()}
 sens = synth.sensitise(plain, 1)

@@ -18,3 +18,15 @@ checksum = _s.checksum
 make_inputs = _s.make_inputs
 make_global_rows = _s.make_global_rows
 tensor_digest = _s.tensor_digest
+
+GOLD = os.path.join(ROOT, "tests", "golden")
+
+
+def load_train_golden(name):
+    """A training-step fixture (oracle/make_golden_train.py).  The post-AdamW parameter samples are stored
+    in <name>.post.pt beside <name>.pt, which keeps every fixture file under 1 MB."""
+    import torch
+
+    fix = torch.load(os.path.join(GOLD, name + ".pt"))
+    fix["post"] = torch.load(os.path.join(GOLD, name + ".post.pt"))
+    return fix

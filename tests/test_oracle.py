@@ -91,7 +91,8 @@ def test_every_fixture_is_covered():
                      "padded_sens_b3_s48", "text_sens_b2_s512", "text_plain_b3_s200",
                      "image_sens_b2_160x96",
                      # training-step fixtures: covered by tests/test_train_oracle.py
-                     "train_p0_bn_eval_b4_s32", "train_p0_bn_train_b4_s32"}
+                     "train_p0_bn_eval_b4_s32", "train_p0_bn_train_b4_s32",
+                     "train_p0_bn_eval_b4_s32.post", "train_p0_bn_train_b4_s32.post"}
 
 
 @pytest.mark.parametrize("use_residual", [True, False])

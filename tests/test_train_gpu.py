@@ -16,7 +16,6 @@ random-init BERT meets that - stock PyTorch bf16 autocast is 16-25 % off fp32 on
 """
 
 import ctypes as C
-import os
 
 import pytest
 import torch
@@ -28,7 +27,6 @@ import synth
 from oracle import train_oracle as T
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 GRAD_TOL = 5e-2
 
 
@@ -270,7 +268,7 @@ def _train_model(sens, zero_dropout=True):
 def test_train_step_vs_reference_fixture(cuda, sens):
     """One src/train.py-style step through the module API: loss.backward() fills .grad through the library's
     backward; clip_grad_norm_ and torch.optim.AdamW stay the caller's, as in the reference."""
-    fix = torch.load(os.path.join(GOLD, "train_p0_bn_eval_b4_s32.pt"))
+    fix = synth.load_train_golden("train_p0_bn_eval_b4_s32")
     model = _train_model(sens)
     images, ids, mask = synth.make_inputs(fix["B"], fix["S"], fix["seed"], fix["lengths"], H=fix["H"], W=fix["W"])
     labels = torch.tensor(fix["labels"]).cuda()
@@ -502,7 +500,7 @@ def test_training_loop_follows_reference(cuda):
 def test_train_step_batchnorm_batch_statistics(cuda, sens):
     """A bare model.train() (what the reference's trainers call, src/train.py:240): the frozen backbone's
     BatchNorm layers use batch statistics and update their running buffers (TV:143-163 in train mode)."""
-    fix = torch.load(os.path.join(GOLD, "train_p0_bn_train_b4_s32.pt"))
+    fix = synth.load_train_golden("train_p0_bn_train_b4_s32")
     model = synth.build_model(0)
     model.load_state_dict(sens)
     _zero_dropout(model)
@@ -718,7 +716,7 @@ def test_fp32_check_backward_vs_reference_fixture(cuda, sens):
     the fixture of the unmodified reference (autograd, fp32), at a fixed relative-L2 bar of 1e-4 per tensor.
     This is what separates a structural error in a layer's backward from bf16 rounding: the bf16 step below is
     then held to fixed bars against these gradients."""
-    fix = torch.load(os.path.join(GOLD, "train_p0_bn_eval_b4_s32.pt"))
+    fix = synth.load_train_golden("train_p0_bn_eval_b4_s32")
     images, ids, mask = synth.make_inputs(fix["B"], fix["S"], fix["seed"], fix["lengths"], H=fix["H"], W=fix["W"])
     loss, logits, grads = _fp32_check_grads(sens, images, ids, mask, labels=torch.tensor(fix["labels"]))
     assert abs(loss - fix["loss"]) <= 1e-5 * abs(fix["loss"]), (loss, fix["loss"])
@@ -792,6 +790,6 @@ def test_bf16_step_fixed_bar_linear_loss(cuda):
 
 
 def test_bf16_step_fixed_bar_cross_entropy(cuda, sens):
-    fix = torch.load(os.path.join(GOLD, "train_p0_bn_eval_b4_s32.pt"))
+    fix = synth.load_train_golden("train_p0_bn_eval_b4_s32")
     images, ids, mask = synth.make_inputs(fix["B"], fix["S"], fix["seed"], fix["lengths"], H=fix["H"], W=fix["W"])
     _bf16_vs_fp32_check(sens, images, ids, mask, "ce", labels=torch.tensor(fix["labels"]))

@@ -2,15 +2,11 @@
 tests/golden/train_*.pt hold loss, gradients and post-AdamW parameters of the UNMODIFIED reference model
 run through one src/train.py-style step with dropout p = 0 (oracle/make_golden_train.py).  CPU only."""
 
-import os
-
 import pytest
 import torch
 
 import synth
 from oracle import train_oracle as T
-
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def _sample(t, stride):
@@ -24,7 +20,7 @@ def sens():
 
 @pytest.mark.parametrize("name", ["train_p0_bn_eval_b4_s32", "train_p0_bn_train_b4_s32"])
 def test_train_oracle_matches_reference_step(sens, name):
-    fix = torch.load(os.path.join(GOLD, name + ".pt"))
+    fix = synth.load_train_golden(name)
     images, ids, mask = synth.make_inputs(fix["B"], fix["S"], fix["seed"], fix["lengths"], H=fix["H"], W=fix["W"])
     labels = torch.tensor(fix["labels"])
     stats = {} if fix["bn_train"] else None
