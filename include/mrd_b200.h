@@ -54,12 +54,9 @@ int mrd_ctx_configure(mrd_ctx* ctx, int img_chunk, int seq_chunk_tokens);
 
 /* Scalar options: "bert_heads" (12), "bert_ln_eps" (1e-12), "bn_eps" (1e-5), "fusion_ln_eps" (1e-5),
  * "fusion_heads" (8), "fusion_residual" (1), "head_act" (MRD_ACT_RELU).  Set before load_weights.
- * "fuse_ds" (1): run conv3 + downsample of each stage's first bottleneck as one K-concatenated GEMM
- * (mrd_conv1x1_dual_bf16); 0 = separate downsample launch + residual read (A/B switch, same results up to
- * the bf16 rounding of the downsample output that the fused form never materialises).
- * "fuse_pool" (1): the stem launch also does the max pooling (mrd_stem_pool_bf16); 0 = separate pooling pass.
- * "fuse_chain" (1): bit L-1 set = the tail of every bottleneck of ResNet stage L is chained with the next
- * block's conv1 in one launch (mrd_conv_chain_bf16); 0 = one launch per convolution. */
+ * "fp32_check" (0): forwards run the plain-fp32 reference kernels.  "load_sync" (1): load_weights synchronises
+ * the device before re-packing and the stream afterwards; 0 drops both.  "train.*": options of the training step.
+ * Any other key returns -1 ("unknown option"). */
 int mrd_ctx_set_option(mrd_ctx* ctx, const char* key, double value);
 
 /* Hands the context the model's fp32 parameters/buffers by their state_dict names
@@ -104,7 +101,7 @@ int mrd_head_fwd(mrd_ctx* ctx, const float* x, int B, float* logits, float* prob
  * (src/fusion_model.py:245-291) -> ClassificationHead -> softmax (src/multimodal_classifier.py:73-83,166-167).
  * img_emb f32 [B,Di], txt_emb f32 [B,Dt] -> logits f32 [B,C]; probs f32 [B,C] and fused f32 [B,Hd] optional.
  * Falls back to the per-layer launches of mrd_fusion_fwd + mrd_head_fwd when the shapes are outside the fused
- * kernel's range or the option "fuse_tail" is 0. */
+ * kernel's range. */
 int mrd_fusion_head_fwd(mrd_ctx* ctx, const float* img_emb, const float* txt_emb, int B, float* fused,
                         float* logits, float* probs, void* stream);
 
@@ -141,12 +138,10 @@ int mrd_gemm_bf16(const void* A, long long lda, int M, int K, const void* W, int
                   long long ld_res, float* out_f32, long long ld_f32, int act, void* stream);
 
 /* C = LayerNorm(A W^T + bias + residual) * gamma + beta over whole rows (HF:models/bert/modeling_bert.py:294-298,
- * 352-356: BertSelfOutput / BertOutput) in ONE launch: a thread-block cluster of N/256 CTAs owns a 128-row stripe and
- * exchanges the row statistics through distributed shared memory.  N in {512, 768, 1024}, otherwise -1.
- * residual may be NULL.
- * stats_ws: NULL = the cluster / distributed-shared-memory exchange described above; otherwise a device buffer of
- * mrd_gemm_ln_ws_bytes(M) bytes, zeroed once by the caller, through which the CTAs of a stripe exchange the
- * statistics (plain launch on every SM; only 45 clusters of 3 such CTAs are co-resident on a B200). */
+ * 352-356: BertSelfOutput / BertOutput) in ONE launch: N/256 CTAs own a 128-row stripe and exchange the row
+ * statistics through stats_ws.  N in {512, 768, 1024}, otherwise -1.  residual may be NULL.
+ * stats_ws (required): a device buffer of mrd_gemm_ln_ws_bytes(M) bytes, zeroed once by the caller (the kernel leaves
+ * it zero again); NULL returns -1. */
 int mrd_gemm_ln_bf16(const void* A, long long lda, int M, int K, const void* W, int N, const float* bias, void* C,
                      long long ldc, const void* residual, long long ld_res, const float* gamma, const float* beta,
                      float eps, void* stats_ws, void* stream);

@@ -536,8 +536,6 @@ int plan_conv_chain(ChainLaunch* g, const __nv_bfloat16* X0, int C0, const __nv_
 
     g->smem = chain_smem(C0, C1, Cout, C2, identity != nullptr, &p.stages1, &p.ring);
     p.stages2 = 0;
-    p.lag = 1;
-    p.hints = 0;
     const int sms = gemm_num_sms();
     g->grid = p.m_tiles < sms ? p.m_tiles : sms;
     g->flops = 2.0 * M * (static_cast<double>(Cout) * (C0 + C1) + static_cast<double>(C2) * Cout);
@@ -545,8 +543,6 @@ int plan_conv_chain(ChainLaunch* g, const __nv_bfloat16* X0, int C0, const __nv_
                       1.0 * M * C2 + 1.0 * Cout * (C0 + C1) + 1.0 * C2 * Cout);
     return 0;
 }
-
-void conv_chain_set_tuning(int, int) {}
 
 int launch_conv_chain(const ChainLaunch* g, cudaStream_t stream) {
     if (g->block_n2 == 64) return launch_bn2<64>(g, stream);

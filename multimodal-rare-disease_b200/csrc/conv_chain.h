@@ -33,9 +33,6 @@ struct alignas(64) ChainParams {
     int tiles_w, tiles_h, tiles_img;
     int m_tiles;
     int stages1, stages2, ring;         // operand pipeline depths, residual ring depth (16 KB sub-tiles)
-    int lag;                            // epilogue handles phase 1 of tile j - lag after phase 0 of tile j
-    int hints;                          // bit 0: streaming loads evict_first; bit 1: y stored evict_last;
-                                        // bit 2: the re-read of y evict_first
 };
 
 struct ChainLaunch {
@@ -57,7 +54,5 @@ int plan_conv_chain(ChainLaunch* out, const __nv_bfloat16* X0, int C0, const __n
                     const float* bias1, __nv_bfloat16* Y, const __nv_bfloat16* W2, int C2, const float* bias2,
                     __nv_bfloat16* Z, int out_pad);
 int launch_conv_chain(const ChainLaunch* g, cudaStream_t stream);
-// tuning switches for plans made afterwards (A/B runs): lag in [1, 3], hints bitmask as ChainParams::hints
-void conv_chain_set_tuning(int lag, int hints);
 
 }  // namespace mrd

@@ -77,8 +77,7 @@ struct BertLayerW {
 
 struct CnnPlan {
     int B = 0, H = 0, W = 0;
-    GemmLaunch stem;
-    bool pooled_stem = false;   // stem launch = conv + BN + ReLU + maxpool (plan_stem_pool)
+    GemmLaunch stem;   // conv + BN + ReLU + maxpool in one launch (plan_stem_pool)
     struct BlockPlan {
         GemmLaunch c1, c2, c3, ds;
         bool has_ds = false;
@@ -98,8 +97,8 @@ struct TextPlan {
     int blocked_qkv = 0;  // QKV written as [36][T][64] for the tcgen05 attention (S <= 128)
     struct LayerPlan {
         GemmLaunch qkv, o, f1, f2;
-        GemmLaunch o_ln, f2_ln;   // dense + residual + LayerNorm in one launch (plan_gemm_ln)
-        bool o_fused = false, f2_fused = false;
+        GemmLaunch f2_ln;   // FFN2 + residual + LayerNorm in one launch (plan_gemm_ln)
+        bool f2_fused = false;
     };
     std::vector<LayerPlan> layers;
     // last layer, CLS rows only (M = B): everything after its attention feeds nothing but the CLS row
@@ -116,7 +115,7 @@ struct BatchPlan {
     GemmLaunch ip, tp, i2t, t2i, f1, f2;
     std::vector<GemmLaunch> head;
     bool has_tail = false;   // fusion + head + softmax as ONE launch (tail_fused.h); the launches above stay planned
-    TailLaunch tail;         // for the module-level entry points and as the A/B reference (option "fuse_tail")
+    TailLaunch tail;         // for the module-level entry points (mrd_fusion_fwd, mrd_head_fwd)
 };
 
 }  // namespace
@@ -162,14 +161,6 @@ struct mrd_ctx {
     int fusion_heads = 8;
     int fusion_residual = 1;
     int head_act = MRD_ACT_RELU;
-    int fuse_ds = 1;       // conv3 + downsample of a stage's first bottleneck as one K-concatenated GEMM
-    int fuse_pool = 1;     // MaxPool2d(3,2,1) fused into the stem's epilogue (plan_stem_pool)
-    // BERT: LayerNorm in the epilogue of the dense + residual GEMMs (plan_gemm_ln).  1 = FFN2 only, statistics through
-    // L2 (measured, r02: the two-pass epilogue hides under the K = 3072 main loop, -25 us per launch; under the K = 768
-    // main loop of the attention output it does not: 153 vs 140 us); 2 = both GEMMs, cluster / DSMEM exchange; 0 = off
-    int fuse_ln = 1;
-    int fuse_tail = 1;     // AttentionFusion + ClassificationHead + softmax in one launch (tail_fused_kernel)
-    int fuse_chain = 1;    // bit (L-1): chain conv3(+ds)+add of the blocks of stage L with the next block's conv1
     // fp32 check mode (fp32_check.h): forwards run the plain-fp32 SIMT kernels on the caller's raw fp32
     // tensors; `raw` keeps the name table of the last load_weights (the host keeps the tensors alive)
     TrainState* train = nullptr;   // training step state (engine_train.cuh), created on first use
@@ -691,11 +682,8 @@ int get_cnn_plan(mrd_ctx* c, int B, int H, int W, CnnPlan** out) {
     }
     CnnPlan p;
     p.B = B; p.H = H; p.W = W;
-    if (c->fuse_pool)   // stem + BN + ReLU + maxpool in one launch: the pooled map goes straight to act0
-        MRD_TRY(plan_stem_pool(&p.stem, c->xpad, B, H, W, c->stem_w, c->stem_b, c->act0));
-    else
-        MRD_TRY(plan_stem(&p.stem, c->xpad, B, H, W, c->stem_w, c->stem_b, c->stem_out, ACT_RELU));
-    p.pooled_stem = c->fuse_pool != 0;
+    // stem + BN + ReLU + maxpool in one launch: the pooled map goes straight to act0
+    MRD_TRY(plan_stem_pool(&p.stem, c->xpad, B, H, W, c->stem_w, c->stem_b, c->act0));
     int h = H / 4, w = W / 4;
     const bf16* x = c->act0;  // maxpool output goes to act0
     bf16* bufs[2] = {c->act0, c->act1};
@@ -729,7 +717,7 @@ int get_cnn_plan(mrd_ctx* c, int B, int H, int W, CnnPlan** out) {
         const bf16* identity = x;
         bp.has_ds = b.has_ds;
         bp.fused_ds = false;
-        if (b.has_ds && c->fuse_ds && b.c3ds_w) {
+        if (b.has_ds && b.c3ds_w) {
             // conv3 + downsample + add in one accumulator: the downsample output is never written or re-read
             MRD_TRY(plan_conv1x1_dual(&bp.c3, c->mid1, b.c3.cin, x, b.ds.cin, b.ds.stride, B, ho, wo, b.c3ds_w,
                                       b.c3.cout, b.c3ds_b, y, ACT_RELU));
@@ -743,8 +731,10 @@ int get_cnn_plan(mrd_ctx* c, int B, int H, int W, CnnPlan** out) {
             MRD_TRY(plan_conv(&bp.c3, c->mid1, B, ho, wo, b.c3.cin, b.c3.w, b.c3.cout, b.c3.k, 1,
                               b.c3.b, y, identity, ACT_RELU));
         }
-        // ---- chain this block's tail with the next block's conv1 (same pixels, one launch, y re-read from L2)
-        if (i + 1 < c->blocks.size() && (c->fuse_chain >> (c->block_stage[i] - 1) & 1)) {
+        // ---- chain this block's tail with the next block's conv1 (same pixels, one launch, y re-read from L2).
+        // Layer1 only: for layers 2-4 the weights no longer stay resident and the chain measured slower than the two
+        // launches it replaces (DESIGN.md section 10).
+        if (i + 1 < c->blocks.size() && c->block_stage[i] == 1) {
             const Bottleneck& nx = c->blocks[i + 1];
             const bool dual = b.has_ds && b.c3ds_w != nullptr;
             const bool ok = b.c3.k == 1 && nx.c1.k == 1 && nx.c1.stride == 1 && nx.c1.cin == b.c3.cout &&
@@ -839,23 +829,16 @@ int get_text_plan(mrd_ctx* c, int B, int S, TextPlan** out) {
                           c->t_h2, Hd, nullptr, 0, ACT_NONE));
         // rows are token-packed: the live count is produced on the device by compact_tokens
         lp.qkv.p.dyn_rows = lp.o.p.dyn_rows = lp.f1.p.dyn_rows = lp.f2.p.dyn_rows = c->t_nrows;
-        // dense + residual + LayerNorm as one launch (a cluster of Hd/256 CTAs per 128-token stripe): the
-        // normalised rows go straight to the buffer the separate LayerNorm launch would have written
-        lp.o_fused = lp.f2_fused = false;
-        if (c->fuse_ln) {
-            void* ws = c->fuse_ln == 1 ? c->t_ln_ws : nullptr;
-            int r2 = plan_gemm_ln(&lp.f2_ln, c->t_ffn, c->ffn, T, c->ffn, L.f2.w, Hd, L.f2.b, c->t_h, Hd, c->t_h2, Hd,
-                                  L.ln2g, L.ln2b, c->bert_ln_eps, ws);
-            if (r2 < 0) return r2;
-            lp.f2_fused = r2 == 0;
-            if (c->fuse_ln >= 2) {
-                int r1 = plan_gemm_ln(&lp.o_ln, c->t_ctx, Hd, T, Hd, L.o.w, Hd, L.o.b, c->t_h2, Hd, c->t_h, Hd,
-                                      L.ln1g, L.ln1b, c->bert_ln_eps, ws);
-                if (r1 < 0) return r1;
-                lp.o_fused = r1 == 0;
-            }
-            lp.o_ln.p.dyn_rows = lp.f2_ln.p.dyn_rows = c->t_nrows;
-        }
+        // FFN2 + residual + LayerNorm as one launch (Hd/256 CTAs per 128-token stripe, statistics exchanged through
+        // L2): the normalised rows go straight to the buffer the separate LayerNorm launch would have written.  The
+        // attention output keeps its separate LayerNorm: its two-pass epilogue hides under FFN2's K = 3072 main loop
+        // (-25 us per launch) but not under the K = 768 one (153 vs 140 us, DESIGN.md section 10).  Widths the
+        // kernel does not cover (plan_gemm_ln returns 1) take the GEMM + layernorm_residual launches.
+        int r2 = plan_gemm_ln(&lp.f2_ln, c->t_ffn, c->ffn, T, c->ffn, L.f2.w, Hd, L.f2.b, c->t_h, Hd, c->t_h2, Hd,
+                              L.ln2g, L.ln2b, c->bert_ln_eps, c->t_ln_ws);
+        if (r2 < 0) return r2;
+        lp.f2_fused = r2 == 0;
+        lp.f2_ln.p.dyn_rows = c->t_nrows;
     }
     {
         const BertLayerW& L = c->layers.back();
@@ -865,13 +848,11 @@ int get_text_plan(mrd_ctx* c, int B, int S, TextPlan** out) {
                           c->ffn, nullptr, 0, nullptr, 0, ACT_GELU));
         MRD_TRY(plan_gemm(&p.f2_cls, c->t_cls_ffn, c->ffn, B, c->ffn, L.f2.w, Hd, L.f2.b,
                           c->t_cls_tmp, Hd, c->t_cls_h2, Hd, nullptr, 0, ACT_NONE));
-        if (c->fuse_ln) {
-            // output = this chunk's rows of b_txt: patched at run time (run_bert), planned on a placeholder
-            int r = plan_gemm_ln(&p.f2_cls_ln, c->t_cls_ffn, c->ffn, B, c->ffn, L.f2.w, Hd, L.f2.b, c->t_cls_tmp, Hd,
-                                 c->t_cls_h2, Hd, L.ln2g, L.ln2b, c->bert_ln_eps, c->fuse_ln == 1 ? c->t_ln_ws : nullptr);
-            if (r < 0) return r;
-            p.f2_cls_fused = r == 0;
-        }
+        // output = this chunk's rows of b_txt: patched at run time (run_bert), planned on a placeholder
+        int r = plan_gemm_ln(&p.f2_cls_ln, c->t_cls_ffn, c->ffn, B, c->ffn, L.f2.w, Hd, L.f2.b, c->t_cls_tmp, Hd,
+                             c->t_cls_h2, Hd, L.ln2g, L.ln2b, c->bert_ln_eps, c->t_ln_ws);
+        if (r < 0) return r;
+        p.f2_cls_fused = r == 0;
     }
     auto ins = c->text_plans.emplace(key, std::move(p));
     *out = &ins.first->second;
@@ -969,7 +950,7 @@ int get_batch_plan(mrd_ctx* c, int B, BatchPlan** out) {
         }
         p.has_head = true;
     }
-    if (c->has_fusion && c->has_head && c->fuse_tail && c->tail_residual == c->fusion_residual &&
+    if (c->has_fusion && c->has_head && c->tail_residual == c->fusion_residual &&
         c->fusion_dim == c->head_in && !c->head_hidden.empty() &&
         c->head_hidden.size() <= 3) {
         TailWeights w = {};
@@ -1074,21 +1055,15 @@ int run_backbone(mrd_ctx* c, const void* images, int img_dtype, int B, int H, in
                          1.0 * nb * (3.0 * H * W * esz + (H + 6.0) * (W + 8) * 8));
             MRD_TRY(repack_images(img, img_dtype == MRD_DT_BF16, nb, H, W, c->xpad, s));
         }
-        if (p->pooled_stem) {
+        {
             // the epilogue folds partial window maxima into act0 with red.global.max: start from zero (= the padding
             // value and the identity of the maximum of post-ReLU values)
             const size_t pooled_bytes = static_cast<size_t>(nb) * (H / 4) * (W / 4) * 64 * sizeof(bf16);
-            {
-                ProfScope ps(c, s, "zero_pooled", CAT_MEM, 0, 1.0 * pooled_bytes);
-                cudaError_t e = cudaMemsetAsync(c->act0, 0, pooled_bytes, s);
-                if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(pooled stem output)");
-            }
-            MRD_TRY(run(c, "conv_stem7x7+maxpool", p->stem, s));
-        } else {
-            MRD_TRY(run(c, "conv_stem7x7", p->stem, s));
-            ProfScope ps(c, s, "maxpool3x3s2", CAT_MEM, 0, 1.0 * nb * (H / 2) * (W / 2) * 64 * 2 * 1.25);
-            MRD_TRY(maxpool3x3s2(c->stem_out, nb, H / 2, W / 2, 64, c->act0, s));
+            ProfScope ps(c, s, "zero_pooled", CAT_MEM, 0, 1.0 * pooled_bytes);
+            cudaError_t e = cudaMemsetAsync(c->act0, 0, pooled_bytes, s);
+            if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(pooled stem output)");
         }
+        MRD_TRY(run(c, "conv_stem7x7+maxpool", p->stem, s));
         for (size_t i = 0; i < p->blocks.size(); ++i) {
             auto& bp = p->blocks[i];
             const char* st = kStage[c->block_stage[i]];
@@ -1232,10 +1207,8 @@ int run_bert(mrd_ctx* c, const long long* ids, const void* mask, int mask_dtype,
                 }
                 break;
             }
-            if (lp.o_fused) {
-                MRD_TRY(run(c, "bert.attn_out+res+ln", lp.o_ln, s));
-            } else {
-                MRD_TRY(run(c, "bert.attn_out+res", lp.o, s));
+            MRD_TRY(run(c, "bert.attn_out+res", lp.o, s));
+            {
                 ProfScope ps(c, s, "bert.layernorm", CAT_MEM, 0, ln_bytes);
                 MRD_TRY(layernorm_residual(c->t_tmp, Hd, nullptr, 0, L.ln1g, L.ln1b, c->bert_ln_eps, T,
                                            Hd, c->t_h2, Hd, nullptr, 0, s, c->t_nrows));
@@ -1400,20 +1373,6 @@ int mrd_ctx_set_option(mrd_ctx* c, const char* key, double v) {
     else if (k == "fusion_residual") { c->fusion_residual = v != 0.0; c->batch_plans.clear(); }
     else if (k == "head_act") { c->head_act = static_cast<int>(v); c->batch_plans.clear(); }
     else if (k == "fp32_check") c->fp32_check = v != 0.0;
-    else if (k == "fuse_ds") { c->fuse_ds = v != 0.0; c->cnn_plans.clear(); }
-    else if (k == "fuse_ln") { c->fuse_ln = static_cast<int>(v); c->text_plans.clear(); }
-    else if (k == "fuse_tail") { c->fuse_tail = v != 0.0; c->batch_plans.clear(); }
-    else if (k == "fuse_pool") { c->fuse_pool = v != 0.0; c->cnn_plans.clear(); }
-    else if (k == "fuse_chain") { c->fuse_chain = static_cast<int>(v); c->cnn_plans.clear(); }
-    else if (k == "pair_gemm") {   // process-wide A/B switch; plans are rebuilt
-        gemm_set_pair(static_cast<int>(v));
-        c->cnn_plans.clear(); c->text_plans.clear(); c->batch_plans.clear();
-    }
-    else if (k == "split_epilogue") gemm_set_split_epilogue(static_cast<int>(v));   // process-wide A/B switch
-    else if (k == "chain_tuning") {   // process-wide A/B switch: value = lag * 8 + hints (conv_chain.h)
-        conv_chain_set_tuning(static_cast<int>(v) / 8, static_cast<int>(v) % 8);
-        c->cnn_plans.clear();
-    }
     else if (k == "load_sync") c->load_sync = v != 0.0;
     else if (k.rfind("train.", 0) == 0) return train_set_option(c, k, v);
     else {

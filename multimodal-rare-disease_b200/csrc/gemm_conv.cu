@@ -31,19 +31,15 @@ namespace mrd {
 namespace {
 
 bool g_use_pdl = true;
-int g_pair_gemm = 1;        // flat GEMMs with 256-wide tiles and many stripes: two-CTA clusters sharing the weight tile (PAIR)
-int g_split_epilogue = 3;   // two-group epilogue (EPI2): bit 0 generic-mode launches, bit 1 flat 3x3, bit 2 stem
 
-// Debugging overrides (tools/stress_kernels.py): MRD_DEBUG_SPLIT_EPILOGUE, MRD_DEBUG_PDL, MRD_DEBUG_RING, read once.
+// Debugging overrides (tools/stress_kernels.py): MRD_DEBUG_PDL, MRD_DEBUG_RING, read once.
 int g_debug_ring = -1;
 void apply_debug_env() {
     static bool done = false;
     if (done) return;
     done = true;
-    if (const char* e = getenv("MRD_DEBUG_SPLIT_EPILOGUE")) g_split_epilogue = atoi(e);
     if (const char* e = getenv("MRD_DEBUG_PDL")) g_use_pdl = atoi(e) != 0;
     if (const char* e = getenv("MRD_DEBUG_RING")) g_debug_ring = atoi(e);
-    if (const char* e = getenv("MRD_DEBUG_PAIR")) g_pair_gemm = atoi(e);
 }
 
 constexpr int kBlockM = 128;
@@ -105,15 +101,13 @@ __device__ __forceinline__ TileCoord decode_tile(const ConvGemmParams& p, int ti
 constexpr int kStemRow = 192;    // bytes per patch row (24 pixels x 8 B)
 constexpr int kStemRows = 37;
 
-// LNC: LayerNorm over the whole output row in the epilogue.  The n_tiles_n CTAs of a thread-block cluster work on
-// the same 128-row stripe (tile = blockIdx.x + i * gridDim.x with gridDim.x a multiple of n_tiles_n: the cluster
-// rank IS the column tile).  Epilogue pass 1: accumulator + bias + residual -> per-row partial (mean, M2) of this
-// CTA's columns, the fp32 sums go BACK into TMEM (tcgen05.st); the partials are written into every CTA of the cluster
-// (st.shared::cluster) and counted on an mbarrier there.  Pass 2: combine the partials (Chan), normalise the TMEM
-// values, store.  HF:models/bert/modeling_bert.py:294-298,352-356.
-constexpr int kLnStatBytes = 2 * 128 * 8 * 8;   // two buffers x 128 rows x up to 8 partials x (mean, M2)
-// exchange through L2: one record per 128-row stripe = 128 rows x 8 partials x (mean, M2), then the arrival / departure
-// counters.  The layout does not depend on the row count, so plans of different sizes can share one workspace.
+// LNC: LayerNorm over the whole output row in the epilogue.  The n_tiles_n CTAs that hold the column tiles of one
+// 128-row stripe are neighbours in the persistent tile order.  Epilogue pass 1: accumulator + bias + residual ->
+// per-row partial (mean, M2) of this CTA's columns, the fp32 sums go BACK into TMEM (tcgen05.st); the partials are
+// exchanged through L2 (ln_stats) and counted on the stripe's arrival counter.  Pass 2: combine the partials (Chan),
+// normalise the TMEM values, store.  HF:models/bert/modeling_bert.py:294-298,352-356.
+// One ln_stats record per 128-row stripe = 128 rows x 8 partials x (mean, M2), then the arrival / departure counters.
+// The layout does not depend on the row count, so plans of different sizes can share one workspace.
 constexpr int kLnStripeBytes = 128 * 8 * 8 + 64;
 
 // PAIR (generic mode, flat GEMMs): tcgen05.mma.cta_group::2.  A cluster of two CTAs takes the 128-row stripes 2j and
@@ -202,10 +196,6 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
             mbar_init(tempty_bar(a), (PAIR ? 2 : 1) * (EPI2 ? 4 * (BLOCK_N / 64) : 8));
         }
         mbar_init(bres_bar, 1);
-        if constexpr (LNC) {   // statistics of one stripe have arrived: one arrival per epilogue warp of the cluster
-            mbar_init(bar_smem + 400u, 8u * p.n_tiles_n);
-            mbar_init(bar_smem + 408u, 8u * p.n_tiles_n);
-        }
         fence_mbar_init();
     }
     if (warp == 1) {
@@ -218,9 +208,7 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    if constexpr (LNC || PAIR) {
-        if (PAIR || !p.ln_stats) cluster_sync_all();   // the peers' barriers exist before anyone arrives on them
-    }
+    if constexpr (PAIR) cluster_sync_all();   // the peer's barriers exist before anyone arrives on them
 
     // Programmatic dependent launch: everything above (barrier init, TMEM allocation, descriptor
     // prefetch) overlaps the tail of the previous kernel in the stream; nothing below may touch
@@ -549,7 +537,7 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
             }
         }
     } else if (LNC) {
-        // ------------------------------------------------------------ epilogue with LayerNorm across the cluster
+        // ------------------------------------------------------------ epilogue with LayerNorm across the row's CTAs
         const int quarter = warp & 3;
         const int half = (warp - 2) >> 2;
         const int row = quarter * 32 + lane;
@@ -557,17 +545,13 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
         const bool has_res = p.has_res != 0;
         const int csize = p.n_tiles_n;
         const int npart = 2 * csize;                     // partials per row: (CTA, column half)
-        const bool via_global = p.ln_stats != nullptr;
-        const uint32_t crank = via_global ? 0u : cluster_ctarank();
-        const uint32_t stats_smem = bar_smem + kBarBytes;
-        const float2* stats_gen = reinterpret_cast<const float2*>(smem_gen + (stats_smem - smem_base));
         constexpr float kPartN = static_cast<float>(NSUB * 32);   // columns behind one partial
         const float inv_n = 1.0f / (static_cast<float>(csize) * BLOCK_N);
         int rslot = 0;
         uint32_t rphase = 0;
         int q = 0;
         for (int it = 0; it < my_tiles; ++it) {
-            const int acc = it & 1, sb = it & 1;
+            const int acc = it & 1;
             const TileCoord t = decode_tile(p, tile_at(it));
             const uint32_t tbase =
                 tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + acc * BLOCK_N + half * 32;
@@ -622,48 +606,35 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
             // ---- publish (mean, M2) of these kPartN columns to the CTAs that hold the rest of the row
             const float mean_p = sum * (1.0f / kPartN);
             const float m2_p = fmaxf(ssq - sum * mean_p, 0.0f);
+            // through L2: the csize CTAs of a stripe are neighbours in the persistent tile order, so all of them are
+            // resident (grid <= SM count) and a spin on the stripe's arrival counter cannot deadlock
             float2 part[8];
-            if (!via_global) {
-                const uint32_t slot_addr =
-                    stats_smem + static_cast<uint32_t>(((sb * 128 + row) * 8 + static_cast<int>(crank) * 2 + half) * 8);
-                for (int r = 0; r < csize; ++r) st_cluster_f32x2(mapa_shared(slot_addr, r), mean_p, m2_p);
-                fence_acq_rel_cluster();
-                __syncwarp();
-                if (lane == 0)
-                    for (int r = 0; r < csize; ++r) mbar_arrive_cluster(mapa_shared(bar_smem + 400u + 8u * sb, r));
-                mbar_wait_cluster(bar_smem + 400u + 8u * sb, (it >> 1) & 1u);
-                const float2* pr = stats_gen + (sb * 128 + row) * 8;
-                for (int i = 0; i < npart; ++i) part[i] = pr[i];
-            } else {
-                // through L2: the csize CTAs of a stripe are neighbours in the persistent tile order, so all of them
-                // are resident (grid <= SM count) and a spin on the stripe's arrival counter cannot deadlock
-                const int stripe = tile_at(it) / csize;
-                char* rec = reinterpret_cast<char*>(p.ln_stats) + static_cast<long long>(stripe) * kLnStripeBytes;
-                float2* srow = reinterpret_cast<float2*>(rec) + row * 8;
-                __stcg(srow + t.n_idx * 2 + half, make_float2(mean_p, m2_p));
-                __threadfence();
-                __syncwarp();
-                unsigned int* cnt = reinterpret_cast<unsigned int*>(rec + 128 * 8 * 8);
-                const unsigned int want = 8u * csize;
-                if (lane == 0) {
-                    asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(cnt) : "memory");
-                    unsigned int seen;
-                    const long long t0 = clock64();
-                    do {
-                        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(cnt) : "memory");
-                        if (clock64() - t0 > 4000000000LL) __trap();
-                    } while (seen < want);
-                }
-                __syncwarp();
-                for (int i = 0; i < npart; ++i) part[i] = __ldcg(srow + i);
-                __syncwarp();
-                if (lane == 0) {   // the last warp to have read the stripe's partials re-arms both counters
-                    unsigned int left;
-                    asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], 1;" : "=r"(left) : "l"(cnt + 1) : "memory");
-                    if (left == want - 1) {
-                        cnt[1] = 0;
-                        asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(cnt), "r"(0u) : "memory");
-                    }
+            const int stripe = tile_at(it) / csize;
+            char* rec = reinterpret_cast<char*>(p.ln_stats) + static_cast<long long>(stripe) * kLnStripeBytes;
+            float2* srow = reinterpret_cast<float2*>(rec) + row * 8;
+            __stcg(srow + t.n_idx * 2 + half, make_float2(mean_p, m2_p));
+            __threadfence();
+            __syncwarp();
+            unsigned int* cnt = reinterpret_cast<unsigned int*>(rec + 128 * 8 * 8);
+            const unsigned int want = 8u * csize;
+            if (lane == 0) {
+                asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(cnt) : "memory");
+                unsigned int seen;
+                const long long t0 = clock64();
+                do {
+                    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(cnt) : "memory");
+                    if (clock64() - t0 > 4000000000LL) __trap();
+                } while (seen < want);
+            }
+            __syncwarp();
+            for (int i = 0; i < npart; ++i) part[i] = __ldcg(srow + i);
+            __syncwarp();
+            if (lane == 0) {   // the last warp to have read the stripe's partials re-arms both counters
+                unsigned int left;
+                asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], 1;" : "=r"(left) : "l"(cnt + 1) : "memory");
+                if (left == want - 1) {
+                    cnt[1] = 0;
+                    asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(cnt), "r"(0u) : "memory");
                 }
             }
             float mean = 0.0f;
@@ -997,10 +968,7 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
 
     tc_fence_before();
     __syncthreads();
-    if constexpr (LNC || PAIR) {
-        // no CTA leaves while a peer may still write its statistics buffer / arrive on its barriers
-        if (PAIR || !p.ln_stats) cluster_sync_all();
-    }
+    if constexpr (PAIR) cluster_sync_all();   // no CTA leaves while its peer may still arrive on its barriers
     if (warp == 1) {
         tc_fence_after();
         if constexpr (PAIR)
@@ -1011,7 +979,7 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
 }
 
 template <int BLOCK_N, int MODE, bool SPLITK = false, bool EPI2 = false, bool LNC = false, bool PAIR = false>
-int launch_variant(const GemmLaunch* g, cudaStream_t stream, int sm_limit) {
+int launch_variant(const GemmLaunch* g, cudaStream_t stream) {
     using C = Cfg<BLOCK_N, MODE>;
     static bool attr_set = false;
     auto kfn = conv_gemm_kernel<BLOCK_N, MODE, SPLITK, EPI2, LNC, PAIR>;
@@ -1027,40 +995,27 @@ int launch_variant(const GemmLaunch* g, cudaStream_t stream, int sm_limit) {
     const int smem = MODE != MODE_GENERIC
                          ? C::FIXED + g->p.stages * g->p.a_stage_bytes + g->p.b_res_bytes
                          : C::FIXED + g->p.stages * (PAIR ? C::A_STAGE + C::B_STAGE / 2 : C::STAGE) +
-                               g->p.ring * kStageBufBytes + (LNC ? kLnStatBytes : 0);
+                               g->p.ring * kStageBufBytes;
     cudaLaunchConfig_t cfg = {};
-    int grid = g->grid;
-    if (sm_limit > 0 && grid > sm_limit) {
-        // the kernel is persistent (tiles strided by gridDim): a smaller grid leaves SMs to a kernel of another
-        // stream.  Weights-resident modes need a multiple of n_tiles_n CTAs.
-        grid = sm_limit;
-        if (MODE != MODE_GENERIC) {
-            grid = grid / g->p.n_tiles_n * g->p.n_tiles_n;
-            if (grid < g->p.n_tiles_n) grid = g->p.n_tiles_n;
-        }
-    }
-    cfg.gridDim = dim3(grid);
+    cfg.gridDim = dim3(g->grid);
     cfg.blockDim = dim3(kNumThreads);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = stream;
     cudaLaunchAttribute attr[2];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    // no programmatic dependent launch under an SM cap: the early-launched CTAs of the next kernel would sit on
-    // the SMs that the cap leaves to the other stream
-    attr[0].val.programmaticStreamSerializationAllowed = (g_use_pdl && sm_limit <= 0) ? 1 : 0;
+    attr[0].val.programmaticStreamSerializationAllowed = g_use_pdl ? 1 : 0;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if (PAIR || (LNC && !g->p.ln_stats)) {
-        // LNC: one cluster = the n_tiles_n column tiles of a 128-row stripe; PAIR: two stripes of one column tile.
-        // As many clusters as are co-resident.
-        const int cs = PAIR ? 2 : g->p.n_tiles_n;
+    if (PAIR) {
+        // one cluster = two stripes of one column tile; as many clusters as are co-resident
+        constexpr int cs = 2;
         attr[1].id = cudaLaunchAttributeClusterDimension;
         attr[1].val.clusterDim.x = cs;
         attr[1].val.clusterDim.y = 1;
         attr[1].val.clusterDim.z = 1;
         cfg.numAttrs = 2;
-        static int max_clusters[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-        if (max_clusters[cs] == 0) {
+        static int max_clusters = 0;
+        if (max_clusters == 0) {
             cfg.gridDim = dim3(cs * 16);
             int n = 0;
             cudaError_t e = cudaOccupancyMaxActiveClusters(&n, kfn, &cfg);
@@ -1068,13 +1023,13 @@ int launch_variant(const GemmLaunch* g, cudaStream_t stream, int sm_limit) {
                 set_last_error("cudaOccupancyMaxActiveClusters(cluster of %d): %s", cs, cudaGetErrorString(e));
                 return e != cudaSuccess ? -static_cast<int>(e) : -1;
             }
-            max_clusters[cs] = n;
+            max_clusters = n;
             if (getenv("MRD_DEBUG_PRINT"))
                 fprintf(stderr, "[mrd] conv_gemm_kernel<%d,%d,%d,%d,%d,%d>: %d co-resident clusters of %d CTAs\n", BLOCK_N,
                         MODE, SPLITK, EPI2, LNC, PAIR, n, cs);
         }
-        int clusters = grid / cs;
-        if (clusters > max_clusters[cs]) clusters = max_clusters[cs];
+        int clusters = g->grid / cs;
+        if (clusters > max_clusters) clusters = max_clusters;
         if (clusters < 1) clusters = 1;
         cfg.gridDim = dim3(clusters * cs);
     }
@@ -1166,8 +1121,6 @@ int finish_plan(GemmLaunch* g, int block_n) {
 }  // namespace
 
 void gemm_set_pdl(bool on) { g_use_pdl = on; }
-void gemm_set_split_epilogue(int mask) { g_split_epilogue = mask; }
-void gemm_set_pair(int on) { g_pair_gemm = on; }
 
 int gemm_num_sms() {
     static int sms = 0;
@@ -1226,9 +1179,8 @@ int plan_gemm_impl(GemmLaunch* g, const __nv_bfloat16* A, long long lda, int M, 
                (out_f32 ? 4.0 * M * N : 0.0);
 
     const int bn = force_bn ? force_bn : pick_block_n(N, p.tiles_w, gemm_num_sms());
-    apply_debug_env();
     // at least two tiles per SM: below that the pairing has nothing to amortise
-    g->pair = (g_pair_gemm && bn == 256 && static_cast<long long>(p.tiles_w) * (N / 256) >= 2LL * gemm_num_sms()) ? 1 : 0;
+    g->pair = (bn == 256 && static_cast<long long>(p.tiles_w) * (N / 256) >= 2LL * gemm_num_sms()) ? 1 : 0;
     {
         uint64_t dims[4] = {(uint64_t)K, (uint64_t)M, 1, 1};
         uint64_t str[3] = {(uint64_t)lda * 2, (uint64_t)lda * 2 * M, (uint64_t)lda * 2 * M};
@@ -1281,36 +1233,25 @@ int plan_gemm_ln(GemmLaunch* g, const __nv_bfloat16* A, long long lda, int M, in
                  const float* bias, __nv_bfloat16* Cout, long long ldc, const __nv_bfloat16* residual,
                  long long ld_res, const float* gamma, const float* beta, float eps, void* stats_ws) {
     if (N % 256 != 0 || N / 256 < 2 || N / 256 > 4 || !Cout || !bias || !gamma || !beta) return 1;
+    if (!stats_ws) {
+        set_last_error("gemm + LayerNorm: stats_ws is required (a zeroed device buffer of mrd_gemm_ln_ws_bytes(M) bytes)");
+        return -1;
+    }
     // always 256-wide tiles, however few rows there are: which kernel (and so which rounding) a row goes through
     // must not depend on the batch it arrives in - sub-batches reproduce the rows of the full batch bit for bit
     MRD_GEMM_TRY(plan_gemm_impl(g, A, lda, M, K, W, N, bias, Cout, ldc, residual, ld_res, nullptr, 0, ACT_NONE, 0, 256));
     ConvGemmParams& p = g->p;
-    if (g->pair && !stats_ws) {   // the cluster is taken by the statistics exchange: whole weight tiles per CTA
-        g->pair = 0;
-        uint64_t dims[2] = {(uint64_t)K, (uint64_t)N};
-        uint64_t str[1] = {(uint64_t)K * 2};
-        uint32_t box[2] = {64, 256};
-        int rc = encode_tensor_map(&p.b_map, W, 2, 2, dims, str, box, 128);
-        if (rc) return rc;
-    }
     p.ln_g = gamma;
     p.ln_b = beta;
     p.ln_eps = eps;
+    p.ln_stats = static_cast<float2*>(stats_ws);   // records of kLnStripeBytes
     g->lnc = 1;
-    // room for the statistics buffers: three operand stages (four of the pair's smaller ones), two residual
-    // sub-tiles in flight
+    // three operand stages (four of the pair's smaller ones), two residual sub-tiles in flight
     if (p.has_res) {
         p.stages = g->pair ? 4 : 3;
         p.ring = 2;
     } else if (p.stages > (g->pair ? 5 : 3)) {
         p.stages = g->pair ? 5 : 3;
-    }
-    const int cs = p.n_tiles_n;
-    if (stats_ws) {
-        p.ln_stats = static_cast<float2*>(stats_ws);   // records of kLnStripeBytes
-    } else {
-        g->grid = g->grid / cs * cs;
-        if (g->grid < cs) g->grid = cs;
     }
     g->bytes += 8.0 * N;   // gamma / beta
     return 0;
@@ -1440,10 +1381,9 @@ int plan_conv(GemmLaunch* g, const __nv_bfloat16* X, int N, int H, int W, int Ci
     }
     const long long m_tiles = static_cast<long long>(p.tiles_w) * p.tiles_h * p.tiles_img;
     const int bn = pick_block_n(Cout, m_tiles, gemm_num_sms());
-    apply_debug_env();
     // CTA pairs (cta_group::2) for the tensor-bound 3x3 / strided convolutions of layers 3 and 4 as well: two tiles of
     // 128 output pixels share each weight block
-    g->pair = (g_pair_gemm && bn == 256 && m_tiles * (Cout / 256) >= 2LL * gemm_num_sms()) ? 1 : 0;
+    g->pair = (bn == 256 && m_tiles * (Cout / 256) >= 2LL * gemm_num_sms()) ? 1 : 0;
     {
         const uint64_t Kt = static_cast<uint64_t>(Cin) * ksize * ksize;
         uint64_t dims[2] = {Kt, (uint64_t)Cout};
@@ -1610,9 +1550,8 @@ int plan_conv3x3_flat(GemmLaunch* g, const __nv_bfloat16* Xpad, int N, int H, in
     // 4.70 -> 2.2-2.7 ms per 4096 images).  A 64-channel layer gains too (layer1 conv2: 4.4 -> 3.7 ms): a
     // 256 x 64 x 16 pair instruction takes ~45-58 cycles against 62 for 128 x 64 x 16 on one SM
     // (tools/exp_pair_rate.cu).  One column tile only (the resident panel fixes a CTA's column tile).
-    apply_debug_env();
     const long long flat_tiles = static_cast<long long>((H + th - 1) / th) * N;
-    if (g_pair_gemm && bn == 64 && (Cout == 128 || Cout == 64) &&
+    if (bn == 64 && (Cout == 128 || Cout == 64) &&
         flat_tiles >= 2LL * gemm_num_sms() && fixed + 2 * a_stage + 9 * (Cin / 64) * (Cout / 2) * 128 <= kSmemLimit) {
         g->pair = 1;
         bn = Cout;
@@ -1751,38 +1690,32 @@ int plan_stem_pool(GemmLaunch* g, const __nv_bfloat16* Xpad, int N, int H, int W
     return 0;
 }
 
-int launch_gemm(const GemmLaunch* g, cudaStream_t stream, int sm_limit) {
+int launch_gemm(const GemmLaunch* g, cudaStream_t stream) {
     apply_debug_env();
     if (g->stem) {
         // the fused pooling lives in the two-group epilogue
-        if ((g_split_epilogue & 4) || g->p.pool_out) return launch_variant<64, MODE_STEM, false, true>(g, stream, sm_limit);
-        return launch_variant<64, MODE_STEM>(g, stream, sm_limit);
+        if (g->p.pool_out) return launch_variant<64, MODE_STEM, false, true>(g, stream);
+        return launch_variant<64, MODE_STEM>(g, stream);
     }
     if (g->lnc)
-        return g->pair ? launch_variant<256, MODE_GENERIC, false, false, true, true>(g, stream, sm_limit)
-                       : launch_variant<256, MODE_GENERIC, false, false, true>(g, stream, sm_limit);
+        return g->pair ? launch_variant<256, MODE_GENERIC, false, false, true, true>(g, stream)
+                       : launch_variant<256, MODE_GENERIC, false, false, true>(g, stream);
     if (g->flat3 && g->pair)
-        return g->block_n == 128 ? launch_variant<128, MODE_FLAT3, false, true, false, true>(g, stream, sm_limit)
-                                 : launch_variant<64, MODE_FLAT3, false, true, false, true>(g, stream, sm_limit);
-    if (g->flat3 && (g_split_epilogue & 2)) {
-        switch (g->block_n) {
-            case 64: return launch_variant<64, MODE_FLAT3, false, true>(g, stream, sm_limit);
-            case 128: return launch_variant<128, MODE_FLAT3, false, true>(g, stream, sm_limit);
-        }
-    }
+        return g->block_n == 128 ? launch_variant<128, MODE_FLAT3, false, true, false, true>(g, stream)
+                                 : launch_variant<64, MODE_FLAT3, false, true, false, true>(g, stream);
     if (g->flat3) {
         switch (g->block_n) {
-            case 64: return launch_variant<64, MODE_FLAT3>(g, stream, sm_limit);
-            case 128: return launch_variant<128, MODE_FLAT3>(g, stream, sm_limit);
+            case 64: return launch_variant<64, MODE_FLAT3, false, true>(g, stream);
+            case 128: return launch_variant<128, MODE_FLAT3, false, true>(g, stream);
         }
         set_last_error("launch_gemm: bad flat3 block_n %d", g->block_n);
         return -1;
     }
     if (g->p.f32_accum) {   // plan_gemm_splitk
         switch (g->block_n) {
-            case 64: return launch_variant<64, MODE_GENERIC, true>(g, stream, sm_limit);
-            case 128: return launch_variant<128, MODE_GENERIC, true>(g, stream, sm_limit);
-            case 256: return launch_variant<256, MODE_GENERIC, true>(g, stream, sm_limit);
+            case 64: return launch_variant<64, MODE_GENERIC, true>(g, stream);
+            case 128: return launch_variant<128, MODE_GENERIC, true>(g, stream);
+            case 256: return launch_variant<256, MODE_GENERIC, true>(g, stream);
         }
     }
     // Two-group epilogue where the per-sub-tile latency chain bounds the launch (measured, r02: GELU epilogue -5 %,
@@ -1790,22 +1723,22 @@ int launch_gemm(const GemmLaunch* g, cudaStream_t stream, int sm_limit) {
     // single-group epilogue with its two shared staging buffers (QKV lost 5 % with the split).
     const bool chain_bound = g->p.act == ACT_GELU || g->p.num_taps * g->p.kc_per_tap <= 6 ||
                              (g->p.kc_split && g->p.num_k_total <= 6);
-    const bool epi2 = (g_split_epilogue & 1) && chain_bound && !(g->p.kc_split && g->p.num_k_total > 6);
+    const bool epi2 = chain_bound && !(g->p.kc_split && g->p.num_k_total > 6);
     if (g->pair && g->block_n == 256) {
-        if (epi2 || (g_split_epilogue & 8)) return launch_variant<256, MODE_GENERIC, false, true, false, true>(g, stream, sm_limit);
-        return launch_variant<256, MODE_GENERIC, false, false, false, true>(g, stream, sm_limit);
+        if (epi2) return launch_variant<256, MODE_GENERIC, false, true, false, true>(g, stream);
+        return launch_variant<256, MODE_GENERIC, false, false, false, true>(g, stream);
     }
     if (epi2) {
         switch (g->block_n) {
-            case 64: return launch_variant<64, MODE_GENERIC, false, true>(g, stream, sm_limit);
-            case 128: return launch_variant<128, MODE_GENERIC, false, true>(g, stream, sm_limit);
-            case 256: return launch_variant<256, MODE_GENERIC, false, true>(g, stream, sm_limit);
+            case 64: return launch_variant<64, MODE_GENERIC, false, true>(g, stream);
+            case 128: return launch_variant<128, MODE_GENERIC, false, true>(g, stream);
+            case 256: return launch_variant<256, MODE_GENERIC, false, true>(g, stream);
         }
     }
     switch (g->block_n) {
-        case 64: return launch_variant<64, MODE_GENERIC>(g, stream, sm_limit);
-        case 128: return launch_variant<128, MODE_GENERIC>(g, stream, sm_limit);
-        case 256: return launch_variant<256, MODE_GENERIC>(g, stream, sm_limit);
+        case 64: return launch_variant<64, MODE_GENERIC>(g, stream);
+        case 128: return launch_variant<128, MODE_GENERIC>(g, stream);
+        case 256: return launch_variant<256, MODE_GENERIC>(g, stream);
     }
     set_last_error("launch_gemm: bad block_n %d", g->block_n);
     return -1;

@@ -64,15 +64,14 @@ struct alignas(64) ConvGemmParams {
     // >= 0, so 0 is the identity of the max and doubles as the padding value).
     __nv_bfloat16* pool_out;
     int pool_h, pool_w;
-    // LayerNorm in the epilogue (plan_gemm_ln): the n_tiles_n CTAs of a thread-block cluster hold one 128-row stripe
-    // of the whole output row between them, exchange per-row partial statistics through distributed shared memory
-    // and store LayerNorm(A W^T + bias + residual) * ln_g + ln_b.
+    // LayerNorm in the epilogue (plan_gemm_ln): the n_tiles_n CTAs that hold one 128-row stripe of the whole output
+    // row between them exchange per-row partial statistics through global memory (ln_stats) and store
+    // LayerNorm(A W^T + bias + residual) * ln_g + ln_b.
     const float* ln_g;
     const float* ln_b;
     float ln_eps;
-    // ln_stats != null: the statistics are exchanged through global memory instead (no cluster launch, every SM
-    // usable): one record per 128-row stripe = [128][8] (mean, M2) partials + arrival / departure counters (zero
-    // between launches: the last warp to leave a stripe resets them).
+    // one record per 128-row stripe = [128][8] (mean, M2) partials + arrival / departure counters (zero between
+    // launches: the last warp to leave a stripe resets them)
     float2* ln_stats;
 };
 
@@ -81,7 +80,7 @@ struct GemmLaunch {
     int block_n;  // 64, 128 or 256
     int stem;     // 1: 5-D overlapping-window A map, BLOCK_K = 32
     int flat3;    // 1: flat-shift 3x3 stride-1 mode (halo span in smem, taps = row-shifted views)
-    int lnc;      // 1: LayerNorm epilogue across a cluster of n_tiles_n CTAs (plan_gemm_ln)
+    int lnc;      // 1: LayerNorm epilogue across the n_tiles_n CTAs of a stripe (plan_gemm_ln)
     int pair;     // 1: two-CTA clusters sharing each weight tile by TMA multicast (b_map's box is half a tile)
     int grid;
     double flops;  // algorithmic FLOPs (2*M*N*K, un-padded), for reporting
@@ -101,13 +100,12 @@ int plan_gemm(GemmLaunch* out, const __nv_bfloat16* A, long long lda, int M, int
 // HF:models/bert/modeling_bert.py:294-298,352-356 (dense -> dropout -> LayerNorm(x + input)) as ONE launch.
 // N = c * 256 with c in [2, 4] (BERT-base: 3): c CTAs own a 128-row stripe.  Returns 1 (no error message) when N
 // is outside that range - the caller then plans the GEMM and a LayerNorm launch.
-// stats_ws (optional, device, gemm_ln_ws_bytes(M) bytes, zeroed once by the caller): exchange the statistics through
-// global memory - a plain launch on every SM (on B200 only 45 clusters of 3 CTAs with 227 KB of shared memory are
-// co-resident = 135 of 148 SMs); null: thread-block cluster + distributed shared memory.
+// stats_ws (required, device, gemm_ln_ws_bytes(M) bytes, zeroed once by the caller): the CTAs of a stripe exchange
+// the statistics through it in global memory.  Null returns -1.
 size_t gemm_ln_ws_bytes(int M);
 int plan_gemm_ln(GemmLaunch* out, const __nv_bfloat16* A, long long lda, int M, int K, const __nv_bfloat16* W, int N,
                  const float* bias, __nv_bfloat16* C, long long ldc, const __nv_bfloat16* residual, long long ld_res,
-                 const float* gamma, const float* beta, float eps, void* stats_ws = nullptr);
+                 const float* gamma, const float* beta, float eps, void* stats_ws);
 
 // ksize in {1,3}, stride in {1,2}, padding = ksize/2.  X: [N,H,W,Cin] bf16, Wt: [Cout][k][k][Cin]
 // bf16 (BN already folded), Y: [N,H/stride,W/stride,Cout] bf16.  Cin % 64 == 0, Cout % 64 == 0.
@@ -149,19 +147,12 @@ int plan_stem_pool(GemmLaunch* out, const __nv_bfloat16* Xpad, int N, int H, int
 int plan_gemm_splitk(GemmLaunch* out, const __nv_bfloat16* A, long long lda, int M, int K,
                      const __nv_bfloat16* W, int N, float* out_f32, long long ld_f32, const int* dyn_k);
 
-// sm_limit > 0 caps the grid (the kernel is persistent, so any grid size covers all tiles).  Used by the
-// branch-overlap experiment (ResNet and BERT side by side on disjoint SM sets, DESIGN.md section 5: slower,
-// not shipped); kept because it costs nothing.
-int launch_gemm(const GemmLaunch* g, cudaStream_t stream, int sm_limit = 0);
+int launch_gemm(const GemmLaunch* g, cudaStream_t stream);
 
 int gemm_num_sms();
 
 // Programmatic dependent launch for the GEMM/conv kernels (on by default; the engine turns it off
 // while profiling so that per-launch event timings do not overlap).
 void gemm_set_pdl(bool on);
-// Two-group epilogue (process-wide A/B switch): bit 0 generic-mode launches, bit 1 flat 3x3, bit 2 stem.
-void gemm_set_split_epilogue(int mask);
-// process-wide A/B switch for plans made afterwards: pair the 128-row stripes of large flat GEMMs (PAIR)
-void gemm_set_pair(int on);
 
 }  // namespace mrd

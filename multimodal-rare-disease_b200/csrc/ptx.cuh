@@ -300,12 +300,6 @@ __device__ __forceinline__ uint32_t mapa_shared(uint32_t addr, uint32_t rank) {
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
     return r;
 }
-__device__ __forceinline__ void st_cluster_f32x2(uint32_t cluster_addr, float a, float b) {
-    asm volatile("st.shared::cluster.v2.f32 [%0], {%1, %2};" ::"r"(cluster_addr), "f"(a), "f"(b) : "memory");
-}
-__device__ __forceinline__ void fence_acq_rel_cluster() {
-    asm volatile("fence.acq_rel.cluster;" ::: "memory");
-}
 // TMA load delivered to the same shared-memory offset (and counted on the same mbarrier offset) of every CTA of the
 // cluster whose bit is set in cta_mask
 __device__ __forceinline__ void tma_load_2d_multicast(const void* map, uint32_t bar, uint32_t dst, int c0, int c1,
@@ -323,31 +317,12 @@ __device__ __forceinline__ void umma_commit_multicast(uint32_t bar, uint16_t cta
         "h"(cta_mask)
         : "memory");
 }
-// arrive on an mbarrier of another CTA of the cluster (address from mapa_shared), release at cluster scope
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_bar) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar) : "memory");
-}
-// the same with the default (CTA-scope release) ordering: for barriers that only pace hardware-tracked work - a TMA
-// landing, accumulator columns drained with tcgen05.ld - and publish no data written by ordinary stores.  (The
-// cluster-scope release above costs the arriving thread on the order of a thousand cycles per call.)
+// arrive on an mbarrier of another CTA of the cluster (address from mapa_shared) with the default (CTA-scope release)
+// ordering: for barriers that only pace hardware-tracked work - a TMA landing, accumulator columns drained with
+// tcgen05.ld - and publish no data written by ordinary stores.  (A cluster-scope release costs the arriving thread on
+// the order of a thousand cycles per call.)
 __device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_bar) {
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar) : "memory");
-}
-// wait on a local mbarrier whose arrivals come from other CTAs: acquire at cluster scope
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
-    uint32_t ok = 0;
-    const long long t0 = clock64();
-    while (true) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.b32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"(bar), "r"(parity)
-            : "memory");
-        if (ok) return;
-        if (clock64() - t0 > 4000000000LL) __trap();
-    }
 }
 
 // ------------------------------------------------------------------ descriptors

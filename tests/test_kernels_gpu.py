@@ -71,19 +71,24 @@ def test_gemm(lib, cuda, M, N, K, act, res, f32):
         _close(C32, ref, rel=1e-4, abs_=2e-3, what="gemm f32 out")
 
 
-@pytest.mark.parametrize("via_global", [False, True])
 @pytest.mark.parametrize("M,N,K,res", [
-    (5, 768, 3072, True),         # a handful of rows: the same kernel (the path must not depend on the batch size)
+    # CTA pairs (at least two 256-wide tiles per SM on a 148-SM B200)
     (19000, 768, 768, True),      # BertSelfOutput: dense + residual + LayerNorm, ragged last stripe
     (19000, 768, 3072, True),     # BertOutput, long K
-    (20480, 1024, 256, False),    # cluster of four, no residual
-    (40000, 512, 128, True),      # cluster of two, more stripes than clusters
+    (12800, 768, 3072, True),     # whole stripes only
+    (20480, 1024, 256, False),    # four CTAs per stripe, no residual
+    (40000, 512, 128, True),      # two CTAs per stripe, several stripes per CTA pair
+    # single CTAs
+    (5, 768, 3072, True),         # a handful of rows: the same kernel (the path must not depend on the batch size)
+    (300, 768, 3072, True),       # a few stripes, ragged
+    (12000, 768, 768, True),      # more tiles than SMs: a stripe's CTAs are at different iterations
+    (4096, 1024, 768, True),      # four CTAs per stripe
+    (9000, 512, 768, False),      # two CTAs per stripe, no residual
 ])
-def test_gemm_layernorm(lib, cuda, M, N, K, res, via_global):
+def test_gemm_layernorm(lib, cuda, M, N, K, res):
     """GEMM with LayerNorm over the whole row in the epilogue against fp32 torch: layer_norm(A W^T + b + R).  The
-    N/256 CTAs of a 128-row stripe exchange their partial statistics through distributed shared memory (cluster
-    launch) or, with a workspace, through global memory (plain launch on every SM)."""
-    ws = torch.zeros(lib.mrd_gemm_ln_ws_bytes(M), device=cuda, dtype=torch.uint8) if via_global else None
+    N/256 CTAs of a 128-row stripe exchange their partial statistics through the workspace in global memory."""
+    ws = torch.zeros(lib.mrd_gemm_ln_ws_bytes(M), device=cuda, dtype=torch.uint8)
     g = torch.Generator(device="cuda").manual_seed(M + N + K)
     A = torch.randn(M, K, device=cuda, generator=g).to(BF)
     W = (torch.randn(N, K, device=cuda, generator=g) / math.sqrt(K)).to(BF)
@@ -99,7 +104,7 @@ def test_gemm_layernorm(lib, cuda, M, N, K, res, via_global):
         C.fill_(float("nan"))
         _check(lib, lib.mrd_gemm_ln_bf16(A.data_ptr(), K, M, K, W.data_ptr(), N, bias.data_ptr(), C.data_ptr(), N,
                                          R.data_ptr() if res else None, N, gamma.data_ptr(), beta.data_ptr(), 1e-12,
-                                         ws.data_ptr() if via_global else None, _stream()))
+                                         ws.data_ptr(), _stream()))
         torch.cuda.synchronize()
         outs.append(C.clone())
     x = A.float() @ W.float().t() + bias
@@ -108,9 +113,9 @@ def test_gemm_layernorm(lib, cuda, M, N, K, res, via_global):
     ref = F.layer_norm(x, (N,), gamma, beta, 1e-12)
     _close(C, ref, what=f"gemm + layernorm {M}x{N}x{K}")
     assert torch.equal(outs[0], outs[1]) and torch.equal(outs[0], outs[2]), "run-to-run difference"
-    if via_global:   # the arrival / departure counters re-arm themselves
-        rec = ws.view(-1, 128 * 8 * 8 + 64)
-        assert int(rec[:, 128 * 8 * 8:].contiguous().view(torch.int32).abs().sum()) == 0
+    # the arrival / departure counters re-arm themselves
+    rec = ws.view(-1, 128 * 8 * 8 + 64)
+    assert int(rec[:, 128 * 8 * 8:].contiguous().view(torch.int32).abs().sum()) == 0
 
 
 def test_gemm_layernorm_rejects_other_widths(lib, cuda):
@@ -119,6 +124,10 @@ def test_gemm_layernorm_rejects_other_widths(lib, cuda):
     rc = lib.mrd_gemm_ln_bf16(A.data_ptr(), 768, 256, 768, A.data_ptr(), 640, v.data_ptr(), A.data_ptr(), 640, None, 0,
                               v.data_ptr(), v.data_ptr(), 1e-12, None, _stream())
     assert rc != 0 and b"outside" in lib.mrd_last_error()
+    # a supported width without the statistics workspace
+    rc = lib.mrd_gemm_ln_bf16(A.data_ptr(), 768, 256, 768, A.data_ptr(), 768, v.data_ptr(), A.data_ptr(), 768, None, 0,
+                              v.data_ptr(), v.data_ptr(), 1e-12, None, _stream())
+    assert rc == -1 and b"mrd_gemm_ln_ws_bytes" in lib.mrd_last_error()
 
 
 def test_gemm_strided(lib, cuda):

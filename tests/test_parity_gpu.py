@@ -150,9 +150,10 @@ def test_fusion_and_head_vs_oracle(cuda, state):
     assert torch.equal(info["image_to_text_attention"].cpu(), torch.ones(5, 8, 1, 1))
 
 
-def test_fused_tail_vs_oracle(cuda, state):
+def test_fused_tail_vs_oracle_and_per_layer(cuda, state):
     """K6 as ONE launch (tail_fused_kernel through mrd_fusion_head_fwd): fusion + head + softmax on fp32
-    embeddings, against the fixture of the unmodified reference, the oracle, and the per-layer launches."""
+    embeddings, against the fixture of the unmodified reference, the oracle, and the per-layer launches of
+    mrd_fusion_fwd + mrd_head_fwd on the same rows."""
     fix = torch.load(os.path.join(GOLD, "padded_sens_b5_s128.pt"))
     model = _use(state, "sens")
     sd = {k: v.float() for k, v in state["sens"].items() if v.is_floating_point()}
@@ -181,14 +182,15 @@ def test_fused_tail_vs_oracle(cuda, state):
     _logits_ok(logits, ref_logits)
     assert (logits.argmax(-1).cpu() == ref_logits.argmax(-1)).float().mean().item() >= 0.99
     assert torch.allclose(probs.sum(-1).cpu(), torch.ones(203), atol=1e-5)
-    eng.set_option("fuse_tail", 0.0)
-    try:
-        n0 = eng.launch_count
-        l2, p2, f2 = eng.fusion_head(img, txt, 512, 10, want_fused=True)
-        torch.cuda.synchronize()
-        assert eng.launch_count - n0 > 10, "fuse_tail=0 must take the per-layer launches"
-    finally:
-        eng.set_option("fuse_tail", 1.0)
+    n0 = eng.launch_count
+    eng.fusion_head(img, txt, 512, 10)
+    torch.cuda.synchronize()
+    assert eng.launch_count - n0 == 3, "two casts + ONE fused launch expected"
+    n0 = eng.launch_count
+    f2 = eng.fusion(img, txt, 512, 8)[0]
+    l2 = eng.head(f2, 10)[0]
+    torch.cuda.synchronize()
+    assert eng.launch_count - n0 > 10, "the per-layer reference takes the per-layer launches"
     _logits_ok(l2, ref_logits)
     assert _rel_rows(fused, f2) <= REL_TOL
     again = eng.fusion_head(img, txt, 512, 10)[0]
@@ -198,10 +200,9 @@ def test_fused_tail_vs_oracle(cuda, state):
     assert torch.equal(one[0], logits[77])
 
 
-def test_fused_layernorm_vs_separate_launch(cuda, state):
-    """BERT with LayerNorm in the GEMM epilogue (option fuse_ln: 1 = FFN2 with the statistics through L2, the
-    default; 2 = both dense + residual GEMMs on clusters; active from ~6.4k tokens per pass) against the separate
-    LayerNorm launches and against the oracle on the first rows."""
+def test_text_encoder_ffn2_layernorm_epilogue_vs_oracle(cuda, state):
+    """BERT with FFN2 + residual + LayerNorm as one GEMM launch (statistics exchanged through L2) in each of the 11
+    full layers and in the CLS-row last layer, against the oracle on all 96 CLS rows (~8k live tokens per pass)."""
     model = _use(state, "sens")
     sd = {k: v.float() for k, v in state["sens"].items() if v.is_floating_point()}
     B, S = 96, 128
@@ -209,25 +210,19 @@ def test_fused_layernorm_vs_separate_launch(cuda, state):
     _, ids, mask = synth.make_inputs(B, S, 11, lengths, H=32, W=32)
     enc = model.text_encoder
     eng = enc._engine()          # the sub-module called on its own has its own engine
-    outs, launches = {}, {}
     with torch.no_grad():
-        ref = oracle.text_encoder(sd, ids[:8], mask[:8])
+        ref = oracle.text_encoder(sd, ids, mask)
+        enc(ids.cuda(), mask.cuda())
+        eng.profile(True)
         try:
-            for mode in (1, 0, 2):
-                eng.set_option("fuse_ln", float(mode))
-                enc(ids.cuda(), mask.cuda())
-                n0 = eng.launch_count
-                outs[mode] = enc(ids.cuda(), mask.cuda()).cpu()
-                launches[mode] = eng.launch_count - n0
-                assert torch.equal(outs[mode], enc(ids.cuda(), mask.cuda()).cpu()), f"fuse_ln={mode} not deterministic"
+            out = enc(ids.cuda(), mask.cuda()).cpu()
+            rows = {r["label"]: r["launches"] for r in eng.profile_report()}
         finally:
-            eng.set_option("fuse_ln", 1.0)
-    # one / two LayerNorm launches less in each of the 11 full layers (the last layer runs on CLS rows)
-    assert launches[0] - launches[1] == 11 and launches[0] - launches[2] == 22, launches
-    for mode in (1, 2):
-        assert _rel_rows(outs[mode], outs[0]) <= REL_TOL
-    for mode in (0, 1, 2):
-        assert _rel_rows(outs[mode][:8], ref) <= REL_TOL
+            eng.profile(False)
+        assert torch.equal(out, enc(ids.cuda(), mask.cuda()).cpu()), "not deterministic"
+    assert rows.get("bert.ffn2+res+ln") == 11 and rows.get("bert.cls.ffn2+res+ln") == 1, rows
+    assert "bert.ffn2+res" not in rows and "bert.attn_out+res+ln" not in rows, rows
+    assert _rel_rows(out, ref) <= REL_TOL, _rel_rows(out, ref)
 
 
 def test_unimodal_classifiers_vs_oracle(cuda, state):

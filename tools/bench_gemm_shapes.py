@@ -1,6 +1,5 @@
 #!/usr/bin/env python
 """Timing of single GEMM launches at the BERT shapes of the benchmark (74 k live tokens per pass).
-MRD_DEBUG_PAIR=0/1 switches the cta_group::2 variant, MRD_DEBUG_SPLIT_EPILOGUE the two-group epilogue.
     python tools/bench_gemm_shapes.py [M]"""
 import ctypes as C
 import math
