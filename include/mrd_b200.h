@@ -331,6 +331,65 @@ int mrd_attention_bwd_bf16(const void* qkv, const void* ctx, const void* dctx, c
 int mrd_layernorm_bwd_bf16(const void* s_in, const void* dy, const float* gamma, float eps, int rows,
                            int width, void* dx, float* dgamma, float* dbeta, void* stream);
 
+/* The other non-GEMM kernels of the training step, one entry each (unit tests, captures of one kernel).  Each
+ * calls the kernel's host wrapper in csrc/train_kernels.h with the same arguments; the semantics are documented
+ * there.  bf16 tensors are void*, dropout is given as (seed, site, p) as in mrd_dropout_mask, and dyn_rows
+ * (optional, device int) bounds the row count on the device as in the engine's token-packed buffers. */
+int mrd_dropout_bf16(const void* x, long long ldx, int rows, int width, const int* dyn_rows,
+                     unsigned long long seed, unsigned int site, double p, void* y, long long ldy, void* stream);
+int mrd_dropout_f32(const float* x, int rows, int width, unsigned long long seed, unsigned int site, double p,
+                    float* y, void* stream);
+int mrd_relu_dropout_f32(const float* x, int rows, int width, unsigned long long seed, unsigned int site,
+                         double p, float* y, void* stream);
+int mrd_head_dropout_f32(const float* x, int rows, int heads, int head_dim, unsigned long long seed,
+                         unsigned int site, double p, float* y, float* w_out, void* stream);
+/* s_out = res + dropout(z) (bf16), y = LayerNorm(s_out)*gamma + beta (bf16); width in {256,512,768,1024}. */
+int mrd_drop_add_layernorm_bf16(const void* z, const void* res, int rows, int width, const int* dyn_rows,
+                                unsigned long long seed, unsigned int site, double p, const float* gamma,
+                                const float* beta, float eps, void* s_out, void* y, void* stream);
+int mrd_layernorm_f32(const float* x, long long ldx, const float* gamma, const float* beta, float eps, int rows,
+                      int width, float* y, long long ldy, void* stream);
+int mrd_layernorm_bwd_f32(const float* x, long long ldx, const float* dy, long long lddy, const float* gamma,
+                          float eps, int rows, int width, float* dx, long long lddx, float* dgamma, float* dbeta,
+                          void* stream);
+int mrd_gelu_fwd_bf16(const void* u, int rows, int width, const int* dyn_rows, void* g, void* stream);
+int mrd_gelu_bwd_bf16(const void* u, const void* dg, int rows, int width, const int* dyn_rows, void* du,
+                      void* stream);
+/* y0 [width0][Kp] = x0^T, y1 [width1][Kp] = x1^T (x1 may be NULL), zero-filled past the live rows; colsum0
+ * (optional) += the column sums of x0 over the live rows. */
+int mrd_transpose_pad2_bf16(const void* x0, long long ldx0, int width0, void* y0, const void* x1, long long ldx1,
+                            int width1, void* y1, int rows, const int* dyn_rows, int Kp, void* stream,
+                            float* colsum0);
+int mrd_colsum_bf16(const void* x, long long ldx, int rows, int width, const int* dyn_rows, float scale,
+                    float* out, void* stream);
+int mrd_colsum_f32(const float* x, long long ldx, int rows, int width, float* out, void* stream);
+int mrd_relu_bwd_f32(const float* y, const float* dy, long long n, float* dx, void* stream);
+int mrd_scatter_cls_rows_bf16(const float* src, const int* seq_off, int B, int width, void* dst, void* stream);
+int mrd_gather_cls_rows_f32(const void* x, const int* seq_off, int B, int width, float* y, void* stream);
+/* Backward of the BERT embeddings (word[id] + pos_type[pos] -> LayerNorm, width 768) into the three tables and
+ * the LayerNorm parameters (each output optional, all accumulated); word rows of pad_idx get nothing. */
+int mrd_embed_layernorm_bwd(const long long* ids, const int* row_tok, int rows, const int* dyn_rows, int S,
+                            const void* word, const float* pos_type, const float* gamma, float eps, int vocab,
+                            int pad_idx, const void* dy, float* dword, float* dpos, float* dtype0, float* dgamma,
+                            float* dbeta, void* stream);
+/* BatchNorm with batch statistics on bf16 [rows, C]: sums about a per-channel shift (the mean of the first 8
+ * rows, written to shift[C]; mean = shift + sum/rows, var = sumsq/rows - (sum/rows)^2), the in-place normalise
+ * (+ identity, + ReLU), and the running-statistics update of several layers from one table of mrd_bn_site. */
+int mrd_bn_stats_bf16(const void* y, long long rows, int C, float* sum, float* sumsq, float* shift, void* stream);
+int mrd_bn_apply_stats_bf16(void* y, long long rows, int C, const float* sum, const float* sumsq,
+                            const float* shift, const float* gamma, const float* beta, float eps,
+                            const void* identity, int relu, void* stream);
+typedef struct {
+    const float* sum;    /* mrd_bn_stats_bf16's outputs for this layer */
+    const float* sumsq;
+    const float* shift;
+    float* running_mean; /* updated in place */
+    float* running_var;
+    float n;             /* rows the sums cover */
+    int C;
+} mrd_bn_site;
+int mrd_bn_update_running(const mrd_bn_site* table_dev, int sites, int max_C, float momentum, void* stream);
+
 /* clip_grad_norm_(parameters, max_norm) + torch.optim.AdamW.step() of the reference's loop (src/train.py:307-320,
  * :193-198) as two multi-tensor launches without a host synchronisation: the global L2 norm of all gradients is
  * reduced into sqnorm_dev[0] (its square; zeroed inside), the clip coefficient min(1, max_norm / (norm + 1e-6)) is

@@ -80,6 +80,26 @@ SIGNATURES = {
                                     _ll, _vp]),
     "mrd_adamw_step": (_i, [_vp, _i, _vp, _vp, _i, _i, _f, _f, _f, _ll, _f, _vp, _vp]),
     "mrd_layernorm_bwd_bf16": (_i, [_vp, _vp, _vp, _f, _i, _i, _vp, _vp, _vp, _vp]),
+    "mrd_dropout_bf16": (_i, [_vp, _ll, _i, _i, _vp, C.c_ulonglong, C.c_uint, _d, _vp, _ll, _vp]),
+    "mrd_dropout_f32": (_i, [_vp, _i, _i, C.c_ulonglong, C.c_uint, _d, _vp, _vp]),
+    "mrd_relu_dropout_f32": (_i, [_vp, _i, _i, C.c_ulonglong, C.c_uint, _d, _vp, _vp]),
+    "mrd_head_dropout_f32": (_i, [_vp, _i, _i, _i, C.c_ulonglong, C.c_uint, _d, _vp, _vp, _vp]),
+    "mrd_drop_add_layernorm_bf16": (_i, [_vp, _vp, _i, _i, _vp, C.c_ulonglong, C.c_uint, _d, _vp, _vp, _f, _vp, _vp, _vp]),
+    "mrd_layernorm_f32": (_i, [_vp, _ll, _vp, _vp, _f, _i, _i, _vp, _ll, _vp]),
+    "mrd_layernorm_bwd_f32": (_i, [_vp, _ll, _vp, _ll, _vp, _f, _i, _i, _vp, _ll, _vp, _vp, _vp]),
+    "mrd_gelu_fwd_bf16": (_i, [_vp, _i, _i, _vp, _vp, _vp]),
+    "mrd_gelu_bwd_bf16": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp]),
+    "mrd_transpose_pad2_bf16": (_i, [_vp, _ll, _i, _vp, _vp, _ll, _i, _vp, _i, _vp, _i, _vp, _vp]),
+    "mrd_colsum_bf16": (_i, [_vp, _ll, _i, _i, _vp, _f, _vp, _vp]),
+    "mrd_colsum_f32": (_i, [_vp, _ll, _i, _i, _vp, _vp]),
+    "mrd_relu_bwd_f32": (_i, [_vp, _vp, _ll, _vp, _vp]),
+    "mrd_scatter_cls_rows_bf16": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
+    "mrd_gather_cls_rows_f32": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
+    "mrd_embed_layernorm_bwd": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp, _vp, _f, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp,
+                                     _vp]),
+    "mrd_bn_stats_bf16": (_i, [_vp, _ll, _i, _vp, _vp, _vp, _vp]),
+    "mrd_bn_apply_stats_bf16": (_i, [_vp, _ll, _i, _vp, _vp, _vp, _vp, _vp, _f, _vp, _i, _vp]),
+    "mrd_bn_update_running": (_i, [_vp, _i, _i, _f, _vp]),
 }
 
 

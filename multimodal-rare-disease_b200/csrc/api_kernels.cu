@@ -8,8 +8,14 @@
 #include "conv_chain.h"
 #include "gemm_conv.h"
 #include "tma_host.h"
+#include "train_kernels.h"
+#include "rng.cuh"
 
 using namespace mrd;
+
+typedef __nv_bfloat16 bf16;
+
+static_assert(sizeof(BnSite) == sizeof(mrd_bn_site), "layout");
 
 extern "C" {
 
@@ -191,6 +197,116 @@ int mrd_compact_tokens(const void* mask, int mask_dtype, int B, int S, int keep_
 
 int mrd_mask_to_bias(const void* mask, int mask_dtype, int B, int S, float* bias, void* stream) {
     return mask_to_bias(mask, mask_dtype, B, S, bias, static_cast<cudaStream_t>(stream));
+}
+
+// ---- training-step kernels (train_kernels.h)
+
+int mrd_dropout_bf16(const void* x, long long ldx, int rows, int width, const int* dyn_rows,
+                     unsigned long long seed, unsigned int site, double p, void* y, long long ldy, void* stream) {
+    return dropout_bf16(static_cast<const bf16*>(x), ldx, rows, width, dyn_rows, make_drop(seed, site, p),
+                        static_cast<bf16*>(y), ldy, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_dropout_f32(const float* x, int rows, int width, unsigned long long seed, unsigned int site, double p,
+                    float* y, void* stream) {
+    return dropout_f32(x, rows, width, make_drop(seed, site, p), y, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_relu_dropout_f32(const float* x, int rows, int width, unsigned long long seed, unsigned int site,
+                         double p, float* y, void* stream) {
+    return relu_dropout_f32(x, rows, width, make_drop(seed, site, p), y, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_head_dropout_f32(const float* x, int rows, int heads, int head_dim, unsigned long long seed,
+                         unsigned int site, double p, float* y, float* w_out, void* stream) {
+    return head_dropout_f32(x, rows, heads, head_dim, make_drop(seed, site, p), y, w_out,
+                            static_cast<cudaStream_t>(stream));
+}
+
+int mrd_drop_add_layernorm_bf16(const void* z, const void* res, int rows, int width, const int* dyn_rows,
+                                unsigned long long seed, unsigned int site, double p, const float* gamma,
+                                const float* beta, float eps, void* s_out, void* y, void* stream) {
+    return drop_add_ln_fwd(static_cast<const bf16*>(z), static_cast<const bf16*>(res), rows, width, dyn_rows,
+                           make_drop(seed, site, p), gamma, beta, eps, static_cast<bf16*>(s_out),
+                           static_cast<bf16*>(y), static_cast<cudaStream_t>(stream));
+}
+
+int mrd_layernorm_f32(const float* x, long long ldx, const float* gamma, const float* beta, float eps, int rows,
+                      int width, float* y, long long ldy, void* stream) {
+    return ln_fwd_f32(x, ldx, gamma, beta, eps, rows, width, y, ldy, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_layernorm_bwd_f32(const float* x, long long ldx, const float* dy, long long lddy, const float* gamma,
+                          float eps, int rows, int width, float* dx, long long lddx, float* dgamma, float* dbeta,
+                          void* stream) {
+    return ln_bwd_f32(x, ldx, dy, lddy, gamma, eps, rows, width, dx, lddx, dgamma, dbeta,
+                      static_cast<cudaStream_t>(stream));
+}
+
+int mrd_gelu_fwd_bf16(const void* u, int rows, int width, const int* dyn_rows, void* g, void* stream) {
+    return gelu_fwd_bf16(static_cast<const bf16*>(u), rows, width, dyn_rows, static_cast<bf16*>(g),
+                         static_cast<cudaStream_t>(stream));
+}
+
+int mrd_gelu_bwd_bf16(const void* u, const void* dg, int rows, int width, const int* dyn_rows, void* du,
+                      void* stream) {
+    return gelu_bwd_bf16(static_cast<const bf16*>(u), static_cast<const bf16*>(dg), rows, width, dyn_rows,
+                         static_cast<bf16*>(du), static_cast<cudaStream_t>(stream));
+}
+
+int mrd_transpose_pad2_bf16(const void* x0, long long ldx0, int width0, void* y0, const void* x1, long long ldx1,
+                            int width1, void* y1, int rows, const int* dyn_rows, int Kp, void* stream,
+                            float* colsum0) {
+    return transpose_pad2_bf16(static_cast<const bf16*>(x0), ldx0, width0, static_cast<bf16*>(y0),
+                               static_cast<const bf16*>(x1), ldx1, width1, static_cast<bf16*>(y1), rows, dyn_rows, Kp,
+                               static_cast<cudaStream_t>(stream), colsum0);
+}
+
+int mrd_colsum_bf16(const void* x, long long ldx, int rows, int width, const int* dyn_rows, float scale,
+                    float* out, void* stream) {
+    return colsum_bf16(static_cast<const bf16*>(x), ldx, rows, width, dyn_rows, scale, out,
+                       static_cast<cudaStream_t>(stream));
+}
+
+int mrd_colsum_f32(const float* x, long long ldx, int rows, int width, float* out, void* stream) {
+    return colsum_f32(x, ldx, rows, width, out, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_relu_bwd_f32(const float* y, const float* dy, long long n, float* dx, void* stream) {
+    return relu_bwd_f32(y, dy, n, dx, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_scatter_cls_rows_bf16(const float* src, const int* seq_off, int B, int width, void* dst, void* stream) {
+    return scatter_cls_rows_bf16(src, seq_off, B, width, static_cast<bf16*>(dst), static_cast<cudaStream_t>(stream));
+}
+
+int mrd_gather_cls_rows_f32(const void* x, const int* seq_off, int B, int width, float* y, void* stream) {
+    return gather_cls_rows_f32(static_cast<const bf16*>(x), seq_off, B, width, y, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_embed_layernorm_bwd(const long long* ids, const int* row_tok, int rows, const int* dyn_rows, int S,
+                            const void* word, const float* pos_type, const float* gamma, float eps, int vocab,
+                            int pad_idx, const void* dy, float* dword, float* dpos, float* dtype0, float* dgamma,
+                            float* dbeta, void* stream) {
+    return embed_ln_bwd(ids, row_tok, rows, dyn_rows, S, static_cast<const bf16*>(word), pos_type, gamma, eps, vocab,
+                        pad_idx, static_cast<const bf16*>(dy), dword, dpos, dtype0, dgamma, dbeta,
+                        static_cast<cudaStream_t>(stream));
+}
+
+int mrd_bn_stats_bf16(const void* y, long long rows, int C, float* sum, float* sumsq, float* shift, void* stream) {
+    return bn_stats_bf16(static_cast<const bf16*>(y), rows, C, sum, sumsq, shift, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_bn_apply_stats_bf16(void* y, long long rows, int C, const float* sum, const float* sumsq,
+                            const float* shift, const float* gamma, const float* beta, float eps,
+                            const void* identity, int relu, void* stream) {
+    return bn_apply_stats_bf16(static_cast<bf16*>(y), rows, C, sum, sumsq, shift, gamma, beta, eps,
+                               static_cast<const bf16*>(identity), relu, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_bn_update_running(const mrd_bn_site* table_dev, int sites, int max_C, float momentum, void* stream) {
+    return bn_update_running(reinterpret_cast<const BnSite*>(table_dev), sites, max_C, momentum,
+                             static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

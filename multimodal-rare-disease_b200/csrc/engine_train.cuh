@@ -279,7 +279,7 @@ struct TrainCnn {
     float *ones = nullptr, *zeros = nullptr;     // [2048] identity BatchNorm for the packers / zero bias
     float* dummy_bias = nullptr;                 // [2048] bias output of the packers (always zero, unused)
     std::vector<Bottleneck> blocks;              // raw (un-folded) filters
-    float* stats = nullptr;                      // [sites][4][2048]: sum, sumsq, (2 spare)
+    float* stats = nullptr;                      // [sites][4][2048]: sum, sumsq, shift, (1 spare)
     BnSite* site_table = nullptr;                // device: one entry per BatchNorm layer (running-stat update)
     std::vector<BnSite> site_host;
     std::vector<std::string> bn_names;           // site -> "cnn_encoder.backbone....bnX"
@@ -424,17 +424,18 @@ int run_backbone_train(mrd_ctx* c, const void* images, int img_dtype, int B, int
             MRD_TRY(raw_need(c, nm + ".running_mean", &rm));
             MRD_TRY(raw_need(c, nm + ".running_var", &rv));
             BnSite& e = tc->site_host[site];
-            e.sum = st; e.sumsq = st + 2048;
+            e.sum = st; e.sumsq = st + 2048; e.shift = st + 2 * 2048;
             e.running_mean = const_cast<float*>(rm->p);
             e.running_var = const_cast<float*>(rv->p);
             e.n = static_cast<float>(rows);
             e.C = C;
         }
         ++site;
-        TRK("train.bn_stats", CAT_MEM, bn_stats_bf16(y, rows, C, st, st + 2048, s));
+        TRK("train.bn_stats", CAT_MEM, bn_stats_bf16(y, rows, C, st, st + 2048, st + 2 * 2048, s));
         // scale / shift are derived from the sums inside the normalise pass; the running buffers of all layers
         // are updated by one launch at the end of the backbone
-        TRK("train.bn_apply", CAT_MEM, bn_apply_stats_bf16(y, rows, C, st, st + 2048, g->p, b->p, c->bn_eps, identity, relu, s));
+        TRK("train.bn_apply", CAT_MEM, bn_apply_stats_bf16(y, rows, C, st, st + 2048, st + 2 * 2048, g->p, b->p, c->bn_eps,
+                                                           identity, relu, s));
         return 0;
     };
     const CnnPlan& p = tc->plan;

@@ -532,19 +532,38 @@ embed_ln_bwd_kernel(const long long* __restrict__ ids, const int* __restrict__ r
 }
 
 // ------------------------------------------------------------------ BatchNorm (batch statistics)
+// The sums are taken about a per-channel shift k, the mean of the first (up to) 8 rows, so |mean - k| is of the
+// order of the spread: var = E[(y-k)^2] - E[y-k]^2 does not cancel when |mean| >> std, as E[y^2] - mean^2 would.
+// Every block derives the same k from the same 8 rows; the blocks of the first row slice store it.
 __global__ void __launch_bounds__(256)
 bn_stats_kernel(const bf16* __restrict__ y, long long rows, int C, float* __restrict__ sum,
-                float* __restrict__ sumsq) {
+                float* __restrict__ sumsq, float* __restrict__ shift) {
     __shared__ float red[2][8][64];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int c = blockIdx.x * 64 + lane * 2;
     float a0 = 0.0f, a1 = 0.0f, q0 = 0.0f, q1 = 0.0f;
     if (c < C) {
+        const int nk = rows < 8 ? static_cast<int>(rows) : 8;
+        float k0 = 0.0f, k1 = 0.0f;
+#pragma unroll
+        for (int r = 0; r < 8; ++r) {   // unrolled: the 8 loads are in flight together
+            if (r < nk) {
+                const float2 v = unpack_bf16(__ldg(reinterpret_cast<const uint32_t*>(y + static_cast<long long>(r) * C + c)));
+                k0 += v.x; k1 += v.y;
+            }
+        }
+        // rounded to bf16 like y, so that y - k is exact in fp32 across the channel's range
+        const float2 k = unpack_bf16(pack_bf16(k0 / nk, k1 / nk));
+        if (blockIdx.y == 0 && warp == 0) {
+            shift[c] = k.x;
+            shift[c + 1] = k.y;
+        }
         for (long long r = static_cast<long long>(blockIdx.y) * 8 + warp; r < rows;
              r += static_cast<long long>(gridDim.y) * 8) {
             const float2 v = unpack_bf16(*reinterpret_cast<const uint32_t*>(y + r * C + c));
-            a0 += v.x; a1 += v.y;
-            q0 = fmaf(v.x, v.x, q0); q1 = fmaf(v.y, v.y, q1);
+            const float d0 = v.x - k.x, d1 = v.y - k.y;
+            a0 += d0; a1 += d1;
+            q0 = fmaf(d0, d0, q0); q1 = fmaf(d1, d1, q1);
         }
     }
     red[0][warp][lane * 2] = a0; red[0][warp][lane * 2 + 1] = a1;
@@ -562,16 +581,16 @@ bn_stats_kernel(const bf16* __restrict__ y, long long rows, int C, float* __rest
 
 // scale / shift of all C channels are derived once per block into shared memory (2*C floats), then applied
 __global__ void bn_apply_stats_kernel(bf16* __restrict__ y, long long n8, int C, const float* __restrict__ sum,
-                                      const float* __restrict__ sumsq, float inv_n, const float* __restrict__ gamma,
-                                      const float* __restrict__ beta, float eps, const bf16* __restrict__ identity,
-                                      int relu) {
+                                      const float* __restrict__ sumsq, const float* __restrict__ shift, float inv_n,
+                                      const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
+                                      const bf16* __restrict__ identity, int relu) {
     extern __shared__ float ss[];   // [C] scale, [C] shift
     for (int c = threadIdx.x; c < C; c += blockDim.x) {
-        const float mean = __ldg(sum + c) * inv_n;
-        const float var = fmaxf(__ldg(sumsq + c) * inv_n - mean * mean, 0.0f);
+        const float md = __ldg(sum + c) * inv_n;   // mean - shift
+        const float var = fmaxf(__ldg(sumsq + c) * inv_n - md * md, 0.0f);
         const float sc = __ldg(gamma + c) * rsqrtf(var + eps);
         ss[c] = sc;
-        ss[C + c] = __ldg(beta + c) - mean * sc;
+        ss[C + c] = __ldg(beta + c) - (__ldg(shift + c) + md) * sc;
     }
     __syncthreads();
     for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n8;
@@ -601,8 +620,9 @@ __global__ void bn_update_running_kernel(const BnSite* __restrict__ table, float
     const BnSite st = table[blockIdx.y];
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= st.C) return;
-    const float mean = st.sum[c] / st.n;
-    const float var = fmaxf(st.sumsq[c] / st.n - mean * mean, 0.0f);
+    const float md = st.sum[c] / st.n;   // mean - shift
+    const float mean = st.shift[c] + md;
+    const float var = fmaxf(st.sumsq[c] / st.n - md * md, 0.0f);
     st.running_mean[c] = (1.0f - momentum) * st.running_mean[c] + momentum * mean;
     st.running_var[c] = (1.0f - momentum) * st.running_var[c] + momentum * var * (st.n / fmaxf(st.n - 1.0f, 1.0f));
 }
@@ -778,7 +798,7 @@ int embed_ln_bwd(const long long* ids, const int* row_tok, int rows, const int* 
     return check_launch("embed_ln_bwd");
 }
 
-int bn_stats_bf16(const bf16* y, long long rows, int C, float* sum, float* sumsq, cudaStream_t s) {
+int bn_stats_bf16(const bf16* y, long long rows, int C, float* sum, float* sumsq, float* shift, cudaStream_t s) {
     if (rows <= 0 || C <= 0) return 0;
     if (C % 2) {
         set_last_error("bn_stats_bf16: odd channel count");
@@ -788,11 +808,12 @@ int bn_stats_bf16(const bf16* y, long long rows, int C, float* sum, float* sumsq
     if (split > 148 * 8) split = 148 * 8;
     if (split < 1) split = 1;
     dim3 grid((C + 63) / 64, static_cast<unsigned>(split));
-    bn_stats_kernel<<<grid, 256, 0, s>>>(y, rows, C, sum, sumsq);
+    bn_stats_kernel<<<grid, 256, 0, s>>>(y, rows, C, sum, sumsq, shift);
     return check_launch("bn_stats_bf16");
 }
-int bn_apply_stats_bf16(bf16* y, long long rows, int C, const float* sum, const float* sumsq, const float* gamma,
-                        const float* beta, float eps, const bf16* identity, int relu, cudaStream_t s) {
+int bn_apply_stats_bf16(bf16* y, long long rows, int C, const float* sum, const float* sumsq, const float* shift,
+                        const float* gamma, const float* beta, float eps, const bf16* identity, int relu,
+                        cudaStream_t s) {
     if (rows <= 0 || C <= 0) return 0;
     if (C % 8) {
         set_last_error("bn_apply_stats_bf16: C %% 8 != 0");
@@ -807,8 +828,9 @@ int bn_apply_stats_bf16(bf16* y, long long rows, int C, const float* sum, const 
     unsigned grid = nblk(n8, 256 * 4);
     if (grid > 148u * 4u) grid = 148u * 4u;
     if (grid < 1u) grid = 1u;
-    bn_apply_stats_kernel<<<grid, 256, 2 * C * sizeof(float), s>>>(y, n8, C, sum, sumsq, 1.0f / static_cast<float>(rows),
-                                                                   gamma, beta, eps, identity, relu);
+    bn_apply_stats_kernel<<<grid, 256, 2 * C * sizeof(float), s>>>(y, n8, C, sum, sumsq, shift,
+                                                                   1.0f / static_cast<float>(rows), gamma, beta, eps,
+                                                                   identity, relu);
     return check_launch("bn_apply_stats_bf16");
 }
 int bn_update_running(const BnSite* table, int sites, int max_C, float momentum, cudaStream_t s) {

@@ -99,19 +99,25 @@ int attention_backward(const __nv_bfloat16* qkv, const __nv_bfloat16* ctx, const
                        __nv_bfloat16* dqkv, cudaStream_t s, float* dkv_acc = nullptr);
 
 // ---- BatchNorm with batch statistics (frozen backbone under model.train(), TV:models/resnet.py:143-163) --
-// sum[c] += sum_r y[r,c], sumsq[c] += sum_r y[r,c]^2 over an NHWC bf16 tensor viewed as [rows, C]; C % 2 == 0.
-int bn_stats_bf16(const __nv_bfloat16* y, long long rows, int C, float* sum, float* sumsq, cudaStream_t s);
+// Shifted sums over an NHWC bf16 tensor viewed as [rows, C] (C % 2 == 0): shift[c] = the mean of y[0..7, c]
+// rounded to bf16 (written),
+// sum[c] += sum_r (y[r,c] - shift[c]), sumsq[c] += sum_r (y[r,c] - shift[c])^2.  The shift keeps the variance
+// free of the cancellation of sumsq/n - mean^2 when a channel's |mean| is large against its spread.
+int bn_stats_bf16(const __nv_bfloat16* y, long long rows, int C, float* sum, float* sumsq, float* shift,
+                  cudaStream_t s);
 // y = act(y*scale[c] + shift[c] (+ identity)) in place on [rows, C] bf16 (C % 8 == 0), scale / shift derived per
-// block from the batch sums: mean = sum/n, var = sumsq/n - mean^2 (biased), scale = gamma*rsqrt(var+eps),
-// shift = beta - mean*scale.
+// block from bn_stats_bf16's sums: d = sum/n, mean = shift + d, var = sumsq/n - d^2 (biased),
+// scale = gamma*rsqrt(var+eps), shift = beta - mean*scale.
 int bn_apply_stats_bf16(__nv_bfloat16* y, long long rows, int C, const float* sum, const float* sumsq,
-                        const float* gamma, const float* beta, float eps, const __nv_bfloat16* identity, int relu,
-                        cudaStream_t s);
+                        const float* shift, const float* gamma, const float* beta, float eps,
+                        const __nv_bfloat16* identity, int relu, cudaStream_t s);
 // Running-statistics update of every BatchNorm layer of a forward in ONE launch (what nn.BatchNorm2d does in
-// train mode: running <- (1-m)*running + m*(mean, var*n/(n-1))).  table: device array, one entry per layer.
+// train mode: running <- (1-m)*running + m*(mean, var*n/(n-1))), from bn_stats_bf16's sums.  table: device
+// array, one entry per layer.  Mirrored by mrd_bn_site (include/mrd_b200.h).
 struct BnSite {
     const float* sum;
     const float* sumsq;
+    const float* shift;
     float* running_mean;
     float* running_var;
     float n;

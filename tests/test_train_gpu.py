@@ -164,9 +164,11 @@ def test_splitk_weight_gradient_gemm(cuda, lib, M, N, K, live):
     assert ((out - 2 * ref).norm() / ref.norm()).item() <= 6e-5
 
 
-@pytest.mark.parametrize("width", [768, 512])
-def test_layernorm_backward_vs_autograd(cuda, lib, width):
-    rows = 1000
+@pytest.mark.parametrize("rows,width", [
+    pytest.param(1000, 768, id="768"), pytest.param(1000, 512, id="512"),
+    # 8192 rows (the training benchmark's B*S) against a grid of 296 blocks x 8 warps: 3-4 rows per warp
+    (8192, 256), (8192, 768), (8192, 1024), (1000, 1024)])
+def test_layernorm_backward_vs_autograd(cuda, lib, rows, width):
     g = torch.Generator().manual_seed(8)
     s_in = (torch.randn(rows, width, generator=g) * 2 + 0.3).to(cuda, torch.bfloat16)
     dy = torch.randn(rows, width, generator=g).to(cuda, torch.bfloat16)
@@ -175,7 +177,7 @@ def test_layernorm_backward_vs_autograd(cuda, lib, width):
     gm = gamma.clone().requires_grad_(True)
     bt = torch.zeros(width, device=cuda, requires_grad=True)
     F.layer_norm(x, (width,), gm, bt, 1e-12).backward(dy.float())
-    dx = torch.empty_like(s_in)
+    dx = torch.full_like(s_in, float("nan"))
     dg, db = torch.zeros(width, device=cuda), torch.zeros(width, device=cuda)
     assert lib.mrd_layernorm_bwd_bf16(_p(s_in), _p(dy), _p(gamma), 1e-12, rows, width, _p(dx), _p(dg), _p(db),
                                       _stream()) == 0, lib.mrd_last_error()

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Small-shape pass over every hand-written kernel for compute-sanitizer (memcheck / racecheck / synccheck /
 initcheck): the unit tests of tests/test_kernels_gpu.py at reduced sizes, one tiny multimodal forward and one
-tiny training step.  Each case also checks its result, so a sanitizer run doubles as a correctness run.
+tiny training step,
+and the training-step kernel tests of tests/test_train_kernels_gpu.py at their smaller shapes.  Each case also checks its result, so a sanitizer run doubles as a correctness run.
 
     compute-sanitizer --tool memcheck  python tools/sanitize_kernels.py
     compute-sanitizer --tool racecheck python tools/sanitize_kernels.py
@@ -19,6 +20,7 @@ import torch  # noqa: E402
 import mrd_b200  # noqa: E402,F401
 import synth  # noqa: E402
 import test_kernels_gpu as K  # noqa: E402
+import test_train_kernels_gpu as TK  # noqa: E402
 from importlib import import_module  # noqa: E402
 
 lib = import_module("multimodal-rare-disease_b200._lib").load()
@@ -44,6 +46,16 @@ cases = [
     ("attention varlen", lambda: K.test_attention_varlen(lib, cuda, "tcgen05", [128, 70, 1, 64, 65], 12)),
     ("attention varlen long", lambda: K.test_attention_varlen(lib, cuda, "tcgen05", [512, 64, 300], 12)),
     ("compact tokens", lambda: K.test_compact_tokens(lib, cuda, 7, 128, 0)),
+    ("dropout bf16 strided", lambda: TK.test_dropout_bf16(lib, cuda, 0.1, True)),
+    ("dropout f32 family", lambda: TK.test_dropout_f32_family(lib, cuda, 0.1)),
+    ("drop + add + layernorm", lambda: TK.test_drop_add_layernorm(lib, cuda, 768, 0.1, False)),
+    ("layernorm f32 fwd / bwd", lambda: TK.test_layernorm_f32_forward_backward(lib, cuda, 300, 64, 1)),
+    ("transpose pad2", lambda: TK.test_transpose_pad2(lib, cuda, 768, 768, 65, True)),
+    ("colsum f32 + relu bwd", lambda: TK.test_colsum_f32_and_relu_bwd(lib, cuda)),
+    ("cls gather / scatter", lambda: TK.test_cls_gather_scatter(lib, cuda)),
+    ("embed layernorm bwd", lambda: TK.test_embed_layernorm_backward(lib, cuda, 8, 512)),
+    ("bn batch stats", lambda: TK.test_batchnorm_batch_statistics(lib, cuda, 3136, 2048, "identity_relu")),
+    ("bn running update", lambda: TK.test_batchnorm_running_update(lib, cuda)),
 ]
 
 
