@@ -87,6 +87,15 @@ int mrd_cnn_encoder_fwd(mrd_ctx* ctx, const void* images, int img_dtype, int B, 
 int mrd_text_encoder_fwd(mrd_ctx* ctx, const long long* ids, const void* mask, int mask_dtype, int B,
                          int S, float* cls, float* last_hidden, float* all_hidden, void* stream);
 
+/* mrd_text_encoder_fwd plus every layer's attention probabilities (HF's eager attention with
+ * output_attentions=True, HF:models/bert/modeling_bert.py:115-140, eval mode).  attn_probs (optional): f32
+ * [layers,B,heads,S,S], element [l,b,h,q,k] = softmax_k(q.k/8 + mask bias) of layer l, for every query row
+ * (padded ones included: requesting it keeps every token, like last_hidden).  Masked keys are exactly 0; a
+ * sample without any attended key gets all-zero rows (its attention output is zero too).  That is
+ * layers*B*heads*S*S*4 bytes.  mrd_text_encoder_fwd is this call with attn_probs = NULL. */
+int mrd_text_encoder_fwd_ex(mrd_ctx* ctx, const long long* ids, const void* mask, int mask_dtype, int B, int S,
+                            float* cls, float* last_hidden, float* all_hidden, float* attn_probs, void* stream);
+
 /* MultimodalFusion.forward with fusion_type="attention" (src/fusion_model.py:245-291).
  * img_emb f32 [B,Di], txt_emb f32 [B,Dt] -> fused f32 [B,Hd].  attn_i2t / attn_t2i (optional):
  * f32 [B,heads,1,1], the cross-attention weights (identically 1: softmax over one key). */
@@ -230,6 +239,13 @@ int mrd_bert_embed_layernorm(const long long* ids, int B, int S, const void* wor
  * [B*S, heads*64]. */
 int mrd_attention_bf16(const void* qkv, const float* mask_bias, int B, int S, int heads, void* out,
                        void* stream);
+
+/* The probabilities of mrd_attention_bf16 (same qkv / mask_bias conventions, S <= 512): probs f32
+ * [B,heads,S,S] = softmax_k(q.k + mask_bias[b,k]) for every query row.  Masked keys are exactly 0; a sample
+ * whose keys are all masked gets all-zero rows.  One tcgen05 product Q K^T per (sample, head, 128-query
+ * block), softmax from TMEM, the output written through shared memory (TMA stores when S % 4 == 0). */
+int mrd_attention_probs_bf16(const void* qkv, const float* mask_bias, int B, int S, int heads, float* probs,
+                             void* stream);
 
 /* Token packing for BERT ("unpadding"): keeps token (b,j) iff mask[b,j] != 0 or j == 0 (or all tokens
  * when keep_all).  Outputs (device): seq_off[B+1] first packed row of each sequence, row_tok[r] =

@@ -37,6 +37,7 @@ SIGNATURES = {
     "mrd_ctx_load_weights": (_i, [_vp, _i, C.POINTER(C.c_char_p), C.POINTER(_vp), C.POINTER(_ll), _vp]),
     "mrd_cnn_encoder_fwd": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "mrd_text_encoder_fwd": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "mrd_text_encoder_fwd_ex": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "mrd_fusion_fwd": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "mrd_head_fwd": (_i, [_vp, _vp, _i, _vp, _vp, _vp]),
     "mrd_fusion_head_fwd": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
@@ -62,6 +63,7 @@ SIGNATURES = {
     "mrd_layernorm_residual": (_i, [_vp, _ll, _vp, _ll, _vp, _vp, _f, _i, _i, _vp, _ll, _vp, _ll, _vp]),
     "mrd_bert_embed_layernorm": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _f, _i, _vp, _vp]),
     "mrd_attention_bf16": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
+    "mrd_attention_probs_bf16": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
     "mrd_mask_to_bias": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "mrd_compact_tokens": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mrd_attention_varlen_bf16": (_i, [_vp, _vp, _vp, _i, _i, _i, _ll, _vp, _vp]),

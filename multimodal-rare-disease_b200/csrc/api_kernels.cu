@@ -169,6 +169,12 @@ int mrd_attention_bf16(const void* qkv, const float* mask_bias, int B, int S, in
                              static_cast<__nv_bfloat16*>(out), static_cast<cudaStream_t>(stream));
 }
 
+int mrd_attention_probs_bf16(const void* qkv, const float* mask_bias, int B, int S, int heads, float* probs,
+                             void* stream) {
+    return attention_probs(static_cast<const __nv_bfloat16*>(qkv), mask_bias, B, S, heads, probs,
+                           static_cast<cudaStream_t>(stream));
+}
+
 int mrd_attention_varlen_bf16(const void* qkv, const float* row_bias, const int* seq_off, int B,
                               int max_len, int heads, long long total_rows, void* out, void* stream) {
     if (!seq_off) {

@@ -920,6 +920,8 @@ attention_tc_long_kernel(const __grid_constant__ TcLongParams p) {
     }
 }
 
+}  // namespace
+
 int encode_qkv_maps(CUtensorMap* maps, const __nv_bfloat16* qkv, int heads, long long rows_alloc, int blocked) {
     // 3-D view {64 dims, rows, 3*heads column blocks}: token-major rows are 3*heads*64 elements apart
     // with the blocks side by side; in the blocked layout every block is a contiguous [rows,64] matrix
@@ -934,6 +936,8 @@ int encode_qkv_maps(CUtensorMap* maps, const __nv_bfloat16* qkv, int heads, long
     }
     return 0;
 }
+
+namespace {
 
 int launch_tc_long(const __nv_bfloat16* qkv, const float* mask_bias, const int* seq_off, int B, int S,
                    int heads, long long rows_alloc, int blocked, __nv_bfloat16* out, cudaStream_t stream,

@@ -1,6 +1,7 @@
 // K3: fused masked-softmax self-attention for BERT (S <= 512, head dim 64).
 #pragma once
 
+#include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
@@ -24,6 +25,19 @@ int attention_forward(const __nv_bfloat16* qkv, const float* mask_bias, const in
 // blocked = 1: qkv is [3*heads][rows_alloc][64] (what plan_gemm(c_blocked=1) writes): each head's Q, K
 // and V tile is one contiguous block - streaming-friendly for the TMA loads of the tcgen05 path.
 bool attention_prefers_blocked_qkv(int S);
+
+// The attention probabilities themselves (what HF's eager attention returns with output_attentions=True,
+// HF:models/bert/modeling_bert.py:115-140 in eval mode): probs[b,h,q,k] = softmax_k(q.k + mask_bias[b,k]) in fp32,
+// [B,heads,S,S], for EVERY query row (padded ones included).  Dense layout: sample b owns rows [b*S, (b+1)*S) of
+// qkv and mask_bias is [B,S] or null; rows_alloc / blocked as for attention_forward.  A masked key gets exactly 0;
+// a sample without any attended key gets all-zero rows (attention_forward gives it a zero context).  S <= 512.
+// attention_probs.cu: one tcgen05 product S = Q K^T per (sample, head, 128-query block), softmax from TMEM, and a
+// write stream staged through shared memory (TMA stores when S % 4 == 0).
+int attention_probs(const __nv_bfloat16* qkv, const float* mask_bias, int B, int S, int heads, float* probs,
+                    cudaStream_t stream, long long rows_alloc = 0, int blocked = 0);
+// 3-D TMA views {64 dims, rows, 3*heads blocks} of qkv with row boxes of 32 / 64 / 96 / 128 (attention.cu)
+int encode_qkv_maps(CUtensorMap* maps, const __nv_bfloat16* qkv, int heads, long long rows_alloc, int blocked);
+
 // test hook: force the mma.sync path for every S
 void attention_set_tc(bool on);
 

@@ -1106,8 +1106,9 @@ int run_projection(mrd_ctx* c, BatchPlan* bp, float* emb_f32, cudaStream_t s) {
 }
 
 // BERT encoder over the whole batch in micro-batches; leaves CLS rows in b_txt (+ optional fp32).
+// attn_probs (optional): f32 [layers,B,heads,S,S], every layer's attention probabilities.
 int run_bert(mrd_ctx* c, const long long* ids, const void* mask, int mask_dtype, int B, int S,
-             float* cls_f32, float* last_hidden, float* all_hidden, cudaStream_t s) {
+             float* cls_f32, float* last_hidden, float* all_hidden, float* attn_probs, cudaStream_t s) {
     if (!c->has_text) {
         set_last_error("text_encoder weights are not loaded in this context");
         return -3;
@@ -1136,7 +1137,8 @@ int run_bert(mrd_ctx* c, const long long* ids, const void* mask, int mask_dtype,
             set_last_error("all_hidden requires last_hidden (both keep every token)");
             return -1;
         }
-        const int keep_all = last_hidden != nullptr;
+        // the probabilities are returned for every query row, padded ones included: they need every token too
+        const int keep_all = last_hidden != nullptr || attn_probs != nullptr;
         // hidden_states[l] of HF BertModel: l = 0 is the embedding output, l = i+1 the output of layer i;
         // layout [L+1, B, S, Hd] fp32 (src/text_encoder.py:129-149)
         auto export_hidden = [&](size_t l) -> int {
@@ -1170,6 +1172,15 @@ int run_bert(mrd_ctx* c, const long long* ids, const void* mask, int mask_dtype,
                 MRD_TRY(attention_forward(c->t_qkv, c->t_bias, c->t_seq_off, nb, S, c->bert_heads,
                                           c->t_ctx, s, p->blocked_qkv ? T : c->text_ws_tokens,
                                           p->blocked_qkv));
+            }
+            if (attn_probs) {
+                // keep_all: the packed layout is the dense one, t_bias is the [nb,S] key bias
+                const int H = c->bert_heads;
+                ProfScope ps(c, s, "bert.attn_probs", CAT_MEM, 0,
+                             4.0 * nb * H * S * S + 2.0 * T * Hd * (1 + (S + 127) / 128));
+                MRD_TRY(attention_probs(c->t_qkv, c->t_bias, nb, S, H,
+                                        attn_probs + (static_cast<long long>(i) * B + b0) * H * S * S, s,
+                                        p->blocked_qkv ? T : c->text_ws_tokens, p->blocked_qkv));
             }
             if (i + 1 == p->layers.size() && !last_hidden) {
                 // ---- last layer: only the CLS row of each sequence is consumed downstream
@@ -1446,6 +1457,11 @@ int mrd_cnn_encoder_fwd(mrd_ctx* c, const void* images, int img_dtype, int B, in
 
 int mrd_text_encoder_fwd(mrd_ctx* c, const long long* ids, const void* mask, int mask_dtype, int B,
                          int S, float* cls, float* last_hidden, float* all_hidden, void* stream) {
+    return mrd_text_encoder_fwd_ex(c, ids, mask, mask_dtype, B, S, cls, last_hidden, all_hidden, nullptr, stream);
+}
+
+int mrd_text_encoder_fwd_ex(mrd_ctx* c, const long long* ids, const void* mask, int mask_dtype, int B, int S,
+                            float* cls, float* last_hidden, float* all_hidden, float* attn_probs, void* stream) {
     MRD_TRY(check_ctx(c));
     if (B <= 0) return 0;
     if (mask && (mask_dtype < MRD_DT_I64 || mask_dtype > MRD_DT_BF16)) {
@@ -1455,10 +1471,10 @@ int mrd_text_encoder_fwd(mrd_ctx* c, const long long* ids, const void* mask, int
     if (c->fp32_check) {
         ++c->launches;
         return fp32_text_encoder(c->raw, c->f32_opts(), &c->f32_ws, ids, mask, mask_dtype, B, S, cls,
-                                 last_hidden, all_hidden, static_cast<cudaStream_t>(stream));
+                                 last_hidden, all_hidden, attn_probs, static_cast<cudaStream_t>(stream));
     }
     MRD_TRY(ensure_batch_ws(c, B));
-    return run_bert(c, ids, mask, mask_dtype, B, S, cls, last_hidden, all_hidden,
+    return run_bert(c, ids, mask, mask_dtype, B, S, cls, last_hidden, all_hidden, attn_probs,
                     static_cast<cudaStream_t>(stream));
 }
 
@@ -1604,7 +1620,7 @@ int mrd_multimodal_fwd(mrd_ctx* c, const void* images, int img_dtype, const long
         c->launches += 4;
         MRD_TRY(fp32_cnn_encoder(c->raw, o, &c->f32_ws, static_cast<const float*>(images), B, H, W, ie,
                                  nullptr, nullptr, s));
-        MRD_TRY(fp32_text_encoder(c->raw, o, &c->f32_ws, ids, mask, mask_dtype, B, S, te, nullptr, nullptr, s));
+        MRD_TRY(fp32_text_encoder(c->raw, o, &c->f32_ws, ids, mask, mask_dtype, B, S, te, nullptr, nullptr, nullptr, s));
         MRD_TRY(fp32_fusion(c->raw, o, &c->f32_ws, ie, te, B, fe, attn_i2t, attn_t2i, s));
         return fp32_head(c->raw, o, &c->f32_ws, fe, B, logits, probs, s);
     }
@@ -1612,7 +1628,7 @@ int mrd_multimodal_fwd(mrd_ctx* c, const void* images, int img_dtype, const long
     MRD_TRY(get_batch_plan(c, B, &bp));
     MRD_TRY(run_backbone(c, images, img_dtype, B, H, W, nullptr, nullptr, s));
     MRD_TRY(run_projection(c, bp, img_emb, s));
-    MRD_TRY(run_bert(c, ids, mask, mask_dtype, B, S, txt_emb, nullptr, nullptr, s));
+    MRD_TRY(run_bert(c, ids, mask, mask_dtype, B, S, txt_emb, nullptr, nullptr, nullptr, s));
     return run_tail(c, bp, B, fused, attn_i2t, attn_t2i, logits, probs, s);
 }
 

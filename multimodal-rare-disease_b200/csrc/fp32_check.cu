@@ -116,9 +116,11 @@ __global__ void embed_sum_kernel(const long long* __restrict__ ids, const float*
 }
 
 // softmax(q k^T / sqrt(d) + key_bias) v for one head; one warp per query row, scores in shared memory.
-// qkv: [T, 3*Hd] fp32 (columns Q | K | V), d = 64.
+// qkv: [T, 3*Hd] fp32 (columns Q | K | V), d = 64.  probs (optional): the probabilities, [B,heads,S,S]; a row
+// without any attended key is written as zeros (attention_probs does the same).
 __global__ void attention_f32_kernel(const float* __restrict__ qkv, const float* __restrict__ key_bias,
-                                     int S, int heads, float scale, float* __restrict__ out) {
+                                     int S, int heads, float scale, float* __restrict__ out,
+                                     float* __restrict__ probs) {
     extern __shared__ float sm[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
     const int b = blockIdx.x / heads, h = blockIdx.x % heads;
@@ -151,6 +153,10 @@ __global__ void attention_f32_kernel(const float* __restrict__ qkv, const float*
     }
     sum = wsum(sum);
     __syncwarp();
+    if (probs) {
+        float* pr = probs + (static_cast<long long>(blockIdx.x) * S + q) * S;
+        for (int j = lane; j < S; j += 32) pr[j] = mx == -INFINITY ? 0.0f : sc[j] / sum;
+    }
     float o0 = 0.0f, o1 = 0.0f;
     for (int j = 0; j < S; ++j) {
         const float* vp = qkv + (row0 + j) * 3 * Hd + 2 * Hd + h * 64;
@@ -358,7 +364,7 @@ int fp32_cnn_encoder(const RawTable& t, const Fp32Opts& o, Fp32Arena* ws, const 
 
 int fp32_text_encoder(const RawTable& t, const Fp32Opts& o, Fp32Arena* ws, const long long* ids,
                       const void* mask, int mask_dtype, int B, int S, float* cls, float* last_hidden,
-                      float* all_hidden, cudaStream_t s) {
+                      float* all_hidden, float* attn_probs, cudaStream_t s) {
     const std::string e = "text_encoder.encoder.embeddings.";
     const RawTensor *we, *pe, *te;
     F32_TRY(need(t, e + "word_embeddings.weight", &we));
@@ -410,7 +416,8 @@ int fp32_text_encoder(const RawTable& t, const Fp32Opts& o, Fp32Arena* ws, const
         F32_TRY(linear(t, p + "attention.self.value", h, Hd, static_cast<int>(T), qkv + 2 * Hd, 3 * Hd,
                        MRD_ACT_NONE, nullptr, 0, s));
         attention_f32_kernel<<<dim3(B * heads, (S + nw - 1) / nw), nw * 32, nw * (S + 64) * sizeof(float), s>>>(
-            qkv, mask ? bias : nullptr, S, heads, 0.125f, ctx);
+            qkv, mask ? bias : nullptr, S, heads, 0.125f, ctx,
+            attn_probs ? attn_probs + static_cast<long long>(i) * B * heads * S * S : nullptr);
         F32_TRY(check_launch("attention_f32"));
         // BertSelfOutput: LayerNorm(dense(ctx) + hidden) (HF:294-298)
         F32_TRY(linear(t, p + "attention.output.dense", ctx, Hd, static_cast<int>(T), tmp, Hd, MRD_ACT_NONE,
@@ -765,7 +772,7 @@ int fp32_bert_train_forward(const RawTable& t, const Fp32Opts& o, Fp32TrainSave*
         F32_TRY(linear(t, p + "attention.self.key", sv->x[i], Hd, Ti, sv->qkv[i] + Hd, 3 * Hd, MRD_ACT_NONE, nullptr, 0, s));
         F32_TRY(linear(t, p + "attention.self.value", sv->x[i], Hd, Ti, sv->qkv[i] + 2 * Hd, 3 * Hd, MRD_ACT_NONE, nullptr, 0, s));
         attention_f32_kernel<<<dim3(B * heads, (S + nw - 1) / nw), nw * 32, nw * (S + 64) * sizeof(float), s>>>(
-            sv->qkv[i], kb, S, heads, 0.125f, sv->ctx[i]);
+            sv->qkv[i], kb, S, heads, 0.125f, sv->ctx[i], nullptr);
         F32_TRY(check_launch("attention_f32"));
         // s1 = dense(ctx) + x ; h1 = LayerNorm(s1)   (HF:294-298)
         F32_TRY(linear(t, p + "attention.output.dense", sv->ctx[i], Hd, Ti, sv->s1[i], Hd, MRD_ACT_NONE, sv->x[i], Hd, s));

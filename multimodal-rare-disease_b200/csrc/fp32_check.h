@@ -41,7 +41,7 @@ int fp32_cnn_encoder(const RawTable& t, const Fp32Opts& o, Fp32Arena* ws, const 
                      int H, int W, float* emb, float* pooled, float* fmap, cudaStream_t s);
 int fp32_text_encoder(const RawTable& t, const Fp32Opts& o, Fp32Arena* ws, const long long* ids,
                       const void* mask, int mask_dtype, int B, int S, float* cls, float* last_hidden,
-                      float* all_hidden, cudaStream_t s);
+                      float* all_hidden, float* attn_probs, cudaStream_t s);
 int fp32_fusion(const RawTable& t, const Fp32Opts& o, Fp32Arena* ws, const float* img, const float* txt,
                 int B, float* fused, float* attn_i2t, float* attn_t2i, cudaStream_t s);
 int fp32_head(const RawTable& t, const Fp32Opts& o, Fp32Arena* ws, const float* x, int B, float* logits,

@@ -165,6 +165,14 @@ __device__ __forceinline__ void tma_prefetch_5d(const void* map, int c0, int c1,
                  : "memory");
 }
 
+__device__ __forceinline__ void tma_store_3d(const void* map, uint32_t src, int c0, int c1, int c2) {
+    asm volatile(
+        "cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::
+            "l"(reinterpret_cast<uint64_t>(map)),
+        "r"(src), "r"(c0), "r"(c1), "r"(c2)
+        : "memory");
+}
+
 __device__ __forceinline__ void tma_store_4d(const void* map, uint32_t src, int c0, int c1,
                                              int c2, int c3) {
     asm volatile(

@@ -220,21 +220,29 @@ class Engine:
         return emb, pooled, fmap
 
     def text_encoder(self, input_ids, attention_mask, hidden: int = 768, want_hidden=False,
-                     all_layers: int = 0):
-        """all_layers = L > 0 additionally returns the [L+1,B,S,hidden] stack of hidden states."""
+                     all_layers: int = 0, want_attn=False, layers: int = 12, heads: int = 12):
+        """all_layers = L > 0 additionally returns the [L+1,B,S,hidden] stack of hidden states.
+        want_attn additionally returns every layer's attention probabilities, f32 [layers,B,heads,S,S]
+        (layers / heads: those of the loaded encoder); it comes last in the returned tuple."""
         ids, mask, code = self._text(input_ids, attention_mask)
         B, S = ids.shape
         cls = self._f32(B, hidden)
         last = self._f32(B, S, hidden) if (want_hidden or all_layers) else None
         stack = self._f32(all_layers + 1, B, S, hidden) if all_layers else None
+        attn = self._f32(layers, B, heads, S, S) if want_attn else None
         if B:
             with torch.cuda.device(self.device):
-                _lib.check(self.lib.mrd_text_encoder_fwd(self._ctx, ids.data_ptr(), _ptr(mask), code,
-                                                         B, S, cls.data_ptr(), _ptr(last), _ptr(stack),
-                                                         _stream(self.device)), "mrd_text_encoder_fwd")
-        if all_layers:
-            return cls, last, stack
-        return cls, last
+                if want_attn:
+                    _lib.check(self.lib.mrd_text_encoder_fwd_ex(self._ctx, ids.data_ptr(), _ptr(mask), code, B, S,
+                                                                cls.data_ptr(), _ptr(last), _ptr(stack),
+                                                                attn.data_ptr(), _stream(self.device)),
+                               "mrd_text_encoder_fwd_ex")
+                else:
+                    _lib.check(self.lib.mrd_text_encoder_fwd(self._ctx, ids.data_ptr(), _ptr(mask), code,
+                                                             B, S, cls.data_ptr(), _ptr(last), _ptr(stack),
+                                                             _stream(self.device)), "mrd_text_encoder_fwd")
+        out = (cls, last, stack) if all_layers else (cls, last)
+        return out + (attn,) if want_attn else out
 
     def fusion(self, img_emb, txt_emb, hidden_dim: int, heads: int):
         if img_emb.dim() != 2 or txt_emb.dim() != 2 or img_emb.shape[0] != txt_emb.shape[0]:

@@ -98,9 +98,30 @@ class TextEncoder(B200Module):
         return last
 
     def get_attention_weights(self, input_ids, attention_mask) -> Tuple[torch.Tensor, tuple]:
-        """(embedding, attentions).  With the installed transformers (sdpa attention) the reference
-        returns an EMPTY attentions tuple here (SURVEY.md section 8(f).3); so does this."""
-        return self.forward(input_ids, attention_mask), ()
+        """(embedding, attentions) - src/text_encoder.py:151-179.  What the reference returns depends on
+        the attention backend of the HF encoder, and so does this:
+
+        * "sdpa" (the default) or any other non-eager backend: HF ignores output_attentions, the
+          attentions tuple is EMPTY, and the embedding is forward()'s.
+        * "eager" (`encoder.set_attn_implementation("eager")` or `attn_implementation="eager"`): one fp32
+          [B, heads, S, S] tensor per layer, views of one [layers, B, heads, S, S] buffer.  Element
+          [b,h,q,k] = softmax_k(q.k/8 + mask bias) (HF:models/bert/modeling_bert.py:115-140, eval mode),
+          for every query row, padded positions included; masked keys are exactly 0 and
+          attention_mask=None attends every key.  The embedding is bitwise what forward() returns.
+          A sample without any attended key gets all-zero rows, not HF's uniform 1/S rows: the B200
+          forward gives such a sample a zero attention output, and the probabilities agree with it.
+          Memory: layers * B * heads * S^2 * 4 bytes (as in the reference), e.g. 604 MB for B=64, S=128
+          and 9.7 GB for B=64, S=512 with BERT-base.
+
+        Eval mode only (train mode raises NotImplementedError, like every accessor here)."""
+        if getattr(self.encoder.config, "_attn_implementation", None) != "eager":
+            return self.forward(input_ids, attention_mask), ()
+        self._check()
+        eng = self._engine()
+        cfg = self.encoder.config
+        cls, _, attn = eng.text_encoder(input_ids, attention_mask, self.embedding_dim, want_attn=True,
+                                        layers=len(self.encoder.encoder.layer), heads=cfg.num_attention_heads)
+        return cls, tuple(attn.unbind(0))
 
 
 class BioBERTEncoder(TextEncoder):
