@@ -320,6 +320,52 @@ int mrd_train_backward_begin(mrd_ctx* ctx, const float* dlogits, int n, const ch
 int mrd_train_backward_stages(mrd_ctx* ctx, int first, int last, void* stream);
 int mrd_train_backward_num_stages(mrd_ctx* ctx);
 
+/* Data gradients through the frozen ResNet50 backbone: d(loss)/d(images) (input saliency, SmoothGrad, integrated
+ * gradients) and the tensors forward / backward hooks on backbone.layer1..layer4 and on every Bottleneck receive.
+ * The backbone's BatchNorm must use running statistics ("train.bn_train" 0) and the fp32 check mode must be off.
+ * Bottlenecks are numbered 0..15 in forward order (layer1.0 = 0, layer4.2 = 15).
+ *
+ * mrd_train_forward_dg = mrd_train_forward_ex (without feat_map) that also keeps every activation the backbone's
+ * backward needs: the stem output before the max-pool, the max-pool output and, per bottleneck, relu(bn1(conv1 x)),
+ * relu(bn2(conv2 .)) and the block output, bf16 NHWC.  9.8 M elements = 19.6 MB per 224 x 224 image, plus 7.6 MB of
+ * backward scratch; B <= 512.  block_out (optional, 16 slots, NULL = not wanted): f32 NCHW [B, C_k, h_k, w_k], the
+ * output of bottleneck k (slot 15 = the layer4 map).
+ *
+ * mrd_train_backward_dg = mrd_train_backward_ex after a mrd_train_forward_dg, continued through the backbone: d_pooled
+ * is optional here (internal scratch when NULL).  Bottlenecks 15 .. first_block run backward (first_block = 16: none,
+ * 0: all).  block_grads (optional, 16 slots) receives d(loss)/d(output of bottleneck k), f32 NCHW, for
+ * first_block - 1 <= k < 15; slot 15 is d_pooled / (h*w) at every position and is not written.  d_block_in (optional)
+ * = d(loss)/d(input of bottleneck first_block), f32 NCHW (for first_block 0: the max-pool output).  d_images
+ * (optional, needs first_block == 0) = d(loss)/d(images), f32 [B,3,H,W], through the max-pool and the stem. */
+int mrd_train_forward_dg(mrd_ctx* ctx, const void* images, int img_dtype, const long long* ids,
+                         const void* mask, int mask_dtype, int B, int H, int W, int S,
+                         unsigned long long seed, float* logits, float* const* block_out, float* img_emb,
+                         float* txt_emb, float* fused, void* stream);
+int mrd_train_backward_dg(mrd_ctx* ctx, const float* dlogits, int n, const char* const* names,
+                          float* const* grads, float* d_pooled, float* const* block_grads, int first_block,
+                          float* d_block_in, float* d_images, void* stream);
+
+/* The pieces of that backward, one entry each (unit tests).
+ * mrd_conv_dgrad_bf16: the data gradient of a convolution on the tcgen05 GEMM as a stride-1 tap convolution over
+ * dY [N,Ho,Wo,Cy] bf16: dX[n, sh*i+ph, sw*j+pw, :] = sum_t dY[n, i+tap_dh[t], j+tap_dw[t], :] Wt_t^T (dY outside
+ * the grid = 0), Wt: [Cx][ntaps*Cy] bf16 with row stride ldw, dX [N, sh*Ho, sw*Wo, Cx] bf16 (only the (ph, pw) phase
+ * is written).  aux: aux_mode 1 = added (may alias dX), 2 = ReLU mask (dX = result * [aux > 0]), 0 = none (NULL).
+ * Shifts in [-1, 1], ntaps <= 9, Cy and Cx multiples of 64.
+ * mrd_relu_mask_bf16: gz = g * [y > 0], n % 8 == 0.
+ * mrd_maxpool3x3s2_bwd_bf16: backward of MaxPool2d(3, 2, 1) fused with the ReLU in front of it: y [N,H,W,C] bf16 the
+ * pooled (post-ReLU) tensor, g [N,H/2,W/2,C] the gradient of the pool output, dx [N,H,W,C]; a window's gradient goes
+ * to its first maximum in row-major order, as in PyTorch.
+ * mrd_pack_stem_dgrad / mrd_stem_dgrad_f32: the stem filter [64,3,7,7] with BatchNorm (gamma, running_var, eps)
+ * folded into [7][7][64][3] f32; the 7x7 / stride-2 / pad-3 stem's data gradient d [N,H/2,W/2,64] bf16 -> f32 NCHW
+ * [N,3,H,W] (CUDA cores). */
+int mrd_conv_dgrad_bf16(const void* dY, int N, int Ho, int Wo, int Cy, const void* Wt, long long ldw, int ntaps,
+                        const int* tap_dh, const int* tap_dw, int Cx, void* dX, int sh, int sw, int ph, int pw,
+                        const void* aux, int aux_mode, void* stream);
+int mrd_relu_mask_bf16(const void* g, const void* y, long long n, void* gz, void* stream);
+int mrd_maxpool3x3s2_bwd_bf16(const void* g, const void* y, int N, int H, int W, int C, void* dx, void* stream);
+int mrd_pack_stem_dgrad(const float* w, const float* gamma, const float* var, float eps, float* out, void* stream);
+int mrd_stem_dgrad_f32(const void* d, const float* wf, int N, int H, int W, float* out, void* stream);
+
 /* out[i] = 1 if element i of dropout site `site` is kept under (seed, p), else 0 (i < n).  The masks
  * of mrd_train_forward are reproducible with this (tests; csrc/rng.cuh documents the site ids and the
  * element indexing). */

@@ -76,6 +76,14 @@ SIGNATURES = {
     "mrd_train_backward_begin": (_i, [_vp, _vp, _i, C.POINTER(C.c_char_p), C.POINTER(_vp), _vp]),
     "mrd_train_backward_stages": (_i, [_vp, _i, _i, _vp]),
     "mrd_train_backward_num_stages": (_i, [_vp]),
+    "mrd_train_forward_dg": (_i, [_vp, _vp, _i, _vp, _vp, _i, _i, _i, _i, _i, C.c_ulonglong, _vp, _vp, _vp, _vp, _vp,
+                                  _vp]),
+    "mrd_train_backward_dg": (_i, [_vp, _vp, _i, C.POINTER(C.c_char_p), C.POINTER(_vp), _vp, _vp, _i, _vp, _vp, _vp]),
+    "mrd_conv_dgrad_bf16": (_i, [_vp, _i, _i, _i, _i, _vp, _ll, _i, _vp, _vp, _i, _vp, _i, _i, _i, _i, _vp, _i, _vp]),
+    "mrd_relu_mask_bf16": (_i, [_vp, _vp, _ll, _vp, _vp]),
+    "mrd_maxpool3x3s2_bwd_bf16": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp]),
+    "mrd_pack_stem_dgrad": (_i, [_vp, _vp, _vp, _f, _vp, _vp]),
+    "mrd_stem_dgrad_f32": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
     "mrd_dropout_mask": (_i, [C.c_ulonglong, C.c_uint, _d, _ll, _vp, _vp]),
     "mrd_attention_train_bf16": (_i, [_vp, _vp, _i, _i, _i, C.c_ulonglong, C.c_uint, _d, _vp, _vp]),
     "mrd_attention_bwd_bf16": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, C.c_ulonglong, C.c_uint, _d, _vp, _vp,

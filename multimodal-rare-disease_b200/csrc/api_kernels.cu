@@ -6,6 +6,7 @@
 #include "elementwise.h"
 #include "attention.h"
 #include "conv_chain.h"
+#include "dgrad.h"
 #include "gemm_conv.h"
 #include "tma_host.h"
 #include "train_kernels.h"
@@ -69,6 +70,47 @@ int mrd_conv2d_nhwc_bf16(const void* X, int N, int H, int W, int Cin, const void
                        act, out_pad);
     if (rc) return rc;
     return launch_gemm(&g, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_conv_dgrad_bf16(const void* dY, int N, int Ho, int Wo, int Cy, const void* Wt, long long ldw, int ntaps,
+                        const int* tap_dh, const int* tap_dw, int Cx, void* dX, int sh, int sw, int ph, int pw,
+                        const void* aux, int aux_mode, void* stream) {
+    if (ntaps < 1 || ntaps > 9 || !tap_dh || !tap_dw) {
+        set_last_error("mrd_conv_dgrad_bf16: 1..9 taps with their shifts required");
+        return -1;
+    }
+    TapDesc taps[9];
+    for (int t = 0; t < ntaps; ++t) {
+        if (tap_dh[t] < -1 || tap_dh[t] > 1 || tap_dw[t] < -1 || tap_dw[t] > 1) {
+            set_last_error("mrd_conv_dgrad_bf16: tap shifts must lie in [-1, 1]");
+            return -1;
+        }
+        taps[t] = TapDesc{0, static_cast<int8_t>(tap_dh[t]), static_cast<int8_t>(tap_dw[t]), 0};
+    }
+    GemmLaunch g;
+    int rc = plan_conv_dgrad(&g, static_cast<const __nv_bfloat16*>(dY), N, Ho, Wo, Cy,
+                             static_cast<const __nv_bfloat16*>(Wt), ldw, ntaps, taps, Cx, static_cast<__nv_bfloat16*>(dX),
+                             sh, sw, ph, pw, static_cast<const __nv_bfloat16*>(aux), aux_mode);
+    if (rc) return rc;
+    return launch_gemm(&g, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_relu_mask_bf16(const void* g, const void* y, long long n, void* gz, void* stream) {
+    return relu_mask_bf16(static_cast<const __nv_bfloat16*>(g), static_cast<const __nv_bfloat16*>(y), n,
+                          static_cast<__nv_bfloat16*>(gz), static_cast<cudaStream_t>(stream));
+}
+
+int mrd_maxpool3x3s2_bwd_bf16(const void* g, const void* y, int N, int H, int W, int C, void* dx, void* stream) {
+    return maxpool3x3s2_bwd_relu(static_cast<const __nv_bfloat16*>(g), static_cast<const __nv_bfloat16*>(y), N, H, W,
+                                 C, static_cast<__nv_bfloat16*>(dx), static_cast<cudaStream_t>(stream));
+}
+
+int mrd_pack_stem_dgrad(const float* w, const float* gamma, const float* var, float eps, float* out, void* stream) {
+    return pack_stem_dgrad(w, gamma, var, eps, out, static_cast<cudaStream_t>(stream));
+}
+
+int mrd_stem_dgrad_f32(const void* d, const float* wf, int N, int H, int W, float* out, void* stream) {
+    return stem_dgrad_nchw(static_cast<const __nv_bfloat16*>(d), wf, N, H, W, out, static_cast<cudaStream_t>(stream));
 }
 
 int mrd_conv1x1_dual_bf16(const void* X0, int C0, const void* X1, int C1, int stride, int N, int Ho, int Wo,

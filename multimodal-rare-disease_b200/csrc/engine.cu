@@ -25,6 +25,7 @@
 
 #include "attention.h"
 #include "conv_chain.h"
+#include "dgrad.h"
 #include "elementwise.h"
 #include "fp32_check.h"
 #include "gemm_conv.h"
@@ -1312,6 +1313,7 @@ int check_ctx(mrd_ctx* c) {
 }
 
 #include "engine_train.cuh"
+#include "engine_dgrad.cuh"
 
 int fp32_images_only(int img_dtype) {
     if (img_dtype != MRD_DT_F32) {
@@ -1732,6 +1734,41 @@ int mrd_train_backward_num_stages(mrd_ctx* c) {
 int mrd_train_backward(mrd_ctx* c, const float* dlogits, int n, const char* const* names, float* const* grads,
                        void* stream) {
     return mrd_train_backward_ex(c, dlogits, n, names, grads, nullptr, stream);
+}
+
+int mrd_train_forward_dg(mrd_ctx* c, const void* images, int img_dtype, const long long* ids, const void* mask,
+                         int mask_dtype, int B, int H, int W, int S, unsigned long long seed, float* logits,
+                         float* const* block_out, float* img_emb, float* txt_emb, float* fused, void* stream) {
+    MRD_TRY(check_ctx(c));
+    if (B <= 0) return 0;
+    TrainState* t = train_state(c);
+    t->dg_save = true;
+    t->dg_block_out = block_out;
+    const int rc = mrd_train_forward_ex(c, images, img_dtype, ids, mask, mask_dtype, B, H, W, S, seed, logits, nullptr,
+                                        img_emb, txt_emb, fused, stream);
+    t->dg_save = false;
+    t->dg_block_out = nullptr;
+    return rc;
+}
+
+int mrd_train_backward_dg(mrd_ctx* c, const float* dlogits, int n, const char* const* names, float* const* grads,
+                          float* d_pooled, float* const* block_grads, int first_block, float* d_block_in,
+                          float* d_images, void* stream) {
+    MRD_TRY(check_ctx(c));
+    DgradCnn* d = c->train ? c->train->dg : nullptr;
+    if (!d || !d->valid) {
+        set_last_error("mrd_train_backward_dg: the pending forward was not a mrd_train_forward_dg");
+        return -1;
+    }
+    float* dp = d_pooled ? d_pooled : d->d_pooled;
+    if (!d_pooled) {
+        cudaError_t e = cudaMemsetAsync(dp, 0, sizeof(float) * d->B * c->feat_dim, static_cast<cudaStream_t>(stream));
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(d_pooled)");
+    }
+    MRD_TRY(mrd_train_backward_ex(c, dlogits, n, names, grads, dp, stream));
+    static float* const kNone[16] = {};
+    return dgrad_backbone(c, dp, block_grads ? block_grads : kNone, first_block, d_block_in, d_images,
+                          static_cast<cudaStream_t>(stream));
 }
 
 int mrd_dropout_mask(unsigned long long seed, unsigned int site, double p, long long n, float* out, void* stream) {

@@ -45,10 +45,14 @@ struct TrainLayerPlan {
 };
 
 struct TrainCnn;
+struct DgradCnn;
 
 struct TrainState {
     TrainOpts o;
     TrainCnn* cnn = nullptr;              // batch-statistics backbone (created when bn_train is first used)
+    DgradCnn* dg = nullptr;               // data gradients through the backbone (engine_dgrad.cuh), created on first use
+    float* const* dg_block_out = nullptr; // set by mrd_train_forward_dg for one forward: save for data gradients,
+    bool dg_save = false;                 // and the optional per-block output maps
     std::vector<TrainLayerWt> wt;
     bool packs_valid = false;
     // plan / workspace for one (B, S)
@@ -96,6 +100,11 @@ TrainState* train_state(mrd_ctx* c) {
 
 void train_cnn_invalidate(TrainState* t);
 void train_cnn_free(TrainState* t);
+void dgrad_invalidate(TrainState* t);
+void dgrad_forget(TrainState* t);
+void dgrad_free(TrainState* t);
+int run_backbone_save(mrd_ctx* c, const void* images, int img_dtype, int B, int H, int W, float* pooled_f32,
+                      float* const* block_out, cudaStream_t s);
 
 void train_invalidate_packs(mrd_ctx* c, bool text, bool backbone) {
     if (!c->train) return;
@@ -490,10 +499,12 @@ int run_backbone_train(mrd_ctx* c, const void* images, int img_dtype, int B, int
 
 void train_cnn_invalidate(TrainState* t) {
     if (t->cnn) t->cnn->packed = false;
+    dgrad_invalidate(t);
 }
 void train_cnn_free(TrainState* t) {
     delete t->cnn;   // device buffers are weight allocations of the context (freed with it)
     t->cnn = nullptr;
+    dgrad_free(t);
 }
 
 typedef std::unordered_map<std::string, float*> GradTable;
@@ -588,8 +599,14 @@ int train_forward(mrd_ctx* c, const void* images, int img_dtype, const long long
     t->fwd_done = false;
     t->seed = seed;
     t->ids = ids;
+    dgrad_forget(t);   // a saving forward re-validates its activations
     const int T = B * S;
 
+    if (t->dg_save && (c->fp32_check || o.bn_train || feat_map)) {
+        set_last_error("data gradients: need the bf16 path (no fp32 check) and the backbone's BatchNorm on running "
+                       "statistics (train.bn_train = 0); the layer4 map is block output 15");
+        return -1;
+    }
     if (c->fp32_check) {
         // fp32 check of the training step: backbone and text encoder in plain fp32 (fp32_check.cu), dropout off;
         // the batch-level layers below are fp32 in either mode
@@ -617,6 +634,8 @@ int train_forward(mrd_ctx* c, const void* images, int img_dtype, const long long
             return -1;
         }
         MRD_TRY(run_backbone_train(c, images, img_dtype, B, H, W, t->pooled, s));
+    } else if (t->dg_save) {
+        MRD_TRY(run_backbone_save(c, images, img_dtype, B, H, W, t->pooled, t->dg_block_out, s));
     } else {
         MRD_TRY(run_backbone(c, images, img_dtype, B, H, W, t->pooled, feat_map, s));
     }

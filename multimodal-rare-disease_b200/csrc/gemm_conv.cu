@@ -89,6 +89,9 @@ __device__ __forceinline__ TileCoord decode_tile(const ConvGemmParams& p, int ti
 // one binary serves the compute-bound GEMMs (deep operand pipeline, no residual ring) and the
 // memory-bound short-K convolutions with residual (shallow operand pipeline, deep residual ring)):
 //   [stages x A_STAGE][stages x B_STAGE][2 x 16 KB store staging][ring x 16 KB residual][barriers]
+// MASK (generic mode, single-group epilogue; plan_conv_dgrad): the tile fetched through r_map is not added but used as
+// a ReLU mask - out = acc * [r > 0] - the backward of a ReLU whose output r was saved by the forward.  Separate
+// instantiations for the same reason as SPLITK: a run-time branch in the shared epilogue costs the forward's kernels.
 // SPLITK (generic mode only) is a separate instantiation so that the forward's kernels compile exactly as they
 // did before split-K existed: measured, the merged version cost the forward 3 % (different epilogue schedule).
 // EPI2: the eight epilogue warps work as two independent groups of four (one warp per TMEM lane quarter each); group g
@@ -120,7 +123,8 @@ constexpr int kLnStripeBytes = 128 * 8 * 8 + 64;
 // warps hand an accumulator back by arriving on the LEADER's `tempty` barrier.  (Measured first: only multicasting the
 // weight tile into both CTAs, each still issuing its own 128 x 256 MMAs, changed nothing - the bytes into each SM
 // stayed the same.)
-template <int BLOCK_N, int MODE, bool SPLITK = false, bool EPI2 = false, bool LNC = false, bool PAIR = false>
+template <int BLOCK_N, int MODE, bool SPLITK = false, bool EPI2 = false, bool LNC = false, bool PAIR = false,
+          bool MASK = false>
 __global__ void __launch_bounds__(kNumThreads, 1)
 conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
     using C = Cfg<BLOCK_N, MODE>;
@@ -899,10 +903,17 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
                     const uint4 r4 = *reinterpret_cast<const uint4*>(r_row + chunk * 16);
                     const float2 r0 = unpack_bf16(r4.x), r1 = unpack_bf16(r4.y),
                                  r2 = unpack_bf16(r4.z), r3 = unpack_bf16(r4.w);
-                    f[c * 8 + 0] += r0.x; f[c * 8 + 1] += r0.y;
-                    f[c * 8 + 2] += r1.x; f[c * 8 + 3] += r1.y;
-                    f[c * 8 + 4] += r2.x; f[c * 8 + 5] += r2.y;
-                    f[c * 8 + 6] += r3.x; f[c * 8 + 7] += r3.y;
+                    if constexpr (MASK) {   // ReLU backward: keep the positions whose saved activation is > 0
+                        f[c * 8 + 0] = r0.x > 0.0f ? f[c * 8 + 0] : 0.0f; f[c * 8 + 1] = r0.y > 0.0f ? f[c * 8 + 1] : 0.0f;
+                        f[c * 8 + 2] = r1.x > 0.0f ? f[c * 8 + 2] : 0.0f; f[c * 8 + 3] = r1.y > 0.0f ? f[c * 8 + 3] : 0.0f;
+                        f[c * 8 + 4] = r2.x > 0.0f ? f[c * 8 + 4] : 0.0f; f[c * 8 + 5] = r2.y > 0.0f ? f[c * 8 + 5] : 0.0f;
+                        f[c * 8 + 6] = r3.x > 0.0f ? f[c * 8 + 6] : 0.0f; f[c * 8 + 7] = r3.y > 0.0f ? f[c * 8 + 7] : 0.0f;
+                    } else {
+                        f[c * 8 + 0] += r0.x; f[c * 8 + 1] += r0.y;
+                        f[c * 8 + 2] += r1.x; f[c * 8 + 3] += r1.y;
+                        f[c * 8 + 4] += r2.x; f[c * 8 + 5] += r2.y;
+                        f[c * 8 + 6] += r3.x; f[c * 8 + 7] += r3.y;
+                    }
                 }
             }
             if (p.act == ACT_RELU) {
@@ -978,11 +989,12 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
     }
 }
 
-template <int BLOCK_N, int MODE, bool SPLITK = false, bool EPI2 = false, bool LNC = false, bool PAIR = false>
+template <int BLOCK_N, int MODE, bool SPLITK = false, bool EPI2 = false, bool LNC = false, bool PAIR = false,
+          bool MASK = false>
 int launch_variant(const GemmLaunch* g, cudaStream_t stream) {
     using C = Cfg<BLOCK_N, MODE>;
     static bool attr_set = false;
-    auto kfn = conv_gemm_kernel<BLOCK_N, MODE, SPLITK, EPI2, LNC, PAIR>;
+    auto kfn = conv_gemm_kernel<BLOCK_N, MODE, SPLITK, EPI2, LNC, PAIR, MASK>;
     if (!attr_set) {
         cudaError_t e =
             cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit);
@@ -1690,6 +1702,83 @@ int plan_stem_pool(GemmLaunch* g, const __nv_bfloat16* Xpad, int N, int H, int W
     return 0;
 }
 
+int plan_conv_dgrad(GemmLaunch* g, const __nv_bfloat16* dY, int N, int Ho, int Wo, int Cy, const __nv_bfloat16* Wt,
+                    long long ldw, int ntaps, const TapDesc* taps, int Cx, __nv_bfloat16* dX, int sh, int sw, int ph,
+                    int pw, const __nv_bfloat16* aux, int aux_mode) {
+    memset(g, 0, sizeof(*g));
+    if (N <= 0 || Ho <= 0 || Wo <= 0 || Cy % 64 != 0 || Cx % 64 != 0 || ntaps < 1 || ntaps > 9 || sh < 1 ||
+        sh > 2 || sw < 1 || sw > 2 || ph < 0 || ph >= sh || pw < 0 || pw >= sw || ldw % 8 != 0 ||
+        ldw < 1LL * ntaps * Cy || aux_mode < 0 || aux_mode > 2 || (aux_mode != 0) != (aux != nullptr)) {
+        set_last_error("plan_conv_dgrad: unsupported N=%d %dx%d Cy=%d Cx=%d taps=%d stride %dx%d phase (%d,%d) aux %d",
+                       N, Ho, Wo, Cy, Cx, ntaps, sh, sw, ph, pw, aux_mode);
+        return -1;
+    }
+    for (int t = 0; t < ntaps; ++t)
+        if (taps[t].dh < -1 || taps[t].dh > 1 || taps[t].dw < -1 || taps[t].dw > 1) {
+            set_last_error("plan_conv_dgrad: tap shifts must lie in [-1, 1]");
+            return -1;
+        }
+    ConvGemmParams& p = g->p;
+    const int Hx = sh * Ho, Wx = sw * Wo;
+    p.bias = nullptr;
+    p.has_res = aux != nullptr;
+    p.num_taps = ntaps;
+    p.kc_per_tap = Cy / 64;
+    for (int t = 0; t < ntaps; ++t) p.taps[t] = TapDesc{0, taps[t].dh, taps[t].dw, 0};
+    p.Wo = Wo; p.Ho = Ho; p.Nimg = N; p.Cout = Cx;
+    p.act = ACT_NONE;
+    p.store_bf16 = 1;
+    g->relu_mask = aux_mode == 2;
+    g->flops = 2.0 * N * Ho * Wo * static_cast<double>(Cx) * Cy * ntaps;
+    g->bytes = 2.0 * (1.0 * N * Ho * Wo * Cy + 1.0 * Cx * Cy * ntaps + 1.0 * N * Ho * Wo * Cx * (aux ? 2.0 : 1.0));
+    // tile box as plan_conv: whole rows, then whole images, of the dY grid
+    p.tw = Wo < 128 ? Wo : 128;
+    p.th = 128 / p.tw;
+    if (p.th > Ho) p.th = Ho;
+    if (p.th < 1) p.th = 1;
+    p.nb = 1;
+    if (p.th == Ho && p.tw == Wo) {
+        p.nb = 128 / (p.tw * p.th);
+        if (p.nb < 1) p.nb = 1;
+        if (p.nb > N) p.nb = N;
+    }
+    p.tiles_w = (Wo + p.tw - 1) / p.tw;
+    p.tiles_h = (Ho + p.th - 1) / p.th;
+    p.tiles_img = (N + p.nb - 1) / p.nb;
+    {   // dY rows / columns shifted outside the grid are zero-filled by TMA (the far edge of a transposed convolution)
+        uint64_t dims[4] = {(uint64_t)Cy, (uint64_t)Wo, (uint64_t)Ho, (uint64_t)N};
+        uint64_t str[3] = {(uint64_t)Cy * 2, (uint64_t)Wo * Cy * 2, (uint64_t)Ho * Wo * Cy * 2};
+        uint32_t box[4] = {64, (uint32_t)p.tw, (uint32_t)p.th, (uint32_t)p.nb};
+        int rc = encode_tensor_map(&p.a_map[0], dY, 2, 4, dims, str, box, 128);
+        if (rc) return rc;
+        for (int i = 1; i < 4; ++i) p.a_map[i] = p.a_map[0];
+    }
+    const long long m_tiles = static_cast<long long>(p.tiles_w) * p.tiles_h * p.tiles_img;
+    const int bn = pick_block_n(Cx, m_tiles, gemm_num_sms());
+    g->pair = (bn == 256 && m_tiles * (Cx / 256) >= 2LL * gemm_num_sms()) ? 1 : 0;
+    {
+        uint64_t dims[2] = {(uint64_t)ntaps * Cy, (uint64_t)Cx};
+        uint64_t str[1] = {(uint64_t)ldw * 2};
+        uint32_t box[2] = {64, (uint32_t)(g->pair ? bn / 2 : bn)};
+        int rc = encode_tensor_map(&p.b_map, Wt, 2, 2, dims, str, box, 128);
+        if (rc) return rc;
+    }
+    {   // the (ph, pw) phase of dX as a [N][Ho][Wo][Cx] view; the mask / addend through the same view
+        const long long off = (static_cast<long long>(ph) * Wx + pw) * Cx;
+        uint64_t dims[4] = {(uint64_t)Cx, (uint64_t)Wo, (uint64_t)Ho, (uint64_t)N};
+        uint64_t str[3] = {(uint64_t)sw * Cx * 2, (uint64_t)sh * Wx * Cx * 2, (uint64_t)Hx * Wx * Cx * 2};
+        uint32_t box[4] = {64, (uint32_t)p.tw, (uint32_t)p.th, (uint32_t)p.nb};
+        int rc = encode_tensor_map(&p.c_map, dX + off, 2, 4, dims, str, box, 128);
+        if (rc) return rc;
+        p.r_map = p.c_map;
+        if (aux) {
+            rc = encode_tensor_map(&p.r_map, aux + off, 2, 4, dims, str, box, 128);
+            if (rc) return rc;
+        }
+    }
+    return finish_plan(g, bn);
+}
+
 int launch_gemm(const GemmLaunch* g, cudaStream_t stream) {
     apply_debug_env();
     if (g->stem) {
@@ -1709,6 +1798,16 @@ int launch_gemm(const GemmLaunch* g, cudaStream_t stream) {
             case 128: return launch_variant<128, MODE_FLAT3, false, true>(g, stream);
         }
         set_last_error("launch_gemm: bad flat3 block_n %d", g->block_n);
+        return -1;
+    }
+    if (g->relu_mask) {   // plan_conv_dgrad with a ReLU mask: single-group epilogue only
+        if (g->pair && g->block_n == 256) return launch_variant<256, MODE_GENERIC, false, false, false, true, true>(g, stream);
+        switch (g->block_n) {
+            case 64: return launch_variant<64, MODE_GENERIC, false, false, false, false, true>(g, stream);
+            case 128: return launch_variant<128, MODE_GENERIC, false, false, false, false, true>(g, stream);
+            case 256: return launch_variant<256, MODE_GENERIC, false, false, false, false, true>(g, stream);
+        }
+        set_last_error("launch_gemm: bad masked block_n %d", g->block_n);
         return -1;
     }
     if (g->p.f32_accum) {   // plan_gemm_splitk

@@ -85,6 +85,7 @@ struct GemmLaunch {
     int grid;
     double flops;  // algorithmic FLOPs (2*M*N*K, un-padded), for reporting
     double bytes;  // algorithmic bytes: A + W read once, C written once (+ residual read)
+    int relu_mask; // 1: the r_map tile masks the result (plan_conv_dgrad, aux_mode 2) instead of being added
 };
 
 // Plain GEMM.  A: [M,K] bf16 with row stride lda; W: [N,K] bf16 (nn.Linear layout); C: [M,N] bf16
@@ -146,6 +147,21 @@ int plan_stem_pool(GemmLaunch* out, const __nv_bfloat16* Xpad, int N, int H, int
 // zero before the launch.  dyn_k: optional device int, the live part of K (<= K).
 int plan_gemm_splitk(GemmLaunch* out, const __nv_bfloat16* A, long long lda, int M, int K,
                      const __nv_bfloat16* W, int N, float* out_f32, long long ld_f32, const int* dyn_k);
+
+// Data gradient of a frozen convolution (the backward with respect to its input) as a stride-1 "tap convolution"
+// over the output-gradient grid, on the same tcgen05 kernel:
+//   dX[n, sh*i + ph, sw*j + pw, :] = sum_t dY[n, i + dh_t, j + dw_t, :] * Wt_t^T      (dY outside the grid = 0)
+// dY: [N,Ho,Wo,Cy] bf16.  Wt: [Cx][ntaps*Cy] bf16, tap-major along K, row stride ldw elements (a view may start at
+// any tap of a larger pack).  dX: [N, sh*Ho, sw*Wo, Cx] bf16, of which this launch writes the (ph, pw) phase only.
+//   1x1 stride 1: one tap (0,0), sh = sw = 1.   3x3 stride 1 pad 1: nine taps (r-1, s-1) with the filter flipped.
+//   3x3 stride 2 pad 1: one launch per output parity phase (1, 2, 2 or 4 taps with shifts 0 / +1).
+//   1x1 stride 2: one tap, phase (0,0) of a stride-2 view (the downsample branch scattered to the even pixels).
+// aux (optional, same phase view and shape as the written part of dX): aux_mode 1 = added to the result (aux may be
+// dX itself: every element is read before it is written, by the same CTA); 2 = ReLU mask, dX = result * [aux > 0].
+// Shifts in [-1, 1], Cy % 64 == 0, Cx % 64 == 0.
+int plan_conv_dgrad(GemmLaunch* out, const __nv_bfloat16* dY, int N, int Ho, int Wo, int Cy, const __nv_bfloat16* Wt,
+                    long long ldw, int ntaps, const TapDesc* taps, int Cx, __nv_bfloat16* dX, int sh, int sw, int ph,
+                    int pw, const __nv_bfloat16* aux, int aux_mode);
 
 int launch_gemm(const GemmLaunch* g, cudaStream_t stream);
 

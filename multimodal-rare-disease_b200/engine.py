@@ -49,6 +49,7 @@ class Engine:
         self.device = device
         self.train_serial = 0
         self.train_opts: Optional[Dict[str, float]] = None   # "train.*" options applied to THIS context
+        self.fp32_check = bool((options or {}).get("fp32_check", 0.0))
         self._sigs: Dict[str, tuple] = {}
         self._dirty = set()
         self._keep: Dict[str, list] = {}
@@ -77,6 +78,8 @@ class Engine:
         with torch.cuda.device(self.device):
             _lib.check(self.lib.mrd_ctx_set_option(self._ctx, key.encode(), float(value)),
                        f"mrd_ctx_set_option({key})")
+        if key == "fp32_check":
+            self.fp32_check = bool(value)
 
     def profile(self, enable: bool) -> None:
         with torch.cuda.device(self.device):
@@ -322,11 +325,13 @@ class Engine:
 
     # ------------------------------------------------------------------ training step
     def train_forward(self, images, input_ids, attention_mask, num_classes: int, seed: int,
-                      want_map: bool = False, emb_dims=None):
+                      want_map: bool = False, emb_dims=None, block_out=None):
         """Train-mode forward (dropout active, activations kept inside the context) -> logits f32 [B,C]
         (and, with want_map, the layer4 feature map f32 [B,2048,H/32,W/32] of this forward).
         emb_dims = (image, text, fused) widths: the three embeddings of this forward are kept in
-        self.last_train_embeddings (what return_embeddings=True hands out)."""
+        self.last_train_embeddings (what return_embeddings=True hands out).
+        block_out = 16 slots (f32 NCHW tensors or None), one per bottleneck: the forward also keeps what the backbone's
+        data-gradient backward needs (mrd_train_forward_dg) and writes the output of every bottleneck given a tensor."""
         images, icode = self._images(images)
         ids, mask, mcode = self._text(input_ids, attention_mask)
         B, _, H, W = images.shape
@@ -338,7 +343,14 @@ class Engine:
         self.last_train_embeddings = embs if emb_dims else None
         self._train_inputs = (images, ids, mask)   # the backward re-reads the ids
         self.train_serial = getattr(self, "train_serial", 0) + 1
-        if B:
+        if B and block_out is not None:
+            slots = (C.c_void_p * 16)(*[_ptr(t) for t in block_out])
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.mrd_train_forward_dg(
+                    self._ctx, images.data_ptr(), icode, ids.data_ptr(), _ptr(mask), mcode, B, H, W,
+                    ids.shape[1], C.c_ulonglong(seed & 0xFFFFFFFFFFFFFFFF), logits.data_ptr(), slots,
+                    _ptr(embs[0]), _ptr(embs[1]), _ptr(embs[2]), _stream(self.device)), "mrd_train_forward_dg")
+        elif B:
             with torch.cuda.device(self.device):
                 _lib.check(self.lib.mrd_train_forward_ex(
                     self._ctx, images.data_ptr(), icode, ids.data_ptr(), _ptr(mask), mcode, B, H, W,
@@ -355,14 +367,17 @@ class Engine:
             return n_layers + 1          # embeddings
         return 0                         # head, fusion, image projection
 
-    def train_backward(self, dlogits: torch.Tensor, named_shapes, want_dpooled: bool = False, on_bucket=None):
+    def train_backward(self, dlogits: torch.Tensor, named_shapes, want_dpooled: bool = False, on_bucket=None,
+                       dgrad=None):
         """named_shapes: [(canonical state_dict name, shape)] of the parameters that want a gradient.
         Returns their f32 gradients as views of ONE flat buffer, laid out in the order the backward completes
         them (head / fusion / projection, BERT layers last to first, embeddings); with want_dpooled also
         d(loss)/d(pooled backbone features) f32 [B,2048].
         on_bucket(flat_slice): data-parallel overlap - the backward is enqueued stage by stage and the callback
         receives each finished slice of the flat buffer right after its stage (it typically starts an
-        asynchronous all-reduce that then runs under the remaining stages)."""
+        asynchronous all-reduce that then runs under the remaining stages).
+        dgrad = (block_grads, first_block, d_block_in, d_images) after a forward with block_out: the backward continues
+        through the backbone (mrd_train_backward_dg); block_grads = 16 slots of f32 NCHW tensors or None."""
         dl = dlogits.to(self.device, torch.float32).contiguous()
         n_stages = int(self.lib.mrd_train_backward_num_stages(self._ctx))
         stage = [self._backward_stage_of(name, n_stages - 2) for name, _ in named_shapes]
@@ -388,7 +403,14 @@ class Engine:
         d_pooled = torch.zeros(dl.shape[0], 2048, dtype=torch.float32, device=self.device) if want_dpooled else None
         if dl.shape[0]:
             with torch.cuda.device(self.device):
-                if on_bucket is None:
+                if dgrad is not None:
+                    block_grads, first_block, d_block_in, d_images = dgrad
+                    slots = (C.c_void_p * 16)(*[_ptr(t) for t in block_grads])
+                    _lib.check(self.lib.mrd_train_backward_dg(self._ctx, dl.data_ptr(), n, names, ptrs, _ptr(d_pooled),
+                                                              slots, int(first_block), _ptr(d_block_in),
+                                                              _ptr(d_images), _stream(self.device)),
+                               "mrd_train_backward_dg")
+                elif on_bucket is None:
                     _lib.check(self.lib.mrd_train_backward_ex(self._ctx, dl.data_ptr(), n, names, ptrs,
                                                               _ptr(d_pooled), _stream(self.device)),
                                "mrd_train_backward")

@@ -32,12 +32,24 @@ class _TrainStep(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, eng, images, input_ids, attention_mask, seed, named_shapes, ddp, *params):
-        """ddp = (num_classes, data_parallel, process_group, hooked): hooked = the backbone module whose
-        forward / backward hooks are served (Grad-CAM on cnn_encoder.get_attention_layer()) or None."""
+        """ddp = (num_classes, data_parallel, process_group, hooked, emb_dims, dgrad): hooked = the backbone module
+        whose forward / backward hooks are served from the layer4 map (Grad-CAM on cnn_encoder.get_attention_layer())
+        or None; dgrad = a _DataGrad (data gradients through the backbone) or None."""
         ctx.eng, ctx.named_shapes, ctx.ddp = eng, named_shapes, ddp
         ctx.hooked = ddp[3] if len(ddp) > 3 else None
         emb_dims = ddp[4] if len(ddp) > 4 else None
-        if ctx.hooked is None:
+        ctx.dgrad = ddp[5] if len(ddp) > 5 else None
+        if ctx.dgrad is not None:
+            dg = ctx.dgrad
+            logits = eng.train_forward(images, input_ids, attention_mask, ddp[0], seed, emb_dims=emb_dims,
+                                       block_out=dg.block_out)
+            # forward hooks of the served modules, in forward order: the module's output (its last bottleneck's), NCHW
+            # fp32; the input tuple is empty as for layer4's hooks
+            for m, lo, hi in dg.hooked:
+                for hook in list(m._forward_hooks.values()):
+                    hook(m, (), dg.block_out[hi])
+            ctx.img_dtype = images.dtype
+        elif ctx.hooked is None:
             logits = eng.train_forward(images, input_ids, attention_mask, ddp[0], seed, emb_dims=emb_dims)
         else:
             logits, fmap = eng.train_forward(images, input_ids, attention_mask, ddp[0], seed, want_map=True,
@@ -57,6 +69,14 @@ class _TrainStep(torch.autograd.Function):
                 "backward through a train-mode forward whose saved activations were overwritten by a newer "
                 "train-mode forward of the same model: the B200 training step keeps ONE forward pending "
                 "(call backward before the next forward, as the reference's loops do)")
+        if ctx.dgrad is not None:
+            dg = ctx.dgrad
+            d_images = dg.new_images_grad() if dg.want_images else None
+            grads, d_pooled = ctx.eng.train_backward(dlogits, ctx.named_shapes, want_dpooled=True,
+                                                     dgrad=(dg.block_grads, dg.first, dg.d_in, d_images))
+            dg.serve_backward_hooks(d_pooled)
+            img_grad = d_images.to(ctx.img_dtype) if d_images is not None else None
+            return (None, img_grad) + (None,) * 5 + tuple(grads)
         if ctx.hooked is not None:
             grads, d_pooled = ctx.eng.train_backward(dlogits, ctx.named_shapes, want_dpooled=True)
             # AdaptiveAvgPool2d(1) backward (TV:models/resnet.py:278): every position of the layer4 map receives
@@ -78,6 +98,72 @@ class _TrainStep(torch.autograd.Function):
         else:
             grads = ctx.eng.train_backward(dlogits, ctx.named_shapes)
         return (None,) * 7 + tuple(grads)
+
+
+class _DataGrad:
+    """What one forward with data gradients through the backbone asks of the library: the bottleneck outputs the
+    forward hooks see, the point the backward chain stops at, and the buffers the backward hooks and images.grad read.
+    Bottlenecks are numbered 0..15 in forward order; a served module covers the bottlenecks [lo, hi]."""
+
+    def __init__(self, hooked, want_images, geometry, B, H, W, device):
+        self.hooked = hooked                  # [(module, lo, hi)] with hooks, in forward order
+        self.want_images = want_images
+        self.geometry = geometry              # per bottleneck: (C_in, h_in, w_in, C_out, h_out, w_out)
+        self.B, self.H, self.W, self.device = B, H, W, device
+        n = len(geometry)
+
+        def f32(*shape):
+            return torch.empty(*shape, dtype=torch.float32, device=device)
+
+        self.block_out = [None] * n
+        for m, lo, hi in hooked:
+            if m._forward_hooks and self.block_out[hi] is None:
+                _, _, _, c, h, w = geometry[hi]
+                self.block_out[hi] = f32(B, c, h, w)
+        # the chain runs down to the lowest point anything asks for: the image, or the output of a hooked module
+        stops = [0] if want_images else []
+        stops += [hi + 1 for m, lo, hi in hooked if m._backward_hooks]
+        self.first = min(stops) if stops else n
+        self.block_grads = [None] * n
+        self.d_in = None
+        for m, lo, hi in hooked:
+            if not m._backward_hooks:
+                continue
+            if hi < n - 1 and self.block_grads[hi] is None:
+                _, _, _, c, h, w = geometry[hi]
+                self.block_grads[hi] = f32(B, c, h, w)
+            if self.first <= lo:
+                if lo == self.first:
+                    if self.d_in is None:
+                        c, h, w = geometry[lo][:3]
+                        self.d_in = f32(B, c, h, w)
+                elif self.block_grads[lo - 1] is None:
+                    _, _, _, c, h, w = geometry[lo - 1]
+                    self.block_grads[lo - 1] = f32(B, c, h, w)
+
+    def new_images_grad(self):
+        return torch.empty(self.B, 3, self.H, self.W, dtype=torch.float32, device=self.device)
+
+    def serve_backward_hooks(self, d_pooled):
+        """Full backward hooks, innermost and highest first (the order autograd completes the modules' inputs):
+        grad_output = (d/d output,), grad_input = (d/d input,) where the chain ran below the module, else (None,)."""
+        n = len(self.geometry)
+        _, _, _, c, h, w = self.geometry[n - 1]
+        top = None
+        for m, lo, hi in sorted(self.hooked, key=lambda e: (-e[1], e[2])):
+            if not m._backward_hooks:
+                continue
+            if hi == n - 1:
+                if top is None:   # AdaptiveAvgPool2d(1) backward: d_pooled / (h*w) at every position of the layer4 map
+                    top = (d_pooled / float(h * w)).view(self.B, c, 1, 1).expand(self.B, c, h, w).contiguous()
+                g_out = top
+            else:
+                g_out = self.block_grads[hi]
+            g_in = None
+            if self.first <= lo:
+                g_in = self.d_in if lo == self.first else self.block_grads[lo - 1]
+            for hook in list(m._backward_hooks.values()):
+                hook(m, (g_in,), (g_out,))
 
 
 class ClassificationHead(B200Module):
@@ -163,13 +249,23 @@ class MultimodalClassifier(B200Module):
         """images [B,3,224,224], input_ids/attention_mask [B,S] -> {"logits","probs"} (+ embeddings
         and the fusion attention weights when return_embeddings=True), all fp32 on the model device."""
         self.text_encoder._check()
+        hooked, want_images = self._data_grad_request(images)
+        layer4 = self._hooked_attention_layer()
+        layer4_only = not want_images and len(hooked) == 1 and layer4 is not None and hooked[0][0] is layer4
+        dgrad = bool(want_images or hooked) and not layer4_only
         if self.training:
-            return self._forward_train(images, input_ids, attention_mask, return_embeddings)
-        hooked = self._hooked_attention_layer()
-        if hooked is not None:
+            # hooks on layer4 alone are not served in train mode (as before data gradients existed)
+            return self._forward_train(images, input_ids, attention_mask, return_embeddings,
+                                       dgrad=(hooked, want_images) if dgrad else None)
+        if dgrad:
+            # input saliency (images.requires_grad) and hooks below layer4: the eval-mode forward made differentiable
+            # down to the image
+            return self._forward_train(images, input_ids, attention_mask, return_embeddings,
+                                       dgrad=(hooked, want_images))
+        if layer4_only:
             # Grad-CAM (notebooks/explainability.ipynb cell 3): hooks on cnn_encoder.get_attention_layer() and
             # logits[0, c].backward() under model.eval() - the eval-mode forward made differentiable
-            return self._forward_train(images, input_ids, attention_mask, return_embeddings, explain=hooked)
+            return self._forward_train(images, input_ids, attention_mask, return_embeddings, explain=layer4)
         logits, probs, img_e, txt_e, fused, a1, a2 = self._engine().multimodal(
             images, input_ids, attention_mask, self._dims(), want_embeddings=return_embeddings,
             logits_out=logits_out)
@@ -190,6 +286,55 @@ class MultimodalClassifier(B200Module):
         except Exception:
             return None
         return m if (len(m._forward_hooks) or len(m._backward_hooks)) else None
+
+    def _served_modules(self):
+        """{id(module): (module, lo, hi)} of the backbone modules whose hooks are served - backbone.layer1..layer4 and
+        every Bottleneck backbone.layerN[i] - and the geometry of every bottleneck (see _DataGrad)."""
+        bb = self.cnn_encoder.backbone
+        served, blocks, k = {}, [], 0
+        for L in range(1, 5):
+            layer = getattr(bb, f"layer{L}")
+            lo = k
+            for blk in layer:
+                served[id(blk)] = (blk, k, k)
+                blocks.append(blk)
+                k += 1
+            served[id(layer)] = (layer, lo, k - 1)
+        return served, blocks
+
+    def _data_grad_request(self, images):
+        """([(module, lo, hi)] served modules with forward or backward hooks, in forward order; whether images.grad is
+        wanted).  A hook on any other module of the backbone raises: its tensors do not exist on the B200 path."""
+        bb = self.cnn_encoder.backbone
+        hooked_any = [(n, m) for n, m in bb.named_modules() if m._forward_hooks or m._backward_hooks]
+        want_images = torch.is_grad_enabled() and images.requires_grad
+        if not hooked_any:
+            return [], want_images
+        served, _ = self._served_modules()
+        hooked = []
+        for name, m in hooked_any:
+            if id(m) not in served:
+                where = "cnn_encoder.backbone" + ("." + name if name else "")
+                raise NotImplementedError(
+                    f"a forward / backward hook on {where} is not served on the B200 path: hooks are served on "
+                    "backbone.layer1 .. backbone.layer4 and on every Bottleneck backbone.layerN[i] (the intermediate "
+                    "tensors of the stem, of a block's convolutions and of the pooling are never materialised)")
+            hooked.append(served[id(m)])
+        hooked.sort(key=lambda e: (e[1], -e[2]))
+        return hooked, want_images
+
+    def _data_grad(self, hooked, want_images, images):
+        if images.dim() != 4:
+            raise ValueError(f"images must be [B,3,H,W], got {tuple(images.shape)}")
+        B, _, H, W = images.shape
+        _, blocks = self._served_modules()
+        geometry, c, h, w = [], 64, H // 4, W // 4
+        for blk in blocks:
+            s = blk.conv2.stride[0]
+            co = blk.conv3.out_channels
+            geometry.append((c, h, w, co, h // s, w // s))
+            c, h, w = co, h // s, w // s
+        return _DataGrad(hooked, want_images, geometry, B, H, W, images.device)
 
     def _train_options(self) -> Dict[str, float]:
         mc = self.text_encoder.model_config
@@ -222,11 +367,14 @@ class MultimodalClassifier(B200Module):
             out.append((name, p))
         return out
 
-    def _forward_train(self, images, input_ids, attention_mask, return_embeddings, explain=None):
+    def _forward_train(self, images, input_ids, attention_mask, return_embeddings, explain=None, dgrad=None):
         """Train-mode forward on the B200 path, differentiable through torch.autograd: the reference's
         training loops (src/train.py:247-333, src/train_multimodal.py:508-556) run unchanged.
         explain = a hooked backbone module: the same machinery in EVAL semantics (no dropout, BatchNorm on running
-        statistics) with the module's hooks served - what Grad-CAM needs."""
+        statistics) with the module's hooks served - what Grad-CAM needs.
+        dgrad = (hooked served modules, images.grad wanted): data gradients through the frozen backbone (input
+        saliency, hooks on any stage or bottleneck) - in eval semantics under model.eval(), with dropout in train mode
+        (where the backbone's BatchNorm must be in eval mode)."""
         p_att = {self.fusion.fusion_layer.image_to_text_attention.dropout.p,
                  self.fusion.fusion_layer.text_to_image_attention.dropout.p,
                  self.fusion.fusion_layer.fusion[2].p}
@@ -234,7 +382,21 @@ class MultimodalClassifier(B200Module):
             raise NotImplementedError("the fusion dropouts must share one probability (FusionConfig.dropout)")
         eng = self._engine(allow_training=True)
         opts = self._train_options()
-        if explain is not None:
+        eval_semantics = explain is not None or (dgrad is not None and not self.training)
+        want_images = dgrad is not None and dgrad[1]
+        if dgrad is not None:
+            if self.training and opts["train.bn_train"]:
+                raise NotImplementedError(
+                    "data gradients through the backbone (images.requires_grad, hooks below layer4) in train mode need "
+                    "the backbone's BatchNorm layers in eval mode (running statistics: "
+                    "model.cnn_encoder.backbone.eval()); batch-statistics BatchNorm is not differentiated")
+            if eng.fp32_check:
+                raise NotImplementedError("data gradients through the backbone are not implemented in the fp32 check "
+                                          "mode (configure_b200(fp32_check=True)); switch it off")
+            if self.__dict__.get("_mrd_ddp", (False, None))[0] and self.training:
+                raise NotImplementedError("data gradients through the backbone are not implemented with "
+                                          "data_parallel()")
+        if eval_semantics:
             opts = {k: (v if k == "train.pad_idx" else 0.0) for k, v in opts.items()}
         if eng.train_opts != opts:
             # the cache of what was applied lives on the Engine: a new engine (model.to(other device), deepcopy,
@@ -246,11 +408,11 @@ class MultimodalClassifier(B200Module):
             eng.set_option("load_sync", 0.0)
             eng.train_opts = dict(opts)
         named = self._trainable()
-        if explain is not None and not named:
+        if eval_semantics and not named and not want_images:
             raise RuntimeError("every parameter is frozen: logits.backward() has nothing to differentiate (the "
                                "reference raises here as well unless the input requires grad)")
         # eval semantics draw nothing from the generator (no dropout): leave torch's RNG stream untouched
-        seed = 0 if explain is not None else int(torch.randint(0, 2 ** 62, (1,)).item())   # CPU generator: follows torch.manual_seed
+        seed = 0 if eval_semantics else int(torch.randint(0, 2 ** 62, (1,)).item())   # CPU generator: follows torch.manual_seed
         shapes = tuple((n, tuple(p.shape)) for n, p in named)
         ddp = self.__dict__.get("_mrd_ddp", (False, None))
         if ddp[0]:
@@ -258,12 +420,13 @@ class MultimodalClassifier(B200Module):
             # same dropout masks to their shards (masks are a pure function of seed, site and element index)
             from .parallel import rank_seed
             seed = rank_seed(seed, ddp[1])
-        if explain is not None:
+        if eval_semantics:
             ddp = (False, None)
         emb_dims = ((self.cnn_encoder.embedding_dim, self.text_encoder.embedding_dim, self.fusion_dim)
                     if return_embeddings else None)
+        dg = self._data_grad(dgrad[0], want_images, images) if dgrad is not None else None
         logits = _TrainStep.apply(eng, images, input_ids, attention_mask, seed, shapes,
-                                  (self.num_classes, ddp[0], ddp[1], explain, emb_dims), *[p for _, p in named])
+                                  (self.num_classes, ddp[0], ddp[1], explain, emb_dims, dg), *[p for _, p in named])
         if opts["train.bn_train"]:
             # the library wrote the new running_mean / running_var straight into the BatchNorm buffers
             # (momentum 0.1, unbiased variance: nn.BatchNorm2d in train mode); the step counters and the
