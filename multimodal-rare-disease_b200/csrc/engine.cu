@@ -1027,14 +1027,9 @@ inline int run_f32(mrd_ctx* c, const char* label, const GemmLaunch& g, float* ou
     return launch_gemm(&t, s);
 }
 
-// ------------------------------------------------------------------ stage runners
-// ResNet50 backbone over the whole batch in micro-batches; leaves pooled features in b_pooled.
-int run_backbone(mrd_ctx* c, const void* images, int img_dtype, int B, int H, int W,
-                 float* feat_pooled, float* feat_map, cudaStream_t s) {
-    if (!c->has_cnn) {
-        set_last_error("cnn_encoder weights are not loaded in this context");
-        return -3;
-    }
+// ------------------------------------------------------------------ input checks
+// images of every backbone forward (eval, batch-statistics BatchNorm, saving forward for data gradients)
+int check_images(int img_dtype, int H, int W) {
     if (img_dtype != MRD_DT_F32 && img_dtype != MRD_DT_BF16) {
         set_last_error("images must be f32 or bf16 (dtype code %d)", img_dtype);
         return -1;
@@ -1043,6 +1038,35 @@ int run_backbone(mrd_ctx* c, const void* images, int img_dtype, int B, int H, in
         set_last_error("image size %dx%d unsupported: H and W must be multiples of 32", H, W);
         return -1;
     }
+    return 0;
+}
+
+int fp32_images_only(int img_dtype) {
+    if (img_dtype != MRD_DT_F32) {
+        set_last_error("fp32 check mode takes fp32 images (dtype code %d given)", img_dtype);
+        return -1;
+    }
+    return 0;
+}
+
+// the attention mask is optional; when given, its dtype code must be one the token compaction reads
+int check_mask_dtype(const void* mask, int mask_dtype) {
+    if (mask && (mask_dtype < MRD_DT_I64 || mask_dtype > MRD_DT_BF16)) {
+        set_last_error("unknown mask dtype code %d", mask_dtype);
+        return -1;
+    }
+    return 0;
+}
+
+// ------------------------------------------------------------------ stage runners
+// ResNet50 backbone over the whole batch in micro-batches; leaves pooled features in b_pooled.
+int run_backbone(mrd_ctx* c, const void* images, int img_dtype, int B, int H, int W,
+                 float* feat_pooled, float* feat_map, cudaStream_t s) {
+    if (!c->has_cnn) {
+        set_last_error("cnn_encoder weights are not loaded in this context");
+        return -3;
+    }
+    MRD_TRY(check_images(img_dtype, H, W));
     MRD_TRY(ensure_cnn_ws(c, B, H, W));
     const size_t esz = img_dtype == MRD_DT_BF16 ? 2 : 4;
     static const char* const kStage[5] = {"", "layer1", "layer2", "layer3", "layer4"};
@@ -1315,12 +1339,17 @@ int check_ctx(mrd_ctx* c) {
 #include "engine_train.cuh"
 #include "engine_dgrad.cuh"
 
-int fp32_images_only(int img_dtype) {
-    if (img_dtype != MRD_DT_F32) {
-        set_last_error("fp32 check mode takes fp32 images (dtype code %d given)", img_dtype);
-        return -1;
-    }
-    return 0;
+// mrd_train_forward_ex and mrd_train_forward_dg (save = true: the saving forward for data gradients)
+int train_forward_entry(mrd_ctx* c, const void* images, int img_dtype, const long long* ids, const void* mask,
+                        int mask_dtype, int B, int H, int W, int S, unsigned long long seed, float* logits,
+                        float* feat_map, bool save, float* const* block_out, float* img_emb, float* txt_emb,
+                        float* fused, cudaStream_t s) {
+    MRD_TRY(check_ctx(c));
+    if (B <= 0) return 0;
+    MRD_TRY(check_mask_dtype(mask, mask_dtype));
+    MRD_TRY(train_forward(c, images, img_dtype, ids, mask, mask_dtype, B, H, W, S, seed, logits, feat_map, save,
+                          block_out, s));
+    return train_export_embeddings(c, B, img_emb, txt_emb, fused, s);
 }
 
 }  // namespace
@@ -1466,10 +1495,7 @@ int mrd_text_encoder_fwd_ex(mrd_ctx* c, const long long* ids, const void* mask, 
                             float* cls, float* last_hidden, float* all_hidden, float* attn_probs, void* stream) {
     MRD_TRY(check_ctx(c));
     if (B <= 0) return 0;
-    if (mask && (mask_dtype < MRD_DT_I64 || mask_dtype > MRD_DT_BF16)) {
-        set_last_error("unknown mask dtype code %d", mask_dtype);
-        return -1;
-    }
+    MRD_TRY(check_mask_dtype(mask, mask_dtype));
     if (c->fp32_check) {
         ++c->launches;
         return fp32_text_encoder(c->raw, c->f32_opts(), &c->f32_ws, ids, mask, mask_dtype, B, S, cls,
@@ -1601,10 +1627,7 @@ int mrd_multimodal_fwd(mrd_ctx* c, const void* images, int img_dtype, const long
                        c->head_in);
         return -1;
     }
-    if (mask && (mask_dtype < MRD_DT_I64 || mask_dtype > MRD_DT_BF16)) {
-        set_last_error("unknown mask dtype code %d", mask_dtype);
-        return -1;
-    }
+    MRD_TRY(check_mask_dtype(mask, mask_dtype));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     MRD_TRY(ensure_batch_ws(c, B));
     if (c->fp32_check) {
@@ -1683,15 +1706,8 @@ int mrd_ctx_profile_report(mrd_ctx* c, char* buf, int cap) {
 int mrd_train_forward_ex(mrd_ctx* c, const void* images, int img_dtype, const long long* ids, const void* mask,
                          int mask_dtype, int B, int H, int W, int S, unsigned long long seed, float* logits,
                          float* feat_map, float* img_emb, float* txt_emb, float* fused, void* stream) {
-    MRD_TRY(check_ctx(c));
-    if (B <= 0) return 0;
-    if (mask && (mask_dtype < MRD_DT_I64 || mask_dtype > MRD_DT_BF16)) {
-        set_last_error("unknown mask dtype code %d", mask_dtype);
-        return -1;
-    }
-    MRD_TRY(train_forward(c, images, img_dtype, ids, mask, mask_dtype, B, H, W, S, seed, logits, feat_map,
-                          static_cast<cudaStream_t>(stream)));
-    return train_export_embeddings(c, B, img_emb, txt_emb, fused, static_cast<cudaStream_t>(stream));
+    return train_forward_entry(c, images, img_dtype, ids, mask, mask_dtype, B, H, W, S, seed, logits, feat_map, false,
+                               nullptr, img_emb, txt_emb, fused, static_cast<cudaStream_t>(stream));
 }
 
 int mrd_train_forward(mrd_ctx* c, const void* images, int img_dtype, const long long* ids, const void* mask,
@@ -1704,21 +1720,13 @@ int mrd_train_forward(mrd_ctx* c, const void* images, int img_dtype, const long 
 int mrd_train_backward_ex(mrd_ctx* c, const float* dlogits, int n, const char* const* names, float* const* grads,
                           float* d_pooled, void* stream) {
     MRD_TRY(check_ctx(c));
-    GradTable gt;
-    gt.reserve(static_cast<size_t>(n) * 2);
-    for (int i = 0; i < n; ++i)
-        if (grads[i]) gt.emplace(names[i], grads[i]);
-    return train_backward(c, dlogits, gt, d_pooled, static_cast<cudaStream_t>(stream));
+    return train_backward(c, dlogits, grad_table(n, names, grads), d_pooled, static_cast<cudaStream_t>(stream));
 }
 
 int mrd_train_backward_begin(mrd_ctx* c, const float* dlogits, int n, const char* const* names,
                              float* const* grads, float* d_pooled) {
     MRD_TRY(check_ctx(c));
-    GradTable gt;
-    gt.reserve(static_cast<size_t>(n) * 2);
-    for (int i = 0; i < n; ++i)
-        if (grads[i]) gt.emplace(names[i], grads[i]);
-    return train_backward_begin(c, dlogits, gt, d_pooled);
+    return train_backward_begin(c, dlogits, grad_table(n, names, grads), d_pooled);
 }
 
 int mrd_train_backward_stages(mrd_ctx* c, int first, int last, void* stream) {
@@ -1739,16 +1747,8 @@ int mrd_train_backward(mrd_ctx* c, const float* dlogits, int n, const char* cons
 int mrd_train_forward_dg(mrd_ctx* c, const void* images, int img_dtype, const long long* ids, const void* mask,
                          int mask_dtype, int B, int H, int W, int S, unsigned long long seed, float* logits,
                          float* const* block_out, float* img_emb, float* txt_emb, float* fused, void* stream) {
-    MRD_TRY(check_ctx(c));
-    if (B <= 0) return 0;
-    TrainState* t = train_state(c);
-    t->dg_save = true;
-    t->dg_block_out = block_out;
-    const int rc = mrd_train_forward_ex(c, images, img_dtype, ids, mask, mask_dtype, B, H, W, S, seed, logits, nullptr,
-                                        img_emb, txt_emb, fused, stream);
-    t->dg_save = false;
-    t->dg_block_out = nullptr;
-    return rc;
+    return train_forward_entry(c, images, img_dtype, ids, mask, mask_dtype, B, H, W, S, seed, logits, nullptr, true,
+                               block_out, img_emb, txt_emb, fused, static_cast<cudaStream_t>(stream));
 }
 
 int mrd_train_backward_dg(mrd_ctx* c, const float* dlogits, int n, const char* const* names, float* const* grads,

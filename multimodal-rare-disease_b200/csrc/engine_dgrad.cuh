@@ -233,14 +233,7 @@ int dgrad_plan(mrd_ctx* c, int B, int H, int W) {
 // backward needs kept, and block_out[k] (optional, f32 NCHW) = the output of bottleneck k.
 int run_backbone_save(mrd_ctx* c, const void* images, int img_dtype, int B, int H, int W, float* pooled_f32,
                       float* const* block_out, cudaStream_t s) {
-    if (img_dtype != MRD_DT_F32 && img_dtype != MRD_DT_BF16) {
-        set_last_error("images must be f32 or bf16 (dtype code %d)", img_dtype);
-        return -1;
-    }
-    if (H % 32 != 0 || W % 32 != 0 || H <= 0 || W <= 0) {
-        set_last_error("image size %dx%d unsupported: H and W must be multiples of 32", H, W);
-        return -1;
-    }
+    MRD_TRY(check_images(img_dtype, H, W));
     if (B > kDgradMaxBatch) {
         set_last_error("data gradients: batch %d exceeds %d images per forward (27 MB of saved activations and "
                        "gradient scratch per 224 x 224 image)", B, kDgradMaxBatch);
@@ -272,15 +265,11 @@ int run_backbone_save(mrd_ctx* c, const void* images, int img_dtype, int B, int 
 // Backward of the saving forward from d_pooled (f32 [B, feat_dim]).  Blocks 15 .. first_block run (first_block = 16:
 // none); block_grads[k] (optional, f32 NCHW) receives d/d(output of block k) for first_block - 1 <= k < 15 (slot 15 is
 // d_pooled / (h*w) at every position and is not written); d_block_in (optional) = d/d(input of block first_block);
-// d_images (optional, first_block == 0) = d/d(images) f32 [B,3,H,W].
+// d_images (optional, first_block == 0) = d/d(images) f32 [B,3,H,W].  The caller has checked that the pending forward
+// was a saving forward (DgradCnn::valid).
 int dgrad_backbone(mrd_ctx* c, const float* d_pooled, float* const* block_grads, int first_block, float* d_block_in,
                    float* d_images, cudaStream_t s) {
-    DgradCnn* d = c->train ? c->train->dg : nullptr;
-    if (!d || !d->valid) {
-        set_last_error("data gradients: the pending training forward did not save the backbone's activations "
-                       "(mrd_train_forward_dg)");
-        return -1;
-    }
+    DgradCnn* d = c->train->dg;
     d->valid = false;
     const int nb = static_cast<int>(d->blk.size());
     if (first_block < 0 || first_block > nb || (d_images && first_block != 0) || (d_block_in && first_block == nb)) {

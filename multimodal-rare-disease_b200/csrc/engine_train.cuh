@@ -51,8 +51,6 @@ struct TrainState {
     TrainOpts o;
     TrainCnn* cnn = nullptr;              // batch-statistics backbone (created when bn_train is first used)
     DgradCnn* dg = nullptr;               // data gradients through the backbone (engine_dgrad.cuh), created on first use
-    float* const* dg_block_out = nullptr; // set by mrd_train_forward_dg for one forward: save for data gradients,
-    bool dg_save = false;                 // and the optional per-block output maps
     std::vector<TrainLayerWt> wt;
     bool packs_valid = false;
     // plan / workspace for one (B, S)
@@ -84,7 +82,6 @@ struct TrainState {
     bool fwd_done = false;
     unsigned long long seed = 0;
     const long long* ids = nullptr;
-    int mask_dtype = 0;
 };
 
 enum : unsigned { SITE_EMB = 1000, SITE_TEXT_OUT = 1001, SITE_CNN_PROJ = 1002, SITE_I2T = 1003,
@@ -404,14 +401,7 @@ int train_cnn_plan(mrd_ctx* c, int B, int H, int W) {
 
 int run_backbone_train(mrd_ctx* c, const void* images, int img_dtype, int B, int H, int W, float* pooled_f32,
                        cudaStream_t s) {
-    if (img_dtype != MRD_DT_F32 && img_dtype != MRD_DT_BF16) {
-        set_last_error("images must be f32 or bf16 (dtype code %d)", img_dtype);
-        return -1;
-    }
-    if (H % 32 != 0 || W % 32 != 0 || H <= 0 || W <= 0) {
-        set_last_error("image size %dx%d unsupported: H and W must be multiples of 32", H, W);
-        return -1;
-    }
+    MRD_TRY(check_images(img_dtype, H, W));
     TrainState* t = train_state(c);
     MRD_TRY(ensure_cnn_ws(c, B, H, W));
     MRD_TRY(train_cnn_pack(c, s));
@@ -508,6 +498,14 @@ void train_cnn_free(TrainState* t) {
 }
 
 typedef std::unordered_map<std::string, float*> GradTable;
+// the parameters of the C ABI's (names, grads) arrays that have a gradient slot
+GradTable grad_table(int n, const char* const* names, float* const* grads) {
+    GradTable gt;
+    gt.reserve(static_cast<size_t>(n) * 2);
+    for (int i = 0; i < n; ++i)
+        if (grads[i]) gt.emplace(names[i], grads[i]);
+    return gt;
+}
 inline float* grad_of(const GradTable& g, const std::string& k) {
     auto it = g.find(k);
     return it == g.end() ? nullptr : it->second;
@@ -560,20 +558,9 @@ int lin_bwd(mrd_ctx* c, const GradTable& gt, const std::string& name, const floa
     return 0;
 }
 
-int fp32_images_only_train(int img_dtype) {
-    if (img_dtype != MRD_DT_F32) {
-        set_last_error("fp32 check mode takes fp32 images (dtype code %d given)", img_dtype);
-        return -1;
-    }
-    return 0;
-}
-
 // ---- forward -------------------------------------------------------------------------------------
-int train_forward(mrd_ctx* c, const void* images, int img_dtype, const long long* ids, const void* mask,
-                  int mask_dtype, int B, int H, int W, int S, unsigned long long seed, float* logits,
-                  float* feat_map, cudaStream_t s) {
-    TrainState* t = train_state(c);
-    const TrainOpts& o = t->o;
+// Refusals that depend on the loaded weights and the shapes: checked before any workspace is resized.
+int train_check_shapes(mrd_ctx* c, int B, int S) {
     if (!(c->has_cnn && c->has_text && c->has_fusion && c->has_head)) {
         set_last_error("training step needs cnn_encoder, text_encoder, fusion and classifier weights");
         return -3;
@@ -591,25 +578,18 @@ int train_forward(mrd_ctx* c, const void* images, int img_dtype, const long long
         set_last_error("training step: classifier activation must be relu");
         return -1;
     }
-    const int Hd = c->hidden, F = c->ffn, Fd = c->fusion_dim;
-    MRD_TRY(ensure_batch_ws(c, B));
-    MRD_TRY(ensure_text_ws(c, B * S, B));
-    MRD_TRY(train_ensure_packs(c, s));
-    MRD_TRY(train_ensure_plan(c, B, S));
-    t->fwd_done = false;
-    t->seed = seed;
-    t->ids = ids;
-    dgrad_forget(t);   // a saving forward re-validates its activations
-    const int T = B * S;
+    return 0;
+}
 
-    if (t->dg_save && (c->fp32_check || o.bn_train || feat_map)) {
+// Refusals that depend on the mode: fp32 check, batch-statistics BatchNorm, the layer4 map, a saving forward.
+int train_check_mode(mrd_ctx* c, int img_dtype, const float* feat_map, bool save) {
+    const TrainOpts& o = c->train->o;
+    if (save && (c->fp32_check || o.bn_train || feat_map)) {
         set_last_error("data gradients: need the bf16 path (no fp32 check) and the backbone's BatchNorm on running "
                        "statistics (train.bn_train = 0); the layer4 map is block output 15");
         return -1;
     }
     if (c->fp32_check) {
-        // fp32 check of the training step: backbone and text encoder in plain fp32 (fp32_check.cu), dropout off;
-        // the batch-level layers below are fp32 in either mode
         if (o.p_bert_hidden != 0.0 || o.p_bert_attn != 0.0 || o.p_text_out != 0.0 || o.p_cnn_proj != 0.0 ||
             o.p_fusion != 0.0 || o.p_head != 0.0) {
             set_last_error("fp32 check (train): every dropout probability must be 0 (the check compares with the "
@@ -620,64 +600,88 @@ int train_forward(mrd_ctx* c, const void* images, int img_dtype, const long long
             set_last_error("fp32 check (train): the frozen backbone must be in eval mode (running statistics)");
             return -1;
         }
-        MRD_TRY(fp32_images_only_train(img_dtype));
-        const Fp32Opts fo = c->f32_opts();
-        c->launches += 2;
-        MRD_TRY(fp32_cnn_encoder(c->raw, fo, &c->f32_ws, static_cast<const float*>(images), B, H, W, t->g4, t->pooled,
-                                 feat_map, s));
-        MRD_TRY(fp32_bert_train_forward(c->raw, fo, &c->f32_train, ids, mask, mask_dtype, B, S, t->cls, s));
-    } else {
-    // ---- image branch: frozen backbone (forward only), then the trainable projection in fp32
-    if (o.bn_train) {
-        if (feat_map) {
-            set_last_error("training step: the layer4 feature map is exported with the backbone in eval mode only");
-            return -1;
-        }
+        return fp32_images_only(img_dtype);
+    }
+    if (o.bn_train && feat_map) {
+        set_last_error("training step: the layer4 feature map is exported with the backbone in eval mode only");
+        return -1;
+    }
+    return 0;
+}
+
+// Image branch: the frozen backbone (forward only; fp32 check, batch-statistics BatchNorm, saving forward for data
+// gradients, or the eval forward) into t->pooled, then the trainable projection in fp32 into t->img.
+int train_forward_image(mrd_ctx* c, const void* images, int img_dtype, int B, int H, int W, float* feat_map, bool save,
+                        float* const* block_out, cudaStream_t s) {
+    TrainState* t = c->train;
+    const TrainOpts& o = t->o;
+    if (c->fp32_check) {
+        ++c->launches;
+        MRD_TRY(fp32_cnn_encoder(c->raw, c->f32_opts(), &c->f32_ws, static_cast<const float*>(images), B, H, W, t->g4,
+                                 t->pooled, feat_map, s));
+    } else if (o.bn_train) {
         MRD_TRY(run_backbone_train(c, images, img_dtype, B, H, W, t->pooled, s));
-    } else if (t->dg_save) {
-        MRD_TRY(run_backbone_save(c, images, img_dtype, B, H, W, t->pooled, t->dg_block_out, s));
+    } else if (save) {
+        MRD_TRY(run_backbone_save(c, images, img_dtype, B, H, W, t->pooled, block_out, s));
     } else {
         MRD_TRY(run_backbone(c, images, img_dtype, B, H, W, t->pooled, feat_map, s));
     }
-    }
     MRD_TRY(lin_fwd(c, "cnn_encoder.projection.0", t->pooled, c->feat_dim, B, t->a1, c->proj1.out, MRD_ACT_NONE,
                     nullptr, 0, s));
-    TRK("train.dropout", CAT_MEM, relu_dropout_f32(t->a1, B, c->proj1.out, make_drop(seed, SITE_CNN_PROJ, o.p_cnn_proj), t->p1, s));
+    TRK("train.dropout", CAT_MEM, relu_dropout_f32(t->a1, B, c->proj1.out, make_drop(t->seed, SITE_CNN_PROJ, o.p_cnn_proj), t->p1, s));
     MRD_TRY(lin_fwd(c, "cnn_encoder.projection.3", t->p1, c->proj1.out, B, t->img, c->proj2.out, MRD_ACT_NONE,
                     nullptr, 0, s));
+    return 0;
+}
 
-    // ---- text branch
-    if (!c->fp32_check) {
-    TRK("train.compact_tokens", CAT_MEM, compact_tokens(mask, mask_dtype, B, S, 0, c->t_seq_off, c->t_row_tok, c->t_bias, c->t_nrows,
-                           c->t_scratch, s));
-    TRK("train.embed_ln", CAT_MEM, bert_embed_layernorm(ids, B, S, c->word_emb, c->pos_type, c->emb_g, c->emb_b, c->bert_ln_eps, c->vocab,
-                                 t->L[0].x, s, c->t_row_tok, c->t_nrows));
-    TRK("train.dropout", CAT_MEM, dropout_bf16(t->L[0].x, Hd, T, Hd, c->t_nrows, make_drop(seed, SITE_EMB, o.p_bert_hidden), t->L[0].x,
-                         Hd, s));
-    const size_t nl = c->layers.size();
-    for (size_t i = 0; i < nl; ++i) {
-        const BertLayerW& Lw = c->layers[i];
-        const TrainLayerBuf& b = t->L[i];
-        TrainLayerPlan& p = t->P[i];
-        bf16* x_next = i + 1 < nl ? t->L[i + 1].x : t->x_final;
-        MRD_TRY(run(c, "train.qkv", p.qkv, s));
-        const DropCfg da = make_drop(seed, site_attn(i), o.p_bert_attn);
-        TRK("train.attention", CAT_ATTN, attention_forward(b.qkv, c->t_bias, c->t_seq_off, B, S, c->bert_heads, b.ctx, s, T, 0, &da));
-        MRD_TRY(run(c, "train.attn_out", p.o, s));
-        TRK("train.drop_add_ln", CAT_MEM, drop_add_ln_fwd(t->z, b.x, T, Hd, c->t_nrows, make_drop(seed, site_attn_out(i), o.p_bert_hidden),
-                                Lw.ln1g, Lw.ln1b, c->bert_ln_eps, b.s1, b.h1, s));
-        MRD_TRY(run(c, "train.ffn1", p.f1, s));
-        TRK("train.gelu", CAT_MEM, gelu_fwd_bf16(b.u, T, F, c->t_nrows, b.g, s));
-        MRD_TRY(run(c, "train.ffn2", p.f2, s));
-        TRK("train.drop_add_ln", CAT_MEM, drop_add_ln_fwd(t->z, b.h1, T, Hd, c->t_nrows, make_drop(seed, site_ffn_out(i), o.p_bert_hidden),
-                                Lw.ln2g, Lw.ln2b, c->bert_ln_eps, b.s2, x_next, s));
-    }
-    // CLS row (src/text_encoder.py:118) + TextEncoder.dropout
-    TRK("train.cls", CAT_MEM, gather_cls_rows_f32(t->x_final, c->t_seq_off, B, Hd, t->cls, s));
+// Text branch: BERT with every activation the backward needs kept (plain fp32 in the fp32 check), its CLS row
+// (src/text_encoder.py:118) into t->cls, then TextEncoder.dropout into t->txt.
+int train_forward_text(mrd_ctx* c, const long long* ids, const void* mask, int mask_dtype, int B, int S,
+                       cudaStream_t s) {
+    TrainState* t = c->train;
+    const TrainOpts& o = t->o;
+    const unsigned long long seed = t->seed;
+    const int Hd = c->hidden, F = c->ffn, T = B * S;
+    if (c->fp32_check) {
+        ++c->launches;
+        MRD_TRY(fp32_bert_train_forward(c->raw, c->f32_opts(), &c->f32_train, ids, mask, mask_dtype, B, S, t->cls, s));
+    } else {
+        TRK("train.compact_tokens", CAT_MEM, compact_tokens(mask, mask_dtype, B, S, 0, c->t_seq_off, c->t_row_tok, c->t_bias, c->t_nrows,
+                               c->t_scratch, s));
+        TRK("train.embed_ln", CAT_MEM, bert_embed_layernorm(ids, B, S, c->word_emb, c->pos_type, c->emb_g, c->emb_b, c->bert_ln_eps, c->vocab,
+                                     t->L[0].x, s, c->t_row_tok, c->t_nrows));
+        TRK("train.dropout", CAT_MEM, dropout_bf16(t->L[0].x, Hd, T, Hd, c->t_nrows, make_drop(seed, SITE_EMB, o.p_bert_hidden), t->L[0].x,
+                             Hd, s));
+        const size_t nl = c->layers.size();
+        for (size_t i = 0; i < nl; ++i) {
+            const BertLayerW& Lw = c->layers[i];
+            const TrainLayerBuf& b = t->L[i];
+            TrainLayerPlan& p = t->P[i];
+            bf16* x_next = i + 1 < nl ? t->L[i + 1].x : t->x_final;
+            MRD_TRY(run(c, "train.qkv", p.qkv, s));
+            const DropCfg da = make_drop(seed, site_attn(i), o.p_bert_attn);
+            TRK("train.attention", CAT_ATTN, attention_forward(b.qkv, c->t_bias, c->t_seq_off, B, S, c->bert_heads, b.ctx, s, T, 0, &da));
+            MRD_TRY(run(c, "train.attn_out", p.o, s));
+            TRK("train.drop_add_ln", CAT_MEM, drop_add_ln_fwd(t->z, b.x, T, Hd, c->t_nrows, make_drop(seed, site_attn_out(i), o.p_bert_hidden),
+                                    Lw.ln1g, Lw.ln1b, c->bert_ln_eps, b.s1, b.h1, s));
+            MRD_TRY(run(c, "train.ffn1", p.f1, s));
+            TRK("train.gelu", CAT_MEM, gelu_fwd_bf16(b.u, T, F, c->t_nrows, b.g, s));
+            MRD_TRY(run(c, "train.ffn2", p.f2, s));
+            TRK("train.drop_add_ln", CAT_MEM, drop_add_ln_fwd(t->z, b.h1, T, Hd, c->t_nrows, make_drop(seed, site_ffn_out(i), o.p_bert_hidden),
+                                    Lw.ln2g, Lw.ln2b, c->bert_ln_eps, b.s2, x_next, s));
+        }
+        TRK("train.cls", CAT_MEM, gather_cls_rows_f32(t->x_final, c->t_seq_off, B, Hd, t->cls, s));
     }
     TRK("train.dropout", CAT_MEM, dropout_f32(t->cls, B, Hd, make_drop(seed, SITE_TEXT_OUT, o.p_text_out), t->txt, s));
+    return 0;
+}
 
-    // ---- fusion (src/fusion_model.py:245-291 in train mode)
+// Fusion (src/fusion_model.py:245-291 in train mode) and head (src/multimodal_classifier.py:73-83) on t->img, t->txt.
+int train_forward_tail(mrd_ctx* c, int B, float* logits, cudaStream_t s) {
+    TrainState* t = c->train;
+    const TrainOpts& o = t->o;
+    const unsigned long long seed = t->seed;
+    const int Fd = c->fusion_dim;
     const std::string f = "fusion.fusion_layer.";
     const int hd = Fd / c->fusion_heads;
     MRD_TRY(lin_fwd(c, f + "image_proj", t->img, c->fusion_img_in, B, t->ip, Fd, MRD_ACT_NONE, nullptr, 0, s));
@@ -696,7 +700,6 @@ int train_forward(mrd_ctx* c, const void* images, int img_dtype, const long long
     TRK("train.dropout", CAT_MEM, relu_dropout_f32(t->g0, B, Fd, make_drop(seed, SITE_FUSION_MLP, o.p_fusion), t->fh, s));
     MRD_TRY(lin_fwd(c, f + "fusion.3", t->fh, Fd, B, t->fused, Fd, MRD_ACT_NONE, nullptr, 0, s));
 
-    // ---- head (src/multimodal_classifier.py:73-83)
     const float* x = t->fused;
     int ld = c->head_in;
     for (size_t j = 0; j < c->head_hidden.size(); ++j) {
@@ -708,11 +711,31 @@ int train_forward(mrd_ctx* c, const void* images, int img_dtype, const long long
         x = t->hh[j];
         ld = n;
     }
-    {
-        char nm[64];
-        snprintf(nm, sizeof(nm), "classifier.classifier.%zu", 3 * c->head_hidden.size());
-        MRD_TRY(lin_fwd(c, nm, x, ld, B, logits, c->num_classes, MRD_ACT_NONE, nullptr, 0, s));
-    }
+    char nm[64];
+    snprintf(nm, sizeof(nm), "classifier.classifier.%zu", 3 * c->head_hidden.size());
+    return lin_fwd(c, nm, x, ld, B, logits, c->num_classes, MRD_ACT_NONE, nullptr, 0, s);
+}
+
+// The training forward.  save: keep what the backbone's data-gradient backward needs (dgrad_backbone), and write the
+// output of bottleneck k into block_out[k] where that slot is given.  In the fp32 check the backbone and BERT run in
+// plain fp32 (fp32_check.cu) with dropout off; the batch-level layers are fp32 in either mode.
+int train_forward(mrd_ctx* c, const void* images, int img_dtype, const long long* ids, const void* mask,
+                  int mask_dtype, int B, int H, int W, int S, unsigned long long seed, float* logits,
+                  float* feat_map, bool save, float* const* block_out, cudaStream_t s) {
+    TrainState* t = train_state(c);
+    MRD_TRY(train_check_shapes(c, B, S));
+    MRD_TRY(ensure_batch_ws(c, B));
+    MRD_TRY(ensure_text_ws(c, B * S, B));
+    MRD_TRY(train_ensure_packs(c, s));
+    MRD_TRY(train_ensure_plan(c, B, S));
+    t->fwd_done = false;
+    t->seed = seed;
+    t->ids = ids;
+    dgrad_forget(t);   // a saving forward re-validates its activations
+    MRD_TRY(train_check_mode(c, img_dtype, feat_map, save));
+    MRD_TRY(train_forward_image(c, images, img_dtype, B, H, W, feat_map, save, block_out, s));
+    MRD_TRY(train_forward_text(c, ids, mask, mask_dtype, B, S, s));
+    MRD_TRY(train_forward_tail(c, B, logits, s));
     t->fwd_done = true;
     t->text_run_epoch = c->text_run_epoch;
     return 0;
@@ -775,42 +798,19 @@ int train_backward_begin(mrd_ctx* c, const float* dlogits, const GradTable& gt, 
     return 0;
 }
 
-// runs stages [lo, hi) of the pending backward; stages must be run in order, each exactly once
-int train_backward_run(mrd_ctx* c, int lo, int hi, cudaStream_t s) {
-    TrainState* t = train_state(c);
-    const int n_stages = train_backward_stages(c);
-    if (!t->bw_active || lo != t->bw_next || hi <= lo || hi > n_stages) {
-        set_last_error("mrd_train_backward_stage: stages [%d, %d) out of order (next %d of %d, %s)", lo, hi,
-                       t->bw_next, n_stages, t->bw_active ? "active" : "no backward begun");
-        return -1;
-    }
-    t->bw_next = hi;
-    if (hi == n_stages) t->bw_active = false;
-    auto runs = [&](int st) { return lo <= st && st < hi; };
+// ---- stage 0: head, fusion, image projection, TextEncoder.dropout, CLS scatter
+// Head (src/multimodal_classifier.py:73-83): dlogits -> *d_fused [B, head_in], one of the ping-pong buffers g1 / g2.
+int bw_head(mrd_ctx* c, TrainState* t, float** d_fused, cudaStream_t s) {
     const GradTable& gt = t->bw_grads;
-    const float* dlogits = t->bw_dlogits;
-    float* d_pooled = t->bw_d_pooled;
     const TrainOpts& o = t->o;
-    const unsigned long long seed = t->seed;
-    const int B = t->B, S = t->S, T = t->Ta, Hd = c->hidden, F = c->ffn, Fd = c->fusion_dim;
-    const int hd = Fd / c->fusion_heads;
-    const long long nB = B;
-
-    const size_t nl = c->layers.size();
-    bf16* dx_top = (nl & 1) ? t->dxb : t->dxa;   // layer nl-1 reads dx[nl & 1]
-    if (runs(0)) {
-    // ---- head
+    const int B = t->B;
     const size_t nh = c->head_hidden.size();
-    const float* dy = dlogits;
-    int ldy = c->num_classes;
     {
         char nm[64];
         snprintf(nm, sizeof(nm), "classifier.classifier.%zu", 3 * nh);
         const float* x = nh ? t->hh[nh - 1] : t->fused;
         const int ldx = nh ? c->head_hidden[nh - 1].out : c->head_in;
-        MRD_TRY(lin_bwd(c, gt, nm, x, ldx, dy, ldy, B, t->g1, ldx, nullptr, 0, s));
-        dy = t->g1;
-        ldy = ldx;
+        MRD_TRY(lin_bwd(c, gt, nm, x, ldx, t->bw_dlogits, c->num_classes, B, t->g1, ldx, nullptr, 0, s));
     }
     float* ping[2] = {t->g1, t->g2};
     int cur = 0;
@@ -818,23 +818,29 @@ int train_backward_run(mrd_ctx* c, int lo, int hi, cudaStream_t s) {
         char nm[64];
         snprintf(nm, sizeof(nm), "classifier.classifier.%zu", 3 * jj);
         const int n = c->head_hidden[jj].out;
-        // dy is the gradient of the post-dropout activation hh[jj]
-        TRK("train.dropout", CAT_MEM, dropout_f32(dy, B, n, make_drop(seed, SITE_HEAD + static_cast<unsigned>(jj), o.p_head), t->g0, s));
-        TRK("train.relu_bwd", CAT_MEM, relu_bwd_f32(t->hh[jj], t->g0, nB * n, t->g0, s));
+        // ping[cur] is the gradient of the post-dropout activation hh[jj]
+        TRK("train.dropout", CAT_MEM, dropout_f32(ping[cur], B, n, make_drop(t->seed, SITE_HEAD + static_cast<unsigned>(jj), o.p_head), t->g0, s));
+        TRK("train.relu_bwd", CAT_MEM, relu_bwd_f32(t->hh[jj], t->g0, 1LL * B * n, t->g0, s));
         const float* x = jj ? t->hh[jj - 1] : t->fused;
         const int ldx = jj ? c->head_hidden[jj - 1].out : c->head_in;
-        float* dx = ping[cur ^ 1];
-        MRD_TRY(lin_bwd(c, gt, nm, x, ldx, t->g0, n, B, dx, ldx, nullptr, 0, s));
-        dy = dx;
-        ldy = ldx;
+        MRD_TRY(lin_bwd(c, gt, nm, x, ldx, t->g0, n, B, ping[cur ^ 1], ldx, nullptr, 0, s));
         cur ^= 1;
     }
-    // dy = d(fused) [B, Fd]
+    *d_fused = ping[cur];
+    return 0;
+}
+
+// Fusion (src/fusion_model.py:245-291): d(fused) -> d(image embedding) in g1, d(text embedding) in g2.
+int bw_fusion(mrd_ctx* c, TrainState* t, const float* d_fused, cudaStream_t s) {
+    const GradTable& gt = t->bw_grads;
+    const TrainOpts& o = t->o;
+    const unsigned long long seed = t->seed;
+    const int B = t->B, Fd = c->fusion_dim, hd = Fd / c->fusion_heads;
     const std::string f = "fusion.fusion_layer.";
-    float* d_fh = ping[cur ^ 1];
-    MRD_TRY(lin_bwd(c, gt, f + "fusion.3", t->fh, Fd, dy, ldy, B, d_fh, Fd, nullptr, 0, s));
+    float* d_fh = d_fused == t->g1 ? t->g2 : t->g1;   // the head's other ping-pong buffer
+    MRD_TRY(lin_bwd(c, gt, f + "fusion.3", t->fh, Fd, d_fused, c->head_in, B, d_fh, Fd, nullptr, 0, s));
     TRK("train.dropout", CAT_MEM, dropout_f32(d_fh, B, Fd, make_drop(seed, SITE_FUSION_MLP, o.p_fusion), t->g0, s));
-    TRK("train.relu_bwd", CAT_MEM, relu_bwd_f32(t->fh, t->g0, nB * Fd, t->g0, s));
+    TRK("train.relu_bwd", CAT_MEM, relu_bwd_f32(t->fh, t->g0, 1LL * B * Fd, t->g0, s));
     float* d_cat = t->g3;  // [B, 2*Fd]
     MRD_TRY(lin_bwd(c, gt, f + "fusion.0", t->cat, 2 * Fd, t->g0, Fd, B, d_cat, 2 * Fd, nullptr, 0, s));
     float* d_pre_i = t->g1;
@@ -855,108 +861,142 @@ int train_backward_run(mrd_ctx* c, int lo, int hi, cudaStream_t s) {
     TRK("train.dropout", CAT_MEM, head_dropout_f32(d_v, B, c->fusion_heads, hd, make_drop(seed, SITE_T2I, o.p_fusion), d_v, nullptr, s));
     MRD_TRY(lin_bwd(c, gt, f + "text_to_image_attention.value_proj", t->ip, Fd, d_v, Fd, B, d_ip, Fd,
                     c->fusion_residual ? d_pre_i : nullptr, Fd, s));
-    float* d_img = t->g1;    // d_pre_i / d_pre_t are dead now
-    float* d_txt = t->g2;
-    MRD_TRY(lin_bwd(c, gt, f + "image_proj", t->img, c->fusion_img_in, d_ip, Fd, B, d_img, c->fusion_img_in, nullptr, 0, s));
-    MRD_TRY(lin_bwd(c, gt, f + "text_proj", t->txt, c->fusion_txt_in, d_tp, Fd, B, d_txt, c->fusion_txt_in, nullptr, 0, s));
+    // d_pre_i / d_pre_t are dead now
+    MRD_TRY(lin_bwd(c, gt, f + "image_proj", t->img, c->fusion_img_in, d_ip, Fd, B, t->g1, c->fusion_img_in, nullptr, 0, s));
+    MRD_TRY(lin_bwd(c, gt, f + "text_proj", t->txt, c->fusion_txt_in, d_tp, Fd, B, t->g2, c->fusion_txt_in, nullptr, 0, s));
+    return 0;
+}
 
-    // ---- image projection (the backbone below it is frozen)
+// Image projection (the backbone below it is frozen): d(image embedding) -> optional d_pooled, the gradient of the
+// backbone's pooled output - what Grad-CAM spreads over the layer4 map.
+int bw_image_projection(mrd_ctx* c, TrainState* t, const float* d_img, cudaStream_t s) {
+    const GradTable& gt = t->bw_grads;
+    const int B = t->B;
     MRD_TRY(lin_bwd(c, gt, "cnn_encoder.projection.3", t->p1, c->proj1.out, d_img, c->proj2.out, B, t->g0,
                     c->proj1.out, nullptr, 0, s));
-    TRK("train.dropout", CAT_MEM, dropout_f32(t->g0, B, c->proj1.out, make_drop(seed, SITE_CNN_PROJ, o.p_cnn_proj), t->g0, s));
-    TRK("train.relu_bwd", CAT_MEM, relu_bwd_f32(t->p1, t->g0, nB * c->proj1.out, t->g0, s));
-    // d_pooled (optional): gradient of the backbone's pooled output - what Grad-CAM spreads over the layer4 map
-    MRD_TRY(lin_bwd(c, gt, "cnn_encoder.projection.0", t->pooled, c->feat_dim, t->g0, c->proj1.out, B, d_pooled,
-                    c->feat_dim, nullptr, 0, s));
+    TRK("train.dropout", CAT_MEM, dropout_f32(t->g0, B, c->proj1.out, make_drop(t->seed, SITE_CNN_PROJ, t->o.p_cnn_proj), t->g0, s));
+    TRK("train.relu_bwd", CAT_MEM, relu_bwd_f32(t->p1, t->g0, 1LL * B * c->proj1.out, t->g0, s));
+    return lin_bwd(c, gt, "cnn_encoder.projection.0", t->pooled, c->feat_dim, t->g0, c->proj1.out, B, t->bw_d_pooled,
+                   c->feat_dim, nullptr, 0, s);
+}
+
+int bw_batch_layers(mrd_ctx* c, TrainState* t, cudaStream_t s) {
+    float* d_fused = nullptr;
+    MRD_TRY(bw_head(c, t, &d_fused, s));
+    MRD_TRY(bw_fusion(c, t, d_fused, s));
+    MRD_TRY(bw_image_projection(c, t, t->g1, s));
     if (!t->bw_want_text) return 0;   // nothing below the text embedding is differentiated (frozen text encoder)
 
-    // ---- text branch: TextEncoder.dropout, CLS scatter, then the encoder layers in reverse
-    TRK("train.dropout", CAT_MEM, dropout_f32(d_txt, B, Hd, make_drop(seed, SITE_TEXT_OUT, o.p_text_out), d_txt, s));
+    // ---- TextEncoder.dropout, then the CLS scatter into the input gradient of the top BERT layer
+    const int B = t->B, Hd = c->hidden;
+    float* d_txt = t->g2;
+    TRK("train.dropout", CAT_MEM, dropout_f32(d_txt, B, Hd, make_drop(t->seed, SITE_TEXT_OUT, t->o.p_text_out), d_txt, s));
     if (c->fp32_check) {
         ++c->launches;
-        return fp32_bert_train_backward(c->raw, c->f32_opts(), &c->f32_train, d_txt, gt, o.pad_idx, s);
+        return fp32_bert_train_backward(c->raw, c->f32_opts(), &c->f32_train, d_txt, t->bw_grads, t->o.pad_idx, s);
     }
-    cudaError_t e = cudaMemsetAsync(dx_top, 0, sizeof(bf16) * static_cast<size_t>(T) * Hd, s);
+    bf16* dx_top = (c->layers.size() & 1) ? t->dxb : t->dxa;   // layer nl-1 reads dx[nl & 1]
+    cudaError_t e = cudaMemsetAsync(dx_top, 0, sizeof(bf16) * static_cast<size_t>(t->Ta) * Hd, s);
     if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(dX)");
     TRK("train.cls", CAT_MEM, scatter_cls_rows_bf16(d_txt, c->t_seq_off, B, Hd, dx_top, s));
-    }   // stage 0
-    if (!t->bw_want_text || c->fp32_check) return 0;   // stage 0 did everything there is to do
-    const std::string enc = "text_encoder.encoder.encoder.layer.";
-    for (size_t i = nl; i-- > 0;) {
-        if (!runs(1 + static_cast<int>(nl - 1 - i))) continue;
-        const BertLayerW& Lw = c->layers[i];
-        const TrainLayerBuf& b = t->L[i];
-        TrainLayerPlan& p = t->P[i];
-        const std::string pre = enc + std::to_string(i) + ".";
-        const bf16* dx_in = ((i + 1) & 1) ? t->dxb : t->dxa;
-        const DropCfg d_ffn = make_drop(seed, site_ffn_out(i), o.p_bert_hidden);
-        const DropCfg d_att = make_drop(seed, site_attn_out(i), o.p_bert_hidden);
-        // x_{i+1} = LN2(s2), s2 = h1 + drop(W2 g + b2)
-        TRK("train.ln_bwd", CAT_MEM, ln_bwd_bf16(b.s2, dx_in, Lw.ln2g, c->bert_ln_eps, T, Hd, c->t_nrows, t->d_s,
-                            grad_of(gt, pre + "output.LayerNorm.weight"), grad_of(gt, pre + "output.LayerNorm.bias"), s));
-        const bf16* dz = t->d_s;
-        if (d_ffn.thresh) {
-            TRK("train.dropout", CAT_MEM, dropout_bf16(t->d_s, Hd, T, Hd, c->t_nrows, d_ffn, t->dz, Hd, s));
-            dz = t->dz;
-        }
-        MRD_TRY(train_wgrad(c, t, t->w_f2, dz, Hd, b.g, F, grad_of(gt, pre + "output.dense.weight"),
-                            grad_of(gt, pre + "output.dense.bias"), s));
-        MRD_TRY(run(c, "train.dgrad", dz == t->dz ? p.d_g : p.d_g0, s));
-        TRK("train.gelu_bwd", CAT_MEM, gelu_bwd_bf16(b.u, t->dbig, T, F, c->t_nrows, t->dbig, s));
-        MRD_TRY(train_wgrad(c, t, t->w_f1, t->dbig, F, b.h1, Hd, grad_of(gt, pre + "intermediate.dense.weight"),
-                            grad_of(gt, pre + "intermediate.dense.bias"), s));
-        MRD_TRY(run(c, "train.dgrad", p.d_h1, s));   // dh1 = du W1 + d_s2
-        // h1 = LN1(s1), s1 = x + drop(Wo ctx + bo)
-        TRK("train.ln_bwd", CAT_MEM, ln_bwd_bf16(b.s1, t->dh1, Lw.ln1g, c->bert_ln_eps, T, Hd, c->t_nrows, t->d_s,
-                            grad_of(gt, pre + "attention.output.LayerNorm.weight"),
-                            grad_of(gt, pre + "attention.output.LayerNorm.bias"), s));
-        dz = t->d_s;
-        if (d_att.thresh) {
-            TRK("train.dropout", CAT_MEM, dropout_bf16(t->d_s, Hd, T, Hd, c->t_nrows, d_att, t->dz, Hd, s));
-            dz = t->dz;
-        }
-        MRD_TRY(train_wgrad(c, t, t->w_o, dz, Hd, b.ctx, Hd, grad_of(gt, pre + "attention.output.dense.weight"),
-                            grad_of(gt, pre + "attention.output.dense.bias"), s));
-        MRD_TRY(run(c, "train.dgrad", dz == t->dz ? p.d_ctx : p.d_ctx0, s));
-        if (t->dkv_acc) cudaMemsetAsync(t->dkv_acc, 0, sizeof(float) * static_cast<size_t>(T) * 2 * Hd, s);
-        TRK("train.attention_bwd", CAT_ATTN, attention_backward(b.qkv, b.ctx, t->dctx, c->t_bias, c->t_seq_off, B, S, c->bert_heads,
-                                   make_drop(seed, site_attn(i), o.p_bert_attn), t->dqkv, s, t->dkv_acc));
-        if (t->dkv_acc)   // fp32 dK | dV accumulators -> the K / V columns of dqkv
-            TRK("train.attention_bwd", CAT_MEM, cast_f32_to_bf16(t->dkv_acc, 2 * Hd, T, 2 * Hd, t->dqkv + Hd, 3 * Hd, s));
-        // QKV: one [3*Hd, Hd] product, split into the three parameters (the query block carries the
-        // folded 1/sqrt(64): d/dWq = 0.125 * d/dWq')
-        float* gq = grad_of(gt, pre + "attention.self.query.weight");
-        float* gk = grad_of(gt, pre + "attention.self.key.weight");
-        float* gv = grad_of(gt, pre + "attention.self.value.weight");
-        float* bq = grad_of(gt, pre + "attention.self.query.bias");
-        float* bk = grad_of(gt, pre + "attention.self.key.bias");
-        float* bv = grad_of(gt, pre + "attention.self.value.bias");
-        const bool want_w = gq || gk || gv, want_b = bq || bk || bv;
-        if (want_w || want_b) {
-            if (want_w) cudaMemsetAsync(t->wq_scratch, 0, sizeof(float) * 3 * static_cast<size_t>(Hd) * Hd, s);
-            if (want_b) cudaMemsetAsync(t->bq_scratch, 0, sizeof(float) * 3 * Hd, s);
-            MRD_TRY(train_wgrad(c, t, t->w_qkv, t->dqkv, 3 * Hd, b.x, Hd, want_w ? t->wq_scratch : nullptr,
-                                want_b ? t->bq_scratch : nullptr, s));
-            const size_t blk = sizeof(float) * static_cast<size_t>(Hd) * Hd;
-            if (gq) {
-                TRK("train.scale", CAT_MEM, scale_f32(t->wq_scratch, 1LL * Hd * Hd, 0.125f, s));
-                cudaMemcpyAsync(gq, t->wq_scratch, blk, cudaMemcpyDeviceToDevice, s);
-            }
-            if (gk) cudaMemcpyAsync(gk, t->wq_scratch + 1LL * Hd * Hd, blk, cudaMemcpyDeviceToDevice, s);
-            if (gv) cudaMemcpyAsync(gv, t->wq_scratch + 2LL * Hd * Hd, blk, cudaMemcpyDeviceToDevice, s);
-            if (bq) {
-                TRK("train.scale", CAT_MEM, scale_f32(t->bq_scratch, Hd, 0.125f, s));
-                cudaMemcpyAsync(bq, t->bq_scratch, sizeof(float) * Hd, cudaMemcpyDeviceToDevice, s);
-            }
-            if (bk) cudaMemcpyAsync(bk, t->bq_scratch + Hd, sizeof(float) * Hd, cudaMemcpyDeviceToDevice, s);
-            if (bv) cudaMemcpyAsync(bv, t->bq_scratch + 2 * Hd, sizeof(float) * Hd, cudaMemcpyDeviceToDevice, s);
-        }
-        MRD_TRY(run(c, "train.dgrad", p.d_x, s));    // dx_i = dqkv Wqkv + d_s1
+    return 0;
+}
+
+// ---- stages 1 .. layers: one BERT layer each, in reverse
+// QKV weight gradient of layer input x: one [3*Hd, Hd] product into zeroed scratch, split into the three parameters.
+// The query block carries the folded 1/sqrt(64): d/dWq = 0.125 * d/dWq'.
+int bw_qkv_wgrad(mrd_ctx* c, TrainState* t, const bf16* x, const std::string& pre, cudaStream_t s) {
+    const GradTable& gt = t->bw_grads;
+    const int Hd = c->hidden;
+    const std::string sa = pre + "attention.self.";
+    struct Part {
+        float* scratch;
+        long long n;       // elements per parameter
+        float* dst[3];     // query, key, value
+        bool want() const { return dst[0] || dst[1] || dst[2]; }
+    };
+    const Part parts[2] = {
+        {t->wq_scratch, 1LL * Hd * Hd,
+         {grad_of(gt, sa + "query.weight"), grad_of(gt, sa + "key.weight"), grad_of(gt, sa + "value.weight")}},
+        {t->bq_scratch, Hd, {grad_of(gt, sa + "query.bias"), grad_of(gt, sa + "key.bias"), grad_of(gt, sa + "value.bias")}}};
+    if (!parts[0].want() && !parts[1].want()) return 0;
+    for (const Part& p : parts) {
+        if (!p.want()) continue;
+        cudaError_t e = cudaMemsetAsync(p.scratch, 0, sizeof(float) * 3 * static_cast<size_t>(p.n), s);
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(QKV gradient scratch)");
     }
-    if (!runs(static_cast<int>(nl) + 1)) return 0;
-    // ---- embeddings: dropout, LayerNorm backward, scatter-add into the three tables
+    MRD_TRY(train_wgrad(c, t, t->w_qkv, t->dqkv, 3 * Hd, x, Hd, parts[0].want() ? t->wq_scratch : nullptr,
+                        parts[1].want() ? t->bq_scratch : nullptr, s));
+    for (const Part& p : parts) {
+        if (p.dst[0]) TRK("train.scale", CAT_MEM, scale_f32(p.scratch, p.n, 0.125f, s));
+        for (int k = 0; k < 3; ++k) {
+            if (!p.dst[k]) continue;
+            cudaError_t e = cudaMemcpyAsync(p.dst[k], p.scratch + k * p.n, sizeof(float) * static_cast<size_t>(p.n),
+                                            cudaMemcpyDeviceToDevice, s);
+            if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync(QKV gradient split)");
+        }
+    }
+    return 0;
+}
+
+// Layer i reads its output gradient from dx[(i+1)&1] and writes its input gradient to dx[i&1] (the d_x plan).
+int bw_bert_layer(mrd_ctx* c, TrainState* t, size_t i, cudaStream_t s) {
+    const GradTable& gt = t->bw_grads;
+    const TrainOpts& o = t->o;
+    const unsigned long long seed = t->seed;
+    const int B = t->B, S = t->S, T = t->Ta, Hd = c->hidden, F = c->ffn;
+    const BertLayerW& Lw = c->layers[i];
+    const TrainLayerBuf& b = t->L[i];
+    TrainLayerPlan& p = t->P[i];
+    const std::string pre = "text_encoder.encoder.encoder.layer." + std::to_string(i) + ".";
+    const bf16* dx_in = ((i + 1) & 1) ? t->dxb : t->dxa;
+    const DropCfg d_ffn = make_drop(seed, site_ffn_out(i), o.p_bert_hidden);
+    const DropCfg d_att = make_drop(seed, site_attn_out(i), o.p_bert_hidden);
+    // x_{i+1} = LN2(s2), s2 = h1 + drop(W2 g + b2)
+    TRK("train.ln_bwd", CAT_MEM, ln_bwd_bf16(b.s2, dx_in, Lw.ln2g, c->bert_ln_eps, T, Hd, c->t_nrows, t->d_s,
+                        grad_of(gt, pre + "output.LayerNorm.weight"), grad_of(gt, pre + "output.LayerNorm.bias"), s));
+    const bf16* dz = t->d_s;
+    if (d_ffn.thresh) {
+        TRK("train.dropout", CAT_MEM, dropout_bf16(t->d_s, Hd, T, Hd, c->t_nrows, d_ffn, t->dz, Hd, s));
+        dz = t->dz;
+    }
+    MRD_TRY(train_wgrad(c, t, t->w_f2, dz, Hd, b.g, F, grad_of(gt, pre + "output.dense.weight"),
+                        grad_of(gt, pre + "output.dense.bias"), s));
+    MRD_TRY(run(c, "train.dgrad", dz == t->dz ? p.d_g : p.d_g0, s));
+    TRK("train.gelu_bwd", CAT_MEM, gelu_bwd_bf16(b.u, t->dbig, T, F, c->t_nrows, t->dbig, s));
+    MRD_TRY(train_wgrad(c, t, t->w_f1, t->dbig, F, b.h1, Hd, grad_of(gt, pre + "intermediate.dense.weight"),
+                        grad_of(gt, pre + "intermediate.dense.bias"), s));
+    MRD_TRY(run(c, "train.dgrad", p.d_h1, s));   // dh1 = du W1 + d_s2
+    // h1 = LN1(s1), s1 = x + drop(Wo ctx + bo)
+    TRK("train.ln_bwd", CAT_MEM, ln_bwd_bf16(b.s1, t->dh1, Lw.ln1g, c->bert_ln_eps, T, Hd, c->t_nrows, t->d_s,
+                        grad_of(gt, pre + "attention.output.LayerNorm.weight"),
+                        grad_of(gt, pre + "attention.output.LayerNorm.bias"), s));
+    dz = t->d_s;
+    if (d_att.thresh) {
+        TRK("train.dropout", CAT_MEM, dropout_bf16(t->d_s, Hd, T, Hd, c->t_nrows, d_att, t->dz, Hd, s));
+        dz = t->dz;
+    }
+    MRD_TRY(train_wgrad(c, t, t->w_o, dz, Hd, b.ctx, Hd, grad_of(gt, pre + "attention.output.dense.weight"),
+                        grad_of(gt, pre + "attention.output.dense.bias"), s));
+    MRD_TRY(run(c, "train.dgrad", dz == t->dz ? p.d_ctx : p.d_ctx0, s));
+    if (t->dkv_acc) {
+        cudaError_t e = cudaMemsetAsync(t->dkv_acc, 0, sizeof(float) * static_cast<size_t>(T) * 2 * Hd, s);
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(dK/dV accumulator)");
+    }
+    TRK("train.attention_bwd", CAT_ATTN, attention_backward(b.qkv, b.ctx, t->dctx, c->t_bias, c->t_seq_off, B, S, c->bert_heads,
+                               make_drop(seed, site_attn(i), o.p_bert_attn), t->dqkv, s, t->dkv_acc));
+    if (t->dkv_acc)   // fp32 dK | dV accumulators -> the K / V columns of dqkv
+        TRK("train.attention_bwd", CAT_MEM, cast_f32_to_bf16(t->dkv_acc, 2 * Hd, T, 2 * Hd, t->dqkv + Hd, 3 * Hd, s));
+    MRD_TRY(bw_qkv_wgrad(c, t, b.x, pre, s));
+    return run(c, "train.dgrad", p.d_x, s);    // dx_i = dqkv Wqkv + d_s1
+}
+
+// ---- stage layers + 1: embeddings: dropout, LayerNorm backward, scatter-add into the three tables
+int bw_embeddings(mrd_ctx* c, TrainState* t, cudaStream_t s) {
+    const GradTable& gt = t->bw_grads;
+    const int T = t->Ta, Hd = c->hidden;
     bf16* dx0 = t->dxa;   // layer 0 wrote dx[0]
-    TRK("train.dropout", CAT_MEM, dropout_bf16(dx0, Hd, T, Hd, c->t_nrows, make_drop(seed, SITE_EMB, o.p_bert_hidden), dx0, Hd, s));
+    TRK("train.dropout", CAT_MEM, dropout_bf16(dx0, Hd, T, Hd, c->t_nrows, make_drop(t->seed, SITE_EMB, t->o.p_bert_hidden), dx0, Hd, s));
     const std::string em = "text_encoder.encoder.embeddings.";
     float* g_word = grad_of(gt, em + "word_embeddings.weight");
     float* g_pos = grad_of(gt, em + "position_embeddings.weight");
@@ -964,10 +1004,32 @@ int train_backward_run(mrd_ctx* c, int lo, int hi, cudaStream_t s) {
     float* g_lg = grad_of(gt, em + "LayerNorm.weight");
     float* g_lb = grad_of(gt, em + "LayerNorm.bias");
     if (g_word || g_pos || g_type || g_lg || g_lb)
-        TRK("train.embed_bwd", CAT_MEM, embed_ln_bwd(t->ids, c->t_row_tok, T, c->t_nrows, S, c->word_emb, c->pos_type, c->emb_g,
-                             c->bert_ln_eps, c->vocab, o.pad_idx, dx0, g_word, g_pos, g_type, g_lg, g_lb, s));
+        TRK("train.embed_bwd", CAT_MEM, embed_ln_bwd(t->ids, c->t_row_tok, T, c->t_nrows, t->S, c->word_emb, c->pos_type, c->emb_g,
+                             c->bert_ln_eps, c->vocab, t->o.pad_idx, dx0, g_word, g_pos, g_type, g_lg, g_lb, s));
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "training backward");
+    return 0;
+}
+
+// Runs stages [lo, hi) of the pending backward; stages must be run in order, each exactly once.  Without a text
+// encoder gradient, and in the fp32 check, stage 0 does everything there is to do and the later stages are no-ops.
+int train_backward_run(mrd_ctx* c, int lo, int hi, cudaStream_t s) {
+    TrainState* t = train_state(c);
+    const int n_stages = train_backward_stages(c);
+    if (!t->bw_active || lo != t->bw_next || hi <= lo || hi > n_stages) {
+        set_last_error("mrd_train_backward_stage: stages [%d, %d) out of order (next %d of %d, %s)", lo, hi,
+                       t->bw_next, n_stages, t->bw_active ? "active" : "no backward begun");
+        return -1;
+    }
+    t->bw_next = hi;
+    if (hi == n_stages) t->bw_active = false;
+    const int nl = n_stages - 2;
+    for (int st = lo; st < hi; ++st) {
+        if (st == 0) MRD_TRY(bw_batch_layers(c, t, s));
+        else if (!t->bw_want_text || c->fp32_check) break;
+        else if (st <= nl) MRD_TRY(bw_bert_layer(c, t, static_cast<size_t>(nl - st), s));
+        else MRD_TRY(bw_embeddings(c, t, s));
+    }
     return 0;
 }
 
