@@ -260,8 +260,8 @@ int mrd_compact_tokens(const void* mask, int mask_dtype, int B, int S, int keep_
 int mrd_attention_varlen_bf16(const void* qkv, const float* row_bias, const int* seq_off, int B,
                               int max_len, int heads, long long total_rows, void* out, void* stream);
 
-/* Attention with max length <= 128 runs on tcgen05 (TMEM scores, TMA tiles); 0 forces the mma.sync
- * kernel that serves longer sequences (process-wide test switch). */
+/* Attention with max length <= 512 runs on tcgen05 (TMEM scores, TMA tiles); 0 forces the mma.sync
+ * kernel for every length, the only way to reach it (dropout included; process-wide test switch). */
 int mrd_attention_use_tcgen05(int on);
 
 /* attention_mask [B,S] -> additive key bias (0 / -inf). */
@@ -377,6 +377,14 @@ int mrd_dropout_mask(unsigned long long seed, unsigned int site, double p, long 
 int mrd_attention_train_bf16(const void* qkv, const float* mask_bias, int B, int S, int heads,
                              unsigned long long seed, unsigned int site, double p, void* out,
                              void* stream);
+
+/* The training step's attention forward on the token-packed layout: mrd_attention_varlen_bf16 (sample b owns rows
+ * [seq_off[b], seq_off[b+1]) of qkv, row_bias and out; S_max bounds the lengths; rows = rows of the qkv / out
+ * allocations) with dropout on the probabilities.  The element index of (b,h,q,k) is ((b*heads + h)*S_max + q)*S_max
+ * + k with q and k counted inside sample b and S_max the padded width, as mrd_attention_bwd_bf16 recomputes it. */
+int mrd_attention_train_varlen_bf16(const void* qkv, const float* row_bias, const int* seq_off, int B, int S_max,
+                                    int heads, long long rows, unsigned long long seed, unsigned int site, double p,
+                                    void* out, void* stream);
 
 /* Backward of the fused attention: qkv / dqkv bf16 [rows, 3*heads*64], ctx (forward output) / dctx bf16
  * [rows, heads*64]; dQ is the gradient of the pre-scaled Q.  seq_off as mrd_attention_varlen_bf16 or

@@ -86,6 +86,7 @@ SIGNATURES = {
     "mrd_stem_dgrad_f32": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
     "mrd_dropout_mask": (_i, [C.c_ulonglong, C.c_uint, _d, _ll, _vp, _vp]),
     "mrd_attention_train_bf16": (_i, [_vp, _vp, _i, _i, _i, C.c_ulonglong, C.c_uint, _d, _vp, _vp]),
+    "mrd_attention_train_varlen_bf16": (_i, [_vp, _vp, _vp, _i, _i, _i, _ll, C.c_ulonglong, C.c_uint, _d, _vp, _vp]),
     "mrd_attention_bwd_bf16": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, C.c_ulonglong, C.c_uint, _d, _vp, _vp,
                                     _ll, _vp]),
     "mrd_adamw_step": (_i, [_vp, _i, _vp, _vp, _i, _i, _f, _f, _f, _ll, _f, _vp, _vp]),

@@ -16,7 +16,7 @@ struct DropCfg;
 // seq_off (optional, device, B+1 ints): token-packed layout - sample b owns rows
 // [seq_off[b], seq_off[b+1]) of qkv/out and of mask_bias; S is then the maximum sequence length.
 // rows_alloc: rows of the qkv / out allocations (>= the last row any sample touches; default B*S).
-// S <= 128 runs on tcgen05 (TMA-fed 128x128 tiles, S and O in TMEM); longer sequences on mma.sync.
+// S <= 512 runs on tcgen05 (TMA-fed 128x128 tiles, S and O in TMEM); attention_set_tc(false) selects mma.sync.
 int attention_forward(const __nv_bfloat16* qkv, const float* mask_bias, const int* seq_off, int B,
                       int S, int heads, __nv_bfloat16* out, cudaStream_t stream,
                       long long rows_alloc = 0, int blocked = 0, const struct DropCfg* drop = nullptr);

@@ -1800,6 +1800,22 @@ int mrd_attention_train_bf16(const void* qkv, const float* mask_bias, int B, int
                              static_cast<bf16*>(out), static_cast<cudaStream_t>(stream), 0, 0, &d);
 }
 
+int mrd_attention_train_varlen_bf16(const void* qkv, const float* row_bias, const int* seq_off, int B, int S_max,
+                                    int heads, long long rows, unsigned long long seed, unsigned int site, double p,
+                                    void* out, void* stream) {
+    if (!seq_off) {
+        set_last_error("mrd_attention_train_varlen_bf16: seq_off is required");
+        return -1;
+    }
+    if (rows <= 0) {
+        set_last_error("mrd_attention_train_varlen_bf16: rows must be the row count of qkv / out");
+        return -1;
+    }
+    const DropCfg d = make_drop(seed, site, p);
+    return attention_forward(static_cast<const bf16*>(qkv), row_bias, seq_off, B, S_max, heads, static_cast<bf16*>(out),
+                             static_cast<cudaStream_t>(stream), rows, 0, &d);
+}
+
 int mrd_layernorm_bwd_bf16(const void* s_in, const void* dy, const float* gamma, float eps, int rows, int width,
                            void* dx, float* dgamma, float* dbeta, void* stream) {
     return ln_bwd_bf16(static_cast<const bf16*>(s_in), static_cast<const bf16*>(dy), gamma, eps, rows, width,

@@ -52,88 +52,6 @@ def _zero_dropout(model):
 
 
 # --------------------------------------------------------------------------------------- kernels
-def _attention_ref(qkv, bias, B, S, heads, dctx, mask=None, p=0.0):
-    """fp32 autograd reference on the bf16-rounded inputs.  qkv [B*S, 3*heads*64] (Q pre-scaled)."""
-    x = qkv.float().clone().requires_grad_(True)
-    q, k, v = x.view(B, S, 3, heads, 64).permute(2, 0, 3, 1, 4)
-    s = q @ k.transpose(-1, -2)
-    if bias is not None:
-        s = s + bias.view(B, 1, 1, S)
-    pr = torch.softmax(s, dim=-1)
-    if mask is not None:
-        pr = pr * mask.view(B, heads, S, S) / (1.0 - p)
-    o = (pr @ v).permute(0, 2, 1, 3).reshape(B * S, heads * 64)
-    o.backward(dctx.float())
-    return o.detach(), x.grad
-
-
-@pytest.mark.parametrize("B,S,lens,p", [(3, 128, [128, 77, 5], 0.0), (4, 48, [48, 48, 17, 1], 0.0),
-                                        (2, 128, [128, 100], 0.1), (5, 32, [32, 9, 32, 20, 31], 0.25),
-                                        # > 128 tokens: tiled backward (fp32 dK/dV accumulation), mma.sync forward
-                                        (3, 256, [256, 130, 3], 0.0), (2, 200, [200, 129], 0.1),
-                                        (2, 512, [512, 385], 0.0), (1, 384, [300], 0.2)])
-def test_attention_backward_vs_autograd(cuda, lib, B, S, lens, p):
-    heads = 12
-    g = torch.Generator().manual_seed(5)
-    qkv = (torch.randn(B * S, 3 * heads * 64, generator=g) * 0.7).to(cuda, torch.bfloat16)
-    dctx = torch.randn(B * S, heads * 64, generator=g).to(cuda, torch.bfloat16)
-    bias = torch.zeros(B, S)
-    for b, L in enumerate(lens):
-        bias[b, L:] = float("-inf")
-    bias = bias.to(cuda)
-    seed, site = 1234567, 7
-    mask = None
-    if p > 0:
-        mask = torch.empty(B * heads * S * S, device=cuda)
-        assert lib.mrd_dropout_mask(C.c_ulonglong(seed), site, p, mask.numel(), _p(mask), _stream()) == 0
-        assert abs(mask.mean().item() - (1 - p)) < 0.01
-    # forward with the same mask (tcgen05 kernel), then the backward kernel
-    out = torch.empty(B * S, heads * 64, device=cuda, dtype=torch.bfloat16)
-    assert lib.mrd_attention_train_bf16(_p(qkv), _p(bias), B, S, heads, C.c_ulonglong(seed), site, p, _p(out),
-                                        _stream()) == 0, lib.mrd_last_error()
-    o_ref, d_ref = _attention_ref(qkv, bias, B, S, heads, dctx, mask, p)
-    live = (bias > float("-inf")).view(B * S)
-    err_o = (out.float()[live] - o_ref[live]).norm() / o_ref[live].norm()
-    assert err_o.item() <= 1e-2, err_o.item()
-    dqkv = torch.zeros_like(qkv)
-    acc = torch.zeros(B * S, 2 * heads * 64, device=cuda) if S > 128 else None
-    assert lib.mrd_attention_bwd_bf16(_p(qkv), _p(out), _p(dctx), _p(bias), None, B, S, heads, C.c_ulonglong(seed),
-                                      site, p, _p(dqkv), None if acc is None else _p(acc), B * S,
-                                      _stream()) == 0, lib.mrd_last_error()
-    torch.cuda.synchronize()
-    # padded QUERY rows are outputs nobody reads: the engine never feeds them a gradient; here they do get
-    # one, so compare everything (keys beyond the length receive exactly zero dK/dV in both)
-    for name, sl in (("dQ", slice(0, 768)), ("dK", slice(768, 1536)), ("dV", slice(1536, 2304))):
-        a, r = dqkv.float()[:, sl], d_ref[:, sl]
-        err = ((a - r).norm() / r.norm()).item()
-        assert err <= 2e-2, (name, err)
-
-
-def test_attention_backward_packed_layout(cuda, lib):
-    """Token-packed rows (seq_off) give the same gradients as the dense layout with a key bias."""
-    B, S, heads, lens = 4, 64, 12, [64, 30, 1, 47]
-    g = torch.Generator().manual_seed(6)
-    qkv = (torch.randn(B * S, 2304, generator=g) * 0.7).to(cuda, torch.bfloat16)
-    dctx = torch.randn(B * S, 768, generator=g).to(cuda, torch.bfloat16)
-    ctx = torch.randn(B * S, 768, generator=g).to(cuda, torch.bfloat16)
-    rows = torch.cat([torch.arange(L) + b * S for b, L in enumerate(lens)]).to(cuda)
-    off = torch.tensor([0] + list(torch.tensor(lens).cumsum(0)), dtype=torch.int32, device=cuda)
-    bias = torch.zeros(B, S)
-    for b, L in enumerate(lens):
-        bias[b, L:] = float("-inf")
-    bias = bias.to(cuda)
-    dctx[(bias == float("-inf")).view(B * S).cpu()] = 0   # padded queries do not exist in the packed layout
-    d_dense = torch.zeros_like(qkv)
-    assert lib.mrd_attention_bwd_bf16(_p(qkv), _p(ctx), _p(dctx), _p(bias), None, B, S, heads, C.c_ulonglong(1), 0,
-                                      0.0, _p(d_dense), None, B * S, _stream()) == 0
-    pq, pc, pd = qkv[rows].contiguous(), ctx[rows].contiguous(), dctx[rows].contiguous()
-    d_pack = torch.zeros_like(pq)
-    assert lib.mrd_attention_bwd_bf16(_p(pq), _p(pc), _p(pd), None, _p(off), B, S, heads, C.c_ulonglong(1), 0, 0.0,
-                                      _p(d_pack), None, pq.shape[0], _stream()) == 0
-    torch.cuda.synchronize()
-    assert torch.equal(d_pack, d_dense[rows])
-
-
 @pytest.mark.parametrize("M,N,K,live", [(768, 3072, 2048, None), (3072, 768, 4096, 2560), (2304, 768, 1024, 700),
                                         (768, 768, 512, 64), (256, 64, 8192, None)])
 def test_splitk_weight_gradient_gemm(cuda, lib, M, N, K, live):

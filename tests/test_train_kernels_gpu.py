@@ -23,6 +23,8 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+import synth
+
 pytestmark = pytest.mark.gpu
 
 BF = torch.bfloat16
@@ -99,27 +101,6 @@ def _scale(p):
     return torch.tensor(1.0 / (1.0 - p), dtype=torch.float64).float().item() if p > 0 else 1.0
 
 
-def _packed(lib, cuda, B, S, seed):
-    """Token packing of a ragged right-padded batch by mrd_compact_tokens: (live row count n, its device copy,
-    seq_off, row_tok, mask).  Lengths are uniform in [1, S] (about half the tokens live) and n % 64 != 0."""
-    g = torch.Generator().manual_seed(seed)
-    lens = torch.randint(1, S + 1, (B,), generator=g)
-    if int(lens.sum()) % 64 == 0:
-        lens[-1] = lens[-1] - 1 if lens[-1] > 1 else 2
-    mask = (torch.arange(S)[None, :] < lens[:, None]).long().to(cuda)
-    seq_off = torch.zeros(B + 1, device=cuda, dtype=torch.int32)
-    # row_tok past the live count keeps valid but unrelated token indices: nothing may use them
-    row_tok = torch.randint(0, B * S, (B * S,), device=cuda, dtype=torch.int32)
-    row_bias = torch.zeros(B * S, device=cuda)
-    n_rows = torch.zeros(1, device=cuda, dtype=torch.int32)
-    scratch = torch.zeros(B, device=cuda, dtype=torch.int32)
-    _check(lib, lib.mrd_compact_tokens(mask.data_ptr(), 0, B, S, 0, seq_off.data_ptr(), row_tok.data_ptr(),
-                                       row_bias.data_ptr(), n_rows.data_ptr(), scratch.data_ptr(), _stream()))
-    n = int(n_rows.item())
-    assert n == int(lens.sum()) and n % 64 != 0
-    return n, n_rows, seq_off, row_tok, mask
-
-
 # ------------------------------------------------------------------ dropout
 @pytest.mark.parametrize("p", [0.0, 0.1, 0.5])
 @pytest.mark.parametrize("strided", [False, True])
@@ -127,7 +108,7 @@ def test_dropout_bf16(lib, cuda, p, strided):
     """In place (as on the embeddings' output), and from / into [T, 2*width] buffers: the mask index is r*width + c
     whatever the strides, and rows past dyn_rows are not touched."""
     width = 768
-    n, n_rows, *_ = _packed(lib, cuda, 64, 128, 1)
+    n, n_rows, *_ = synth.packed(lib, cuda, 64, 128, 1)
     g = _gen(2)
     seed, site = 0x5eed, 11
     ld = 2 * width if strided else width
@@ -193,7 +174,7 @@ def test_drop_add_layernorm(lib, cuda, width, p, ragged):
     """s = res + dropout(z) stored in bf16, y = LayerNorm(s): T = 8192 rows with a ragged dyn_rows, or 1003 rows
     (not a multiple of the 8 rows of a block) without it."""
     if ragged:
-        rows, (n, n_rows, *_) = T_ROWS, _packed(lib, cuda, 64, 128, width)
+        rows, (n, n_rows, *_) = T_ROWS, synth.packed(lib, cuda, 64, 128, width)
     else:
         rows, n, n_rows = 1003, 1003, None
     g = _gen(width + 1)
@@ -293,7 +274,7 @@ def _gelu_sweep(n, cuda):
 def test_gelu_forward_backward(lib, cuda, ragged):
     """Exact-erf GELU and its derivative Phi(u) + u phi(u) over T x 3072 (several grid-stride passes)."""
     width = 3072
-    n, n_rows, *_ = _packed(lib, cuda, 64, 128, 5) if ragged else (T_ROWS, None)
+    n, n_rows, *_ = synth.packed(lib, cuda, 64, 128, 5) if ragged else (T_ROWS, None)
     u = _gelu_sweep(T_ROWS * width, cuda).view(T_ROWS, width)
     u[n:] = float("nan")
     dg = torch.randn(T_ROWS, width, device=cuda, generator=_gen(6)).to(BF)
@@ -345,7 +326,7 @@ def test_transpose_pad2(lib, cuda, w0, w1, live, dyn):
     """y[c][r] = x[r][c] below the live count, zeros up to the next multiple of 64, then (dyn_rows) nothing written
     or (static count) zeros up to Kp; colsum0 += the column sums of x0 over the live rows."""
     if live is None:
-        live = _packed(lib, cuda, 64, 128, 7)[0]
+        live = synth.packed(lib, cuda, 64, 128, 7)[0]
     x0, x1, y0, y1, cs0, cs, _ = _stage(lib, cuda, w0, w1, live, dyn, w0 + live)
     up = min((live + 63) // 64 * 64, T_ROWS)
     zero = torch.zeros((), device=cuda, dtype=BF)
@@ -366,7 +347,7 @@ def test_wgrad_staging_and_splitk(lib, cuda, w0, w1, live):
     """The weight gradient as the training step computes it: stage dY and X with transpose_pad2_bf16 (sentinel NaN
     left beyond the live 64-row blocks), then dW = dY^T X with the split-K GEMM bounded by dyn_k = live."""
     if live is None:
-        live = _packed(lib, cuda, 64, 128, 8)[0]
+        live = synth.packed(lib, cuda, 64, 128, 8)[0]
     x0, x1, y0, y1, _, _, n_rows = _stage(lib, cuda, w0, w1, live, True, w1 + live)
     out = torch.zeros(w0, w1, device=cuda)
     _check(lib, lib.mrd_gemm_splitk_f32(y0.data_ptr(), T_ROWS, w0, T_ROWS, y1.data_ptr(), w1, out.data_ptr(), w1,
@@ -383,7 +364,7 @@ def test_wgrad_staging_and_splitk(lib, cuda, w0, w1, live):
 def test_colsum_bf16(lib, cuda, width, rows):
     """out[c] += scale * sum over the live rows; the rows past dyn_rows are NaN.  20,000 rows: the row split is
     capped at 64 blocks, so every warp loops."""
-    live = _packed(lib, cuda, 64, 128, 9)[0] if rows == T_ROWS else rows - 37
+    live = synth.packed(lib, cuda, 64, 128, 9)[0] if rows == T_ROWS else rows - 37
     n_rows = torch.tensor([live], device=cuda, dtype=torch.int32)
     g = _gen(width + rows)
     x = torch.randn(rows, width, device=cuda, generator=g).to(BF)
@@ -420,7 +401,7 @@ def test_colsum_f32_and_relu_bwd(lib, cuda):
 
 def test_cls_gather_scatter(lib, cuda):
     B, S, Hd = 64, 128, 768
-    n, _, seq_off, *_ = _packed(lib, cuda, B, S, 12)
+    n, _, seq_off, *_ = synth.packed(lib, cuda, B, S, 12)
     g = _gen(12)
     cls = seq_off[:B].long()
     x = torch.randn(T_ROWS, Hd, device=cuda, generator=g).to(BF)
@@ -442,7 +423,7 @@ def test_embed_layernorm_backward(lib, cuda, B, S):
     """LayerNorm backward of word[id] + pos_type[pos] on the packed rows, scattered into the word / position tables
     (a few hot ids: many adds per row), token_type row 0 and gamma / beta; pad_idx receives nothing."""
     Hd, vocab, pad, eps = 768, 30522, 0, 1e-12
-    n, n_rows, _, row_tok, mask = _packed(lib, cuda, B, S, 13 + S)
+    n, n_rows, _, row_tok, mask, _ = synth.packed(lib, cuda, B, S, 13 + S)
     g = _gen(S)
     ids = torch.randint(0, vocab, (B, S), device=cuda, generator=g)
     hot = torch.tensor([101, 1996, 2000, 7592], device=cuda)
